@@ -2,6 +2,7 @@
 """Benchmark of the flow hot path (BASELINE.json metric: flow Mpix/s & pairs/s, DAISY+kNN+BCD+consistency).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl flowb200|reference] [--workload NAME]
+                  [--dump-outputs DIR]
 
 One step = one synthetic image pair through the whole path: 2 x DAISY, per direction exact per-cell kNN
 proposals + random-neighbour proposals + `sweeps` BCD sweeps, then the forward/backward check.
@@ -21,6 +22,9 @@ huge   : (unless --no-huge) a short run of the single-huge-image mode (configs[4
          (dist.shard_units), each rank's share through flowb200_ctx_flow_pairs_host (copies overlapped).
 --impl reference: the CPU oracle alone, same metric/config (the reference itself is pure Python that
          needs opencv-contrib + pyflann, absent offline; its unmodified source runs only on tiny crops).
+--dump-outputs DIR: the outputs of the last timed step as .npy files (dump_outputs); the inputs are seeded, so two
+         builds run with the same arguments can be compared output for output.  With N ranks each rank writes its own
+         files (suffix _rank<r>), except in the huge mode, where every rank holds the same field.
 """
 import argparse
 import importlib
@@ -112,6 +116,34 @@ class ClockSampler:
         reasons = [n for j, n in enumerate(names) if any(len(r) >= 7 and r[3 + j].lower() == "active" for r in self.rows)]
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": reasons, "samples": len(sm)}
+
+
+DUMP_BYTES = 64_000_000          # all files of one --dump-outputs run together
+NPY_HEADER_BYTES = 4096          # upper bound of an .npy header (numpy pads it to a multiple of 64 bytes)
+
+
+def dump_outputs(dirname, arrays, suffix="", budget=DUMP_BYTES):
+    """Writes every array of `arrays` (name -> what a caller of the timed path received in its last step) as
+    <dirname>/<name><suffix>.npy, float64 kept and anything else as float32; the files, headers included, take at
+    most `budget` bytes.  When the arrays do not fit, every array is cut down to the same fixed, seeded sample of its
+    pixels (rows over its last axis), and <name>_index<suffix>.npy holds the flat indices of the pixels kept, so that
+    two builds can be compared element for element on identical inputs."""
+    os.makedirs(dirname, exist_ok=True)
+    arrays = {k: np.asarray(v.cpu() if hasattr(v, "cpu") else v) for k, v in arrays.items()}
+    arrays = {k: v if v.dtype == np.float64 else v.astype(np.float32) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    sample = total + NPY_HEADER_BYTES * len(arrays) > budget
+    payload = budget - 2 * NPY_HEADER_BYTES * len(arrays)        # a data and an index file per array
+    for name, a in arrays.items():
+        if sample:
+            rows = a.reshape(-1, a.shape[-1])
+            row_bytes = rows.shape[1] * rows.itemsize + 8          # the pixel and its float64 index
+            k = max(1, int(payload * a.nbytes / total) // row_bytes)
+            idx = np.sort(np.random.default_rng(0).choice(rows.shape[0], size=min(k, rows.shape[0]), replace=False))
+            # float64 because every dump file is float32 or float64; flat indices are exact in it below 2^53
+            np.save(os.path.join(dirname, f"{name}_index{suffix}.npy"), idx.astype(np.float64))
+            a = rows[idx]
+        np.save(os.path.join(dirname, f"{name}{suffix}.npy"), a)
 
 
 def make_params(workload, knn_mode):
@@ -242,7 +274,7 @@ def cpu_sample(p, sweeps, directions, steps=1):
     ts = []
     for s in range(steps):
         t0 = time.perf_counter()
-        cpu_oracle_pipeline(img1, img2, op, sweeps, directions, p.con_tresh, seed=s)
+        out = cpu_oracle_pipeline(img1, img2, op, sweeps, directions, p.con_tresh, seed=s)
         ts.append(time.perf_counter() - t0)
     t = float(np.mean(ts))
 
@@ -262,7 +294,7 @@ def cpu_sample(p, sweeps, directions, steps=1):
                     "be lower (the exact search is ~60 % of the CPU time)",
             "sample": f"{steps} x {Ws}x{Hs} crop (5x5 cells of {p.cellw}x{p.cellh}), K={p.maxnprop}, bcd_times={sweeps}, "
                       f"{directions} direction(s), {t:.2f} s/step; C oracle with OpenMP + numpy DAISY",
-            "seconds_per_step": t}
+            "seconds_per_step": t, "output": out}
 
 
 def run_reference(args):
@@ -270,8 +302,10 @@ def run_reference(args):
     if rank != 0:
         return
     p, sweeps, directions = make_params(args.workload, 0)
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     r = cpu_sample(p, sweeps, directions, steps=steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"flow": r["output"]})
     line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": "Mpix/s", "n_gpus": args.gpus,
             "steps": steps, "warmup": 1, "ms_per_step": r["seconds_per_step"] * 1e3, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
@@ -326,11 +360,14 @@ def run_huge(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        step(W_ + i)
+        out = step(W_ + i)
     e1.record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
     launches = lib.load().flowb200_launch_count() - L0
+    if args.dump_outputs and rank == 0:       # the same field on every rank
+        dump_outputs(args.dump_outputs, {"flow": out})
+    del out
     t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -483,6 +520,9 @@ def run_batch(args):
     barrier()
     clocks = sampler.stop() if rank == 0 else None
     L.flowb200_ctx_destroy(ctx)
+    if args.dump_outputs:      # this rank's pairs, in the order of dist.shard_units
+        dump_outputs(args.dump_outputs, {"flow": np.stack(outs)}, f"_rank{rank}" if world > 1 else "",
+                     DUMP_BYTES // world)
     secs = float(t.item())
     if rank == 0:
         val = n_pairs * p.H * p.W / 1e6 / secs
@@ -518,7 +558,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-breakdown", action="store_true")
     ap.add_argument("--no-huge", action="store_true", help="skip the short single-huge-image run (key 'huge')")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy "
+                         "(float32 / float64, at most 64 MB = 64,000,000 bytes in all, over all ranks: "
+                         "a fixed, seeded sample of larger outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     if "huge" in args.workload:
@@ -589,7 +635,7 @@ def main():
                 raise errs[0]
             for s_ in side:
                 cur.wait_stream(s_)
-            return outs[0]
+            return outs
     step = step_batch if inflight > 1 else step_one
 
     def barrier():
@@ -612,6 +658,11 @@ def main():
     barrier()
     clocks = sampler.stop() if rank == 0 else None
     launches = (L.flowb200_launch_count() - launches0)
+    if args.dump_outputs:      # the checked forward field of every pair of the last step
+        outs = out if inflight > 1 else [out]
+        names = ["flow"] if inflight == 1 else [f"flow_{j}" for j in range(inflight)]
+        dump_outputs(args.dump_outputs, dict(zip(names, outs)), f"_rank{rank}" if world > 1 else "",
+                     DUMP_BYTES // world)
     ms = e0.elapsed_time(e1)
     t = torch.tensor([ms], dtype=torch.float64, device="cuda")
     if world > 1:

@@ -9,11 +9,14 @@ import importlib
 import os
 import sys
 import tempfile
+import zipfile
 
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+import helpers                                # noqa: E402
 from oracle import ref_harness as rh          # noqa: E402
 from oracle import daisy as odaisy            # noqa: E402
 
@@ -65,12 +68,32 @@ def stage_case(name, H, W, cw, ch, pair, sweeps, seed, both_dirs, thresholds=())
         data[f"sparse_thr{thr}"] = np.load(out)
         assert np.array_equal(fi.flow, data[f"sparse_thr{thr}"])
         print(name, "thr", thr, "valid", float(data[f"sparse_thr{thr}"][..., 2].mean()))
-    np.savez_compressed(os.path.join(OUT, name + ".npz"), **data)
+    save_case(os.path.join(OUT, name + ".npz"), data)
+    return data
 
 
-def bcd_quantised_case(name, src_case, sweeps, shift):
-    """Reference BCD on costs quantised to 20*m/2^S (exact in float64): pins the int32 mode."""
-    z = np.load(os.path.join(OUT, src_case + ".npz"))
+def save_case(path, data):
+    """Writes a stage case with the stage-1 proposals, costs and K-set bits of every direction replaced by digests
+    (tests/helpers.load_case recomputes them with the oracle and checks them against the digests), LZMA-compressed:
+    the full arrays would make the file several MB."""
+    data = dict(data)
+    K = int(data[[k for k in data if k.endswith("_proposals")][0]].shape[2])
+    for b in (0, 1):
+        if f"b{b}_proposals" not in data:
+            continue
+        nprop = data[f"b{b}_nprop"].astype(np.int64)
+        data[f"b{b}_proposals_sha256"] = helpers.digest(data.pop(f"b{b}_proposals").astype(np.int64))
+        data[f"b{b}_lcosts_sha256"] = helpers.digest(data.pop(f"b{b}_lcosts").astype(np.float64))
+        data[f"b{b}_packedksets_sha256"] = helpers.ksets_digest(data.pop(f"b{b}_packedksets"), nprop, K)
+    with zipfile.ZipFile(path, "w", compression=zipfile.ZIP_LZMA) as zf:
+        for k, v in data.items():
+            with zf.open(k + ".npy", "w") as f:
+                np.lib.format.write_array(f, np.asanyarray(v))
+
+
+def bcd_quantised_case(name, z, sweeps, shift):
+    """Reference BCD on costs quantised to 20*m/2^S (exact in float64): pins the int32 mode.  z: what stage_case
+    returned, i.e. the reference's own stage-1 arrays (the saved case keeps only their digests)."""
     H, W, cw, ch, pair, _, _ = (int(v) for v in z["meta"])
     lc = z["b0_lcosts"].astype(np.float64)
     m = np.rint(0.05 * lc * (1 << shift)).astype(np.int64)
@@ -131,6 +154,6 @@ if __name__ == "__main__":
     assert rh.available(), "reference source not found"
     consistency_cases()
     parovi_case()
-    stage_case("pair_a", 40, 48, 12, 10, pair=3, sweeps=2, seed=5, both_dirs=True, thresholds=(10, 2))
+    pair_a = stage_case("pair_a", 40, 48, 12, 10, pair=3, sweeps=2, seed=5, both_dirs=True, thresholds=(10, 2))
     stage_case("pair_b", 44, 50, 12, 10, pair=7, sweeps=1, seed=9, both_dirs=False)
-    bcd_quantised_case("bcd_q12", "pair_a", sweeps=3, shift=12)
+    bcd_quantised_case("bcd_q12", pair_a, sweeps=3, shift=12)

@@ -1,4 +1,6 @@
 """Shared test helpers: golden fixture loading and the importable product package."""
+import functools
+import hashlib
 import importlib
 import os
 
@@ -16,19 +18,66 @@ def load_npz(name):
     return dict(np.load(os.path.join(GOLDEN, name + ".npz")))
 
 
-def load_case(name):
-    """Restore the reference dtypes (int64 proposals / nprop / labels, float64 lcosts / flows)."""
+def digest(a):
+    """SHA-256 of an array's dtype, shape and bytes, as uint8 (32,)."""
+    a = np.ascontiguousarray(a)
+    h = hashlib.sha256(f"{a.dtype.str} {a.shape}".encode())
+    h.update(a.tobytes())
+    return np.frombuffer(h.digest(), dtype=np.uint8)
+
+
+def ksets_digest(packed, nprop, K):
+    """digest of the meaningful K-set bits of a packedksets array (H,W,2,K*K//8+1): pixel p and its down (slot 0) /
+    right (slot 1) neighbour q, bits [:nprop[p], :nprop[q]] (oracle.proposals.ksets_masked_equal compares the same)."""
+    H, W = nprop.shape
+    nq = np.zeros((H, W, 2), np.int64)
+    nq[:-1, :, 0] = nprop[1:, :]
+    nq[:, :-1, 1] = nprop[:, 1:]
+    k = np.arange(K)
+    mask = (k[:, None] < nprop[:, :, None, None, None]) & (k[None, :] < nq[..., None, None])
+    bits = np.unpackbits(packed, axis=-1)[..., :K * K].reshape(H, W, 2, K, K)
+    return digest(np.packbits(bits[mask]))
+
+
+@functools.lru_cache(maxsize=None)
+def _case(name):
     z = load_npz(name)
     out = {}
     for k, v in z.items():
         base = k.split("_", 1)[1] if k[:1] == "b" and k[1:2].isdigit() else k
+        if base.endswith("_sha256"):
+            continue
         if base in ("proposals", "nprop", "labels00", "draws") or base.startswith("labels"):
             out[k] = v.astype(np.int64)
         elif base == "lcosts" or base.startswith("flow"):
             out[k] = v.astype(np.float64)
         else:
             out[k] = v
+    # The reference's stage-1 proposals, costs and K-set bits are stored as digests (the arrays would exceed the
+    # fixture size): the oracle recomputes them from the stored descriptors and Gaussian draws, and they must be the
+    # reference's bit for bit.
+    from oracle import proposals as oprop
+    p = oracle_params(out["meta"])
+    for b in (0, 1):
+        if f"b{b}_proposals_sha256" not in z:
+            continue
+        d1, d2 = (out["desc1"], out["desc2"]) if b == 0 else (out["desc2"], out["desc1"])
+        P, L, N, B = oprop.generisi(d1, d2, p)
+        oprop.nasumicni(d1, d2, P, L, N, B, p, out[f"b{b}_draws"])
+        pk = oprop.pakovanje(P, N, p)
+        for key, ok in (("proposals", np.array_equal(digest(P), z[f"b{b}_proposals_sha256"])),
+                        ("lcosts", np.array_equal(digest(L), z[f"b{b}_lcosts_sha256"])),
+                        ("nprop", np.array_equal(N, out[f"b{b}_nprop"])),
+                        ("packedksets", np.array_equal(ksets_digest(pk, N, p.maxnprop), z[f"b{b}_packedksets_sha256"]))):
+            assert ok, f"{name} b{b}_{key}: the oracle's stage 1 differs from the reference's output"
+        out.update({f"b{b}_proposals": P, f"b{b}_lcosts": L, f"b{b}_packedksets": pk})
     return out
+
+
+def load_case(name):
+    """Restore the reference dtypes (int64 proposals / nprop / labels, float64 lcosts / flows).  The stage-1 proposals,
+    costs and K-set bits are recomputed and checked against the reference's digests once per process (_case)."""
+    return {k: v.copy() for k, v in _case(name).items()}
 
 
 def oracle_params(meta, **kw):

@@ -1,4 +1,9 @@
-"""The oracle restatements against outputs of the reference's own source (tests/golden, CPU only)."""
+"""The oracle restatements against outputs of the reference's own source (tests/golden, CPU only).
+
+pair_a / pair_b keep the reference's stage-1 proposals, costs and K-set bits as SHA-256 digests only: helpers.load_case
+recomputes them with the numpy oracle and checks them against the digests before any test sees them.  A regression of
+the oracle's stage 1 therefore fails in load_case (naming the case, direction and array), in every test that loads the
+case.  The comparisons below (and those of test_oracle_c and the GPU parity tests) use the verified arrays."""
 import numpy as np
 import pytest
 
