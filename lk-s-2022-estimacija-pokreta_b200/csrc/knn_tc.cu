@@ -576,12 +576,21 @@ __device__ __forceinline__ void screen_and_cost(const float* __restrict__ q, con
   cost = res;
 }
 
+// Interval [screen_lo(ds), screen_hi(ds)] that certainly holds the real-valued distance of a screening distance ds.
+// Relative part: 70 roundings of at most 2^-24 each (4.2e-6) for normal floats.  Absolute part: once partial sums are
+// subnormal, every fma rounds by up to half a subnormal ulp (2^-150) whatever the size of its result, so 68 of them
+// plus the rounding of the bound itself stay below 2^-142.  It matters at the rim of flat image regions, where
+// descriptors of ~1e-20 give squared distances below 2^-126 that the fma chain cannot order.
+__device__ __forceinline__ float screen_lo(float ds) { return ds * (1.0f - 1.0e-5f) - 0x1p-142f; }
+__device__ __forceinline__ float screen_hi(float ds) { return ds * (1.0f + 1.0e-5f) + 0x1p-142f; }
+
 __device__ __noinline__ double exact_dist_call(const float* __restrict__ q, const float* __restrict__ t) {
   return exact_dist(q, t);
 }
 
 // One half-warp per source pixel, looping over the pixel's cells (= blocks of the slot order); lane = candidate.
-// Ranking uses the float32 screening distance wherever it decides the order with certainty (relative gap > 2e-5);
+// Ranking uses the float32 screening distance wherever it decides the order with certainty (relative gap > 2e-5 and
+// absolute gap > 2^-141, see screen_lo / screen_hi);
 // candidates involved in an uncertain pair get the exact float64 distance of the oracle, so the final order is
 // always the oracle's (distance, index) order.
 template <int KC>
@@ -610,7 +619,7 @@ knn_rerank_kernel(const float* __restrict__ desc_src, const float* __restrict__ 
       if (ci < g.cx0 || ci >= g.cx1) continue;   // (uniform over the half-warp) another caller's band: slots left unwritten
       const int n = cand_cnt[task];
       if (n == 255) {
-        if (sub == 0) {
+        if (sub == 0) {   // (past fb_cap the fallback finds the overflowed tasks in cand_cnt instead)
           const int at = atomicAdd(fb_count, 1);
           if (at < fb_cap) {
             fb_list[2 * at] = (int)pix;
@@ -641,22 +650,24 @@ knn_rerank_kernel(const float* __restrict__ desc_src, const float* __restrict__ 
         screen_and_cost(qp, tp1, ds1, co1);
       }
       // rank by the screening distance; note every pair it cannot order with certainty
-      const float lo0 = ds0 * (1.0f - 1.0e-5f), hi0 = ds0 * (1.0f + 1.0e-5f);
-      const float lo1 = ds1 * (1.0f - 1.0e-5f), hi1 = ds1 * (1.0f + 1.0e-5f);
+      const float lo0 = screen_lo(ds0), hi0 = screen_hi(ds0);
+      const float lo1 = screen_lo(ds1), hi1 = screen_hi(ds1);
       int rank0 = 0, rank1 = 0;
       bool amb0 = false, amb1 = false;
       const int nl = n < 16 ? n : 16;   // (lanes >= n hold infinity: "certainly larger", they change nothing)
       if (!two) {   // (uniform over the half-warp) the common case: one round, candidates 0..n-1
         for (int l = 0; l < nl; ++l) {
           const float od = __shfl_sync(gmask, ds0, l, 16);     // (a shuffle is a pass of the L1 data pipe: send one value)
-          const float ol = od * (1.0f - 1.0e-5f), oh = od * (1.0f + 1.0e-5f);
+          const float ol = screen_lo(od), oh = screen_hi(od);
           rank0 += oh < lo0;                                   // certainly smaller
           amb0 |= (l != sub) && !(oh < lo0) && !(hi0 < ol);    // intervals overlap
         }
       } else {
+        // (raw od < ds ranks like the intervals wherever they are disjoint, as lo <= ds <= hi; every pair where they
+        // overlap is ambiguous and re-ranked below)
         for (int l = 0; l < 16; ++l) {
           const float od = __shfl_sync(gmask, ds0, l, 16);
-          const float ol = od * (1.0f - 1.0e-5f), oh = od * (1.0f + 1.0e-5f);
+          const float ol = screen_lo(od), oh = screen_hi(od);
           rank0 += od < ds0;
           amb0 |= (l != sub) && !(oh < lo0) && !(hi0 < ol);
           rank1 += od < ds1;
@@ -664,7 +675,7 @@ knn_rerank_kernel(const float* __restrict__ desc_src, const float* __restrict__ 
         }
         for (int l = 0; l < 16; ++l) {
           const float od = __shfl_sync(gmask, ds1, l, 16);
-          const float ol = od * (1.0f - 1.0e-5f), oh = od * (1.0f + 1.0e-5f);
+          const float ol = screen_lo(od), oh = screen_hi(od);
           rank0 += od < ds0;
           amb0 |= !(oh < lo0) && !(hi0 < ol);
           rank1 += od < ds1;
@@ -736,66 +747,112 @@ __global__ void labels_from_best_kernel(const unsigned long long* __restrict__ b
   if (i < n) labels[i] = (int32_t)(best64[i] & 0xffffffffu);
 }
 
-// brute force for the (rare) tasks whose candidate lists overflowed: one block per task
+// brute force of one (query, cell) task by the whole block (128 threads); fb_d: [T] doubles of shared memory
+template <int KC>
+__device__ void fallback_task(const float* __restrict__ desc_src, const float* __restrict__ desc_tgt, const KnnTcGeom& g,
+                              int pix, int ci, int cj, double* fb_d, int32_t* __restrict__ pvec, float* __restrict__ lcost,
+                              int32_t* __restrict__ knn_idx, unsigned long long* __restrict__ best64) {
+  __shared__ double red_d[4];
+  __shared__ int red_i[4];
+  const int qy = pix / g.W, qx = pix - qy * g.W;
+  const float* q = desc_src + (size_t)pix * kDescDim;
+  const int ty0 = cj * g.cellh, tx0 = ci * g.cellw;
+  __syncthreads();
+  for (int i = threadIdx.x; i < g.T; i += blockDim.x) {
+    const int r = i / g.cellw, c = i - r * g.cellw;
+    fb_d[i] = exact_dist(q, desc_tgt + ((size_t)(ty0 + r) * g.W + tx0 + c) * kDescDim);
+  }
+  __syncthreads();
+  int cimin, cimax, cjmin, cjmax;
+  cell_range(qx, g.cellw, g.ncellx, g.R, &cimin, &cimax);
+  cell_range(qy, g.cellh, g.ncelly, g.R, &cjmin, &cjmax);
+  const int blk = (ci - cimin) * (cjmax - cjmin + 1) + (cj - cjmin);
+  for (int rank = 0; rank < KC; ++rank) {
+    double bd = CUDART_INF;
+    int bi = 0x7fffffff;
+    for (int i = threadIdx.x; i < g.T; i += blockDim.x)
+      if (fb_d[i] < bd) {     // ascending i: strict < keeps the lowest index
+        bd = fb_d[i];
+        bi = i;
+      }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+      const double od = __shfl_xor_sync(0xffffffffu, bd, off);
+      const int oi = __shfl_xor_sync(0xffffffffu, bi, off);
+      if (od < bd || (od == bd && oi < bi)) {
+        bd = od;
+        bi = oi;
+      }
+    }
+    if ((threadIdx.x & 31) == 0) {
+      red_d[threadIdx.x >> 5] = bd;
+      red_i[threadIdx.x >> 5] = bi;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      for (int w = 1; w < 4; ++w)
+        if (red_d[w] < bd || (red_d[w] == bd && red_i[w] < bi)) {
+          bd = red_d[w];
+          bi = red_i[w];
+        }
+      fb_d[bi] = CUDART_INF;
+      emit_proposal<KC>(g, q, desc_tgt, qx, qy, ci, cj, blk, rank, bi, pvec, lcost, knn_idx, best64);
+    }
+    __syncthreads();
+  }
+}
+
+// Brute force for the (rare) tasks whose candidate lists overflowed (cand_cnt == 255), one block per task.  The
+// re-rank lists up to fb_cap of them.  When more overflowed (*fb_count > fb_cap: large flat regions, where every query
+// ties with every target of a flat cell), the list is incomplete, and the blocks find every overflowed task by scanning
+// cand_cnt instead: no task is dropped, and the workspace does not grow with the worst case.
 template <int KC>
 __global__ void __launch_bounds__(128)
 knn_fallback_kernel(const float* __restrict__ desc_src, const float* __restrict__ desc_tgt, KnnTcGeom g,
-                    const int32_t* __restrict__ fb_list, const int32_t* __restrict__ fb_count, int fb_cap,
-                    int32_t* __restrict__ pvec, float* __restrict__ lcost, int32_t* __restrict__ knn_idx,
-                    unsigned long long* __restrict__ best64) {
+                    const uint8_t* __restrict__ cand_cnt, const int32_t* __restrict__ fb_list,
+                    const int32_t* __restrict__ fb_count, int fb_cap, int32_t* __restrict__ pvec,
+                    float* __restrict__ lcost, int32_t* __restrict__ knn_idx, unsigned long long* __restrict__ best64) {
   extern __shared__ double fb_d[];       // [T]
-  __shared__ double red_d[4];
-  __shared__ int red_i[4];
-  const int ntask = min(*fb_count, fb_cap);
-  for (int t = blockIdx.x; t < ntask; t += gridDim.x) {
-    const int pix = fb_list[2 * t], cell = fb_list[2 * t + 1];
-    const int qy = pix / g.W, qx = pix - qy * g.W;
-    const int ci = cell % g.ncellx, cj = cell / g.ncellx;
-    const float* q = desc_src + (size_t)pix * kDescDim;
-    const int ty0 = cj * g.cellh, tx0 = ci * g.cellw;
+  const int count = *fb_count;
+  if (count <= fb_cap) {
+    for (int t = blockIdx.x; t < count; t += gridDim.x) {
+      const int cell = fb_list[2 * t + 1];
+      fallback_task<KC>(desc_src, desc_tgt, g, fb_list[2 * t], cell % g.ncellx, cell / g.ncellx, fb_d, pvec, lcost,
+                        knn_idx, best64);
+    }
+    return;
+  }
+  __shared__ int hit_pix[128], hit_ci[128], hit_cj[128];
+  __shared__ int nhit;
+  const size_t ntask = (size_t)g.H * g.W * g.nblk;
+  for (size_t base = (size_t)blockIdx.x * blockDim.x; base < ntask; base += (size_t)gridDim.x * blockDim.x) {
+    const size_t task = base + threadIdx.x;
+    __syncthreads();                     // the previous chunk's hits are consumed
+    if (threadIdx.x == 0) nhit = 0;
     __syncthreads();
-    for (int i = threadIdx.x; i < g.T; i += blockDim.x) {
-      const int r = i / g.cellw, c = i - r * g.cellw;
-      fb_d[i] = exact_dist(q, desc_tgt + ((size_t)(ty0 + r) * g.W + tx0 + c) * kDescDim);
+    // cand_cnt holds no value for tasks past a pixel's cell window (which is empty for a pixel of the remainder strip
+    // when R = 0) or of cells outside [cx0, cx1): those are skipped before their block number is decoded
+    if (task < ntask && cand_cnt[task] == 255) {
+      const int pix = (int)(task / g.nblk), blk = (int)(task - (size_t)pix * g.nblk);
+      const int qy = pix / g.W, qx = pix - qy * g.W;
+      int cimin, cimax, cjmin, cjmax;
+      cell_range(qx, g.cellw, g.ncellx, g.R, &cimin, &cimax);
+      cell_range(qy, g.cellh, g.ncelly, g.R, &cjmin, &cjmax);
+      const int nbx = cimax - cimin + 1, nby = cjmax - cjmin + 1;
+      if (nbx > 0 && nby > 0 && blk < nbx * nby) {
+        const int ci = cimin + blk / nby, cj = cjmin + blk % nby;
+        if (ci >= g.cx0 && ci < g.cx1) {
+          const int h = atomicAdd(&nhit, 1);
+          hit_pix[h] = pix;
+          hit_ci[h] = ci;
+          hit_cj[h] = cj;
+        }
+      }
     }
     __syncthreads();
-    int cimin, cimax, cjmin, cjmax;
-    cell_range(qx, g.cellw, g.ncellx, g.R, &cimin, &cimax);
-    cell_range(qy, g.cellh, g.ncelly, g.R, &cjmin, &cjmax);
-    const int blk = (ci - cimin) * (cjmax - cjmin + 1) + (cj - cjmin);
-    for (int rank = 0; rank < KC; ++rank) {
-      double bd = CUDART_INF;
-      int bi = 0x7fffffff;
-      for (int i = threadIdx.x; i < g.T; i += blockDim.x)
-        if (fb_d[i] < bd) {     // ascending i: strict < keeps the lowest index
-          bd = fb_d[i];
-          bi = i;
-        }
-#pragma unroll
-      for (int off = 16; off > 0; off >>= 1) {
-        const double od = __shfl_xor_sync(0xffffffffu, bd, off);
-        const int oi = __shfl_xor_sync(0xffffffffu, bi, off);
-        if (od < bd || (od == bd && oi < bi)) {
-          bd = od;
-          bi = oi;
-        }
-      }
-      if ((threadIdx.x & 31) == 0) {
-        red_d[threadIdx.x >> 5] = bd;
-        red_i[threadIdx.x >> 5] = bi;
-      }
-      __syncthreads();
-      if (threadIdx.x == 0) {
-        for (int w = 1; w < 4; ++w)
-          if (red_d[w] < bd || (red_d[w] == bd && red_i[w] < bi)) {
-            bd = red_d[w];
-            bi = red_i[w];
-          }
-        fb_d[bi] = CUDART_INF;
-        emit_proposal<KC>(g, q, desc_tgt, qx, qy, ci, cj, blk, rank, bi, pvec, lcost, knn_idx, best64);
-      }
-      __syncthreads();
-    }
+    const int nh = nhit;
+    for (int h = 0; h < nh; ++h)           // (tasks write disjoint slots; best64 is an atomic minimum: any order)
+      fallback_task<KC>(desc_src, desc_tgt, g, hit_pix[h], hit_ci[h], hit_cj[h], fb_d, pvec, lcost, knn_idx, best64);
   }
 }
 
@@ -936,8 +993,8 @@ static int run_tc(const float* desc_src, const float* desc_tgt, const flowb200_p
   auto fkern = knn_fallback_kernel<KC>;
   const size_t fsmem = (size_t)g.T * sizeof(double);
   if (fsmem > 48 * 1024) FB_CUDA_CHECK(cudaFuncSetAttribute(fkern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsmem));
-  fkern<<<4 * kNumSMs, 128, fsmem, stream>>>(desc_src, desc_tgt, g, fb_list, fb_count, L.fb_cap, pvec, lcost, knn_idx,
-                                                   best64);
+  fkern<<<4 * kNumSMs, 128, fsmem, stream>>>(desc_src, desc_tgt, g, cnt, fb_list, fb_count, L.fb_cap, pvec, lcost,
+                                             knn_idx, best64);
   FB_LAUNCH_CHECK();
   labels_from_best_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(best64, labels, (int)n);
   FB_LAUNCH_CHECK();
