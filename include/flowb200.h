@@ -44,7 +44,7 @@ enum {
  *   FP64_F32COST / FP64_F64COST: float64 dynamic programme with the reference's operation order,
  *       bit-exact labels for arbitrary data costs (cost array float32 resp. float64);
  *   INT32: int32 dynamic programme in units of 2^-cost_shift on integer data costs m
- *       (lamda*lcost*2^S == m, 0 <= m < 65536, 4 <= cost_shift <= 14); bit-exact with the reference whenever
+ *       (lamda*lcost*2^S == m, 0 <= m < 65536, 0 <= cost_shift <= 14); bit-exact with the reference whenever
  *       lcost == 20*m/2^S;
  *   INT32_F32COST: the same int32 programme fed with float32 costs, m = rint(lamda*lcost*2^S) on the fly
  *       (what flowb200_quantise_costs computes, without the extra array). */
@@ -133,10 +133,13 @@ int flowb200_quantise_costs(const float* lcost, int32_t* m, size_t n, double lam
  * Runs `sweeps` sweeps of the four phases (even columns down, even rows right-to-left, odd columns up,
  * odd rows left-to-right) on `labels` in place.  cost: float32 / float64 / int32 [H][W][K] per bcd_mode.
  * labels_per_sweep (optional): int32 [sweeps][H][W] snapshot after every sweep (what ceoBCD saves).
- * The int32 modes compile the K-sets S_l = {k : L1(v_l,u_k) < tpsi} of every (pixel, chain direction) once per call
+ * tpsi: 0..32 (larger: FLOWB200_EUNSUPPORTED); cost_shift (int32 modes): 0..14.
+ * Every mode compiles the K-sets S_l = {k : L1(v_l,u_k) < tpsi} of every (pixel, chain direction) once per call
  * into sparse records in the workspace (the reference caches them too: pakovanje, daisy i flann.py:256-309) and the
  * chains stream them; K-sets that do not fit are evaluated on the fly, so any workspace between
- * flowb200_bcd_min_workspace_bytes() and flowb200_bcd_workspace_bytes() (the recommended size) gives the same labels. */
+ * flowb200_bcd_min_workspace_bytes() and flowb200_bcd_workspace_bytes() (the recommended size) gives the same labels.
+ * Inputs outside the record format (tpsi outside 1..8, or an int32 mode with cost_shift < 4) get no records: every
+ * step is evaluated on the fly. */
 size_t flowb200_bcd_workspace_bytes(int H, int W, int K);
 size_t flowb200_bcd_min_workspace_bytes(int H, int W, int K);
 int flowb200_bcd(const int32_t* pvec, const void* cost, const int32_t* nprop, int32_t* labels,

@@ -1,6 +1,11 @@
-// BCD with compiled K-sets: the int32 programme of bcd.cu restructured around what the reference itself does --
-// it evaluates the K-sets S_l = {k : L1(v_l, u_k) < tpsi} ONCE per proposal set (pakovanje, daisy i flann.py:256-309,
-// the 2.6 GB packedksets cache) and only reads them inside bcd() (python bcd.py:131-142).  Here the cache is sparse:
+// Block-coordinate-descent MRF inference: row/column chain Viterbi over the K proposal labels.
+// Reference: `python bcd.py` bcd() :101-257 (one chain), ceoBCD() :261-284 (phase order), sidepsi :84-88; see
+// oracle/bcd.py for the recurrence in words.  Arithmetic modes (include/flowb200.h): float64 with the reference's
+// operation order, or uint32 in units of 2^-S.
+//
+// It is organised around what the reference itself does -- it evaluates the K-sets S_l = {k : L1(v_l, u_k) < tpsi}
+// ONCE per proposal set (pakovanje, daisy i flann.py:256-309, the 2.6 GB packedksets cache) and only reads them inside
+// bcd() (python bcd.py:131-142).  Here the cache is sparse:
 //
 //   kset_sort_kernel   per pixel: label indices (and vectors) ordered by the spatial-hash bucket of the flow vector
 //   kset_build_kernel  per (pixel, chain orientation): one RECORD = everything a chain step needs, contiguous (layout
@@ -22,18 +27,56 @@
 // A record that does not fit (arena exhausted, staging or slot too small, list longer than 124, data cost out of 16
 // bits) gets descriptor 0 and
 // its step is evaluated densely from pvec/cost inside the chain kernel, so any workspace size gives the exact result.
+// Records are built for tpsi 1..8 (an entry holds L1 in 3 bits) and, in the int32 modes, cost shifts 4..14.  Other
+// inputs (tpsi 0 or 9..32, cost shift 0..3) get no records: every descriptor is 0 and every step is evaluated densely.
 // Precondition of the int32 modes: 0 <= m < 65536 for every used slot (the uint32 dp bound of make_plan assumes it).
 #include <math_constants.h>
 
 #include <algorithm>
 #include <type_traits>
 
-#include "bcd_common.cuh"
+#include "common.cuh"
 #include "sm100_ptx.cuh"
 
 namespace flowb200 {
 
 namespace {
+
+struct ChainGeom {
+  int sy, sx, ystep, xstep, len;
+};
+
+__device__ __forceinline__ ChainGeom chain_geom(int phase, int c, int H, int W) {
+  ChainGeom g;
+  switch (phase) {
+    case 0: g = {0, 2 * c, 1, 0, H}; break;           // even columns, downwards   (:265-266)
+    case 1: g = {2 * c, W - 1, 0, -1, W}; break;      // even rows, right to left  (:270-271)
+    case 2: g = {H - 1, 2 * c + 1, -1, 0, H}; break;  // odd columns, upwards      (:273-274)
+    default: g = {2 * c + 1, 0, 0, 1, W}; break;      // odd rows, left to right   (:276-277)
+  }
+  return g;
+}
+
+int phase_chains(int phase, int H, int W) {
+  switch (phase) {
+    case 0: return (W + 1) / 2;
+    case 1: return (H + 1) / 2;
+    case 2: return W / 2;
+    default: return H / 2;
+  }
+}
+
+// Spatial hash of flow vectors: bucket edge 2^bshift >= tpsi, 16 x 64 buckets (offset and clamped), so that every
+// u with L1(v, u) < tpsi lies in the 3 x 3 buckets around v's bucket.
+constexpr int kHashY = 16, kHashX = 64, kHashSize = kHashY * kHashX;
+// bucket coordinates are offset and clamped (not wrapped) so that buckets adjacent in x have consecutive keys:
+// the labels of three x-adjacent buckets form ONE contiguous range.  Clamping merges far-away buckets into the
+// border ones, which is harmless because membership is always decided by the exact L1 test.
+__device__ __forceinline__ int bkt_y(int b) { return min(max(b + kHashY / 2, 0), kHashY - 1); }
+__device__ __forceinline__ int bkt_x(int b) { return min(max(b + kHashX / 2, 0), kHashX - 1); }
+__device__ __forceinline__ int bucket_key(int32_t v, int bshift) {
+  return (bkt_y(vec_dy(v) >> bshift) << 6) | bkt_x(vec_dx(v) >> bshift);
+}
 
 constexpr uint32_t kRngEmpty = 0x0000FFFFu;   // first = 0xFFFF, last+1 = 0
 constexpr int kRecHeader = 16;
@@ -1086,11 +1129,6 @@ KsetLayout kset_layout(int H, int W, int K, size_t workspace_bytes) {
   return L;
 }
 
-}  // namespace
-
-size_t ksets_workspace_bytes(int H, int W, int K) { return kset_layout(H, W, K, 0).total; }
-size_t ksets_min_workspace_bytes(int H, int W, int K) { return kset_layout(H, W, K, 0).arena; }
-
 // chains [c0, c1) of `phase` that part `part` of `nparts` owns (single-huge-image mode: a phase's independent chains
 // are split over the GPUs, python bcd.py:265-277 makes every chain of a phase independent of the others)
 static inline void owned_chains(int phase, int H, int W, int part, int nparts, int* c0, int* c1) {
@@ -1108,6 +1146,7 @@ struct KsetPlan {
   void (*kern64)(const ChainArgs) = nullptr;   // the chains the first could not certify
   void (*kernf64)(const ChainArgs) = nullptr;  // the float64 programme (every chain)
   int T = 0, bshift = 0, slot_shift = 2, minb = 1;
+  bool records = false;   // false: no record is built, every step is evaluated densely
   uint32_t slot_bytes = 0;
   size_t smem32[2] = {0, 0}, smem64 = 0;   // smem32: by chain orientation (column chains are H long, row chains W)
 };
@@ -1115,7 +1154,8 @@ struct KsetPlan {
 // shift < 0 selects the float64 programme (kset_chainf64_kernel): the records then carry no data costs
 template <typename CostT>
 static int make_plan(int H, int W, int K, int tpsi, int shift, size_t workspace_bytes, KsetPlan<CostT>* P) {
-  if (K > 512 || tpsi < 1 || tpsi > 8) return FLOWB200_EUNSUPPORTED;
+  if (K > 512 || tpsi < 0 || tpsi > 32) return FLOWB200_EUNSUPPORTED;
+  P->records = tpsi >= 1 && tpsi <= 8 && (shift < 0 || shift >= 4);
   if (shift >= 0) {   // dp is a uint32
     const unsigned long long per_step = ((unsigned long long)(3 * tpsi) << shift) + 65535ull;
     if ((unsigned long long)(H > W ? H : W) * per_step >= 0xFFFF0000ull) return FLOWB200_EUNSUPPORTED;
@@ -1176,6 +1216,10 @@ int ksets_prepare(const int32_t* pvec, const CostT* cost, const int32_t* nprop, 
   const KsetLayout& L = P.L;
   char* ws = static_cast<char*>(workspace);
   const int npix = H * W;
+  if (!P.records) {   // every descriptor 0: the chain kernels evaluate every step densely
+    FB_CUDA_CHECK(cudaMemsetAsync(ws + L.desc, 0, 2 * (size_t)npix * sizeof(unsigned long long), stream));
+    return FLOWB200_OK;
+  }
   uint16_t* sorig = reinterpret_cast<uint16_t*>(ws + L.sorig);
   unsigned long long* cursor = reinterpret_cast<unsigned long long*>(ws + L.cursor);
   FB_CUDA_CHECK(cudaMemsetAsync(cursor, 0, sizeof(unsigned long long), stream));
@@ -1262,16 +1306,91 @@ int launch_sweeps_ksets(const int32_t* pvec, const CostT* cost, const int32_t* n
   return FLOWB200_OK;
 }
 
-#define FB_KS_INSTANTIATE(CT)                                                                                          \
-  template int launch_sweeps_ksets<CT>(const int32_t*, const CT*, const int32_t*, int32_t*, int, int, int, double, int, \
-                                       int, int, int32_t*, void*, size_t, cudaStream_t);                               \
-  template int ksets_prepare<CT>(const int32_t*, const CT*, const int32_t*, int, int, int, double, int, int, int, int,  \
-                                 void*, size_t, cudaStream_t);                                                         \
-  template int ksets_phase<CT>(const int32_t*, const CT*, const int32_t*, int32_t*, int, int, int, double, int, int,    \
-                               int, int, int, void*, size_t, cudaStream_t);
-FB_KS_INSTANTIATE(int32_t)
-FB_KS_INSTANTIATE(float)
-FB_KS_INSTANTIATE(double)
-#undef FB_KS_INSTANTIATE
+bool is_int_mode(int bcd_mode) { return bcd_mode == FLOWB200_BCD_INT32 || bcd_mode == FLOWB200_BCD_INT32_F32COST; }
+
+// run(cost, shift) with the cost array typed for bcd_mode; shift -1 selects the float64 programme
+template <typename Run>
+int with_mode(int bcd_mode, const void* cost, int cost_shift, Run run) {
+  switch (bcd_mode) {
+    case FLOWB200_BCD_FP64_F32COST: return run(static_cast<const float*>(cost), -1);
+    case FLOWB200_BCD_FP64_F64COST: return run(static_cast<const double*>(cost), -1);
+    case FLOWB200_BCD_INT32: return run(static_cast<const int32_t*>(cost), cost_shift);
+    case FLOWB200_BCD_INT32_F32COST: return run(static_cast<const float*>(cost), cost_shift);
+    default: return FLOWB200_EINVAL;
+  }
+}
+
+}  // namespace
+
+__global__ void quantise_costs_kernel(const float* __restrict__ lcost, int32_t* __restrict__ m, size_t n, double lamda,
+                                      double scale) {
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  float c = lcost[i];
+  m[i] = (c == FLOWB200_UNUSED_COST) ? 0 : (int32_t)rint(__dmul_rn(__dmul_rn(lamda, (double)c), scale));
+}
 
 }  // namespace flowb200
+
+using namespace flowb200;
+
+extern "C" size_t flowb200_bcd_workspace_bytes(int H, int W, int K) {
+  if (H <= 0 || W <= 0 || K <= 0) return 0;
+  return kset_layout(H, W, K, 0).total;
+}
+
+// fixed part only: every K-set is then evaluated densely
+extern "C" size_t flowb200_bcd_min_workspace_bytes(int H, int W, int K) {
+  if (H <= 0 || W <= 0 || K <= 0) return 0;
+  return kset_layout(H, W, K, 0).arena;
+}
+
+extern "C" int flowb200_bcd(const int32_t* pvec, const void* cost, const int32_t* nprop, int32_t* labels, int H, int W,
+                            int K, int bcd_mode, double lamda, int tpsi, int cost_shift, int sweeps,
+                            int32_t* labels_per_sweep, void* workspace, size_t workspace_bytes,
+                            flowb200_stream_t stream) {
+  if (!pvec || !cost || !nprop || !labels || !workspace) return FLOWB200_EINVAL;
+  if (H <= 0 || W <= 0 || K <= 0 || K > 512 || sweeps < 0 || tpsi < 0) return FLOWB200_EINVAL;
+  if (H > 16384 || W > 16384) return FLOWB200_EINVAL;
+  if (is_int_mode(bcd_mode) && (cost_shift < 0 || cost_shift > 14)) return FLOWB200_EINVAL;
+  // any workspace that holds the fixed part is accepted: records that do not fit are evaluated densely
+  return with_mode(bcd_mode, cost, cost_shift, [&](auto c, int shift) {
+    return launch_sweeps_ksets(pvec, c, nprop, labels, H, W, K, lamda, tpsi, shift, sweeps, labels_per_sweep, workspace,
+                               workspace_bytes, stream);
+  });
+}
+
+// ---- the K-set programme in pieces: one part of every phase's chains (single-huge-image mode) ----
+extern "C" int flowb200_bcd_prepare(const int32_t* pvec, const void* cost, const int32_t* nprop, int H, int W, int K,
+                                    int bcd_mode, double lamda, int tpsi, int cost_shift, int part, int nparts,
+                                    void* workspace, size_t workspace_bytes, flowb200_stream_t stream) {
+  if (!pvec || !cost || !nprop || !workspace) return FLOWB200_EINVAL;
+  if (H <= 0 || W <= 0 || K <= 0 || K > 512 || H > 16384 || W > 16384) return FLOWB200_EINVAL;
+  if (cost_shift < 0 || cost_shift > 14) return FLOWB200_EINVAL;
+  if (!is_int_mode(bcd_mode)) return FLOWB200_EUNSUPPORTED;
+  return with_mode(bcd_mode, cost, cost_shift, [&](auto c, int shift) {
+    return ksets_prepare(pvec, c, nprop, H, W, K, lamda, tpsi, shift, part, nparts, workspace, workspace_bytes, stream);
+  });
+}
+
+extern "C" int flowb200_bcd_phase(const int32_t* pvec, const void* cost, const int32_t* nprop, int32_t* labels, int H,
+                                  int W, int K, int bcd_mode, double lamda, int tpsi, int cost_shift, int phase, int part,
+                                  int nparts, void* workspace, size_t workspace_bytes, flowb200_stream_t stream) {
+  if (!pvec || !cost || !nprop || !labels || !workspace) return FLOWB200_EINVAL;
+  if (H <= 0 || W <= 0 || K <= 0 || K > 512 || H > 16384 || W > 16384) return FLOWB200_EINVAL;
+  if (cost_shift < 0 || cost_shift > 14) return FLOWB200_EINVAL;
+  if (!is_int_mode(bcd_mode)) return FLOWB200_EUNSUPPORTED;
+  return with_mode(bcd_mode, cost, cost_shift, [&](auto c, int shift) {
+    return ksets_phase(pvec, c, nprop, labels, H, W, K, lamda, tpsi, shift, phase, part, nparts, workspace,
+                       workspace_bytes, stream);
+  });
+}
+
+extern "C" int flowb200_quantise_costs(const float* lcost, int32_t* m, size_t n, double lamda, int shift,
+                                       flowb200_stream_t stream) {
+  if (!lcost || !m || shift < 0 || shift > 14) return FLOWB200_EINVAL;
+  if (n == 0) return FLOWB200_OK;
+  quantise_costs_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(lcost, m, n, lamda, (double)(1 << shift));
+  FB_LAUNCH_CHECK();
+  return FLOWB200_OK;
+}

@@ -1,11 +1,11 @@
-"""Full-size (BASELINE.json configs[1]: 1024x436, K=300) checks through properties that do not need the CPU oracle
-(the oracle comparisons at this size are in test_gpu_baseline_configs.py; they take minutes, these take seconds):
+"""Full-size (BASELINE.json configs[1]: 1024x436, K=300) checks, mostly through properties that do not need the CPU
+oracle (the stage-by-stage oracle comparisons at this size are in test_gpu_baseline_configs.py; they take minutes):
 
 * the tcgen05 search equals an independent float64 brute force (torch) on sampled (pixel, cell) tasks, and every
   block of k proposals is sorted by distance;
-* the K-set BCD (bcd_ksets.cu: int32 programme and float64 programme) and the first implementation (bcd.cu, K-sets
-  re-evaluated on the fly, FLOWB200_BCD_LEGACY) -- independent code -- give identical labels after every sweep on costs
-  quantised to 20*m/2^12, and the K-set BCD does not depend on how much of the record cache fits the workspace;
+* the two BCD programmes (bcd_ksets.cu: int32 and float64) give the C oracle's labels after every sweep on costs
+  quantised to 20*m/2^12 (the oracle's two sweeps take about 30 s on 8 host threads), and the int32 programme does not
+  depend on how much of the record cache fits the workspace;
 * the consistency check is idempotent.
 """
 import numpy as np
@@ -55,22 +55,23 @@ def test_search_equals_float64_brute_force_on_sampled_tasks(stage1):
         assert torch.equal(dy.long(), cj * p.cellh + got // p.cellw - y) and torch.equal(dx.long(), ci * p.cellw + got % p.cellw - x)
 
 
-def test_two_bcd_implementations_agree_and_cache_size_does_not_matter(stage1, monkeypatch):
-    ops, lib = pkg("ops"), pkg("_lib")
+def test_two_bcd_implementations_agree_and_cache_size_does_not_matter(stage1):
+    from oracle import cport
+    ops, lib, ioc = pkg("ops"), pkg("_lib"), pkg("io_contract")
     p, d1, d2, pvec, lcost, nprop, labels, _ = stage1
     pv, lc, npr = pvec.clone(), lcost.clone(), nprop.clone()
     ops.random_proposals(d1, d2, p, pv, lc, npr, labels, seed=3)
     m = ops.quantise_costs(lc, p.lamda, 12)
     lq = (m.double() * (20.0 / 4096.0))
     lq = torch.where(lc == 1000.0, torch.full_like(lq, 1000.0), lq)
-    a, b = labels.clone(), labels.clone()
-    sa = ops.bcd(pv, m, npr, a, 2, mode=lib.BCD_INT32, cost_shift=12, per_sweep=True)
-    monkeypatch.setenv("FLOWB200_BCD_LEGACY", "1")
-    sb = ops.bcd(pv, lq, npr, b, 2, mode=lib.BCD_FP64_F64COST, per_sweep=True)
-    monkeypatch.delenv("FLOWB200_BCD_LEGACY")
-    assert torch.equal(sa, sb)
-    sc = ops.bcd(pv, lq, npr, labels.clone(), 2, mode=lib.BCD_FP64_F64COST, per_sweep=True)   # float64 programme on K-sets
-    assert torch.equal(sc, sb)
+    want = np.stack(cport.ceo_bcd(ioc.unpack_proposals(pv.cpu().numpy()), lq.cpu().numpy(), npr.cpu().numpy(),
+                                  labels.cpu().numpy(), 2))
+    a = labels.clone()
+    sa = ops.bcd(pv, m, npr, a, 2, mode=lib.BCD_INT32, cost_shift=12, per_sweep=True).cpu().numpy()
+    sb = ops.bcd(pv, lq, npr, labels.clone(), 2, mode=lib.BCD_FP64_F64COST, per_sweep=True).cpu().numpy()
+    for w in range(2):
+        assert np.array_equal(sa[w], want[w]), ("int32", w, float((sa[w] != want[w]).mean()))
+        assert np.array_equal(sb[w], want[w]), ("float64", w, float((sb[w] != want[w]).mean()))
     assert float((a != labels).float().mean()) > 0.05          # the sweeps did something
     c = labels.clone()
     L = lib.load()

@@ -271,9 +271,13 @@ def test_bcd_int32_golden():
         assert np.array_equal(snaps[w], z[f"labels{w + 1:02d}"]), w
 
 
-@pytest.mark.parametrize("H,W,K", [(37, 41, 150), (36, 64, 300), (48, 40, 500), (1, 40, 60), (40, 1, 60), (2, 2, 33)])
-def test_bcd_vs_oracle_random(H, W, K):
-    """Random proposal sets incl. degenerate shapes, ragged nprop, heavy ties (int costs), K up to 500."""
+@pytest.mark.parametrize("H,W,K,tpsi,shift", [
+    pytest.param(H, W, K, 8, 12, id=f"{H}-{W}-{K}")
+    for H, W, K in ((37, 41, 150), (36, 64, 300), (48, 40, 500), (1, 40, 60), (40, 1, 60), (2, 2, 33))] + [
+    # other tpsi and cost shifts; tpsi 0 and 9..32 and cost shifts below 4 run without K-set records
+    (37, 41, 150, 0, 12), (20, 24, 300, 3, 12), (24, 20, 500, 12, 12), (37, 41, 150, 32, 12), (20, 24, 300, 8, 2)])
+def test_bcd_vs_oracle_random(H, W, K, tpsi, shift):
+    """Random proposal sets incl. degenerate shapes, ragged nprop, heavy ties (int costs), K up to 500, tpsi 0..32."""
     from oracle import bcd as obcd
     ops, ioc, lib = pkg("ops"), pkg("io_contract"), pkg("_lib")
     rng = np.random.default_rng(H * 1000 + W + K)
@@ -281,14 +285,18 @@ def test_bcd_vs_oracle_random(H, W, K):
     nprop = rng.integers(max(1, K // 3), K + 1, (H, W)).astype(np.int64)
     m = rng.integers(0, 513, (H, W, K)).astype(np.int64)
     lab0 = (rng.integers(0, 1 << 30, (H, W)) % nprop).astype(np.int64)
-    lq = 20.0 * m / 4096.0
-    want = obcd.ceo_bcd(prop, lq, nprop, lab0, 2)
+    lq = 20.0 * m / float(1 << shift)
+    want = obcd.ceo_bcd(prop, lq, nprop, lab0, 2, tpsi=tpsi)
     pvec = dev(ioc.pack_proposals(prop))
-    for mode, cost, kw in ((lib.BCD_INT32, dev(m, torch.int32), dict(cost_shift=12)),
+    for mode, cost, kw in ((lib.BCD_INT32, dev(m, torch.int32), dict(cost_shift=shift)),
                            (lib.BCD_FP64_F64COST, dev(lq, torch.float64), {})):
         labels = dev(lab0, torch.int32)
-        snaps = ops.bcd(pvec, cost, dev(nprop, torch.int32), labels, 2, mode=mode, per_sweep=True, **kw).cpu().numpy()
+        snaps = ops.bcd(pvec, cost, dev(nprop, torch.int32), labels, 2, mode=mode, tpsi=tpsi, per_sweep=True,
+                        **kw).cpu().numpy()
         assert np.array_equal(snaps[0], want[0]) and np.array_equal(snaps[1], want[1]), mode
+        if tpsi == 32:   # the largest tpsi accepted
+            with pytest.raises(lib.FlowB200Error, match="unsupported"):
+                ops.bcd(pvec, cost, dev(nprop, torch.int32), labels, 2, mode=mode, tpsi=33, **kw)
 
 
 @pytest.mark.parametrize("extra", [0, 40 << 10, 400 << 10])
@@ -339,10 +347,11 @@ def test_bcd_int32_generic_kernel(monkeypatch):
         assert np.array_equal(snaps[0], want[0]) and np.array_equal(snaps[1], want[1]), force
 
 
-def test_bcd_fp64_ksets_equal_legacy_and_any_workspace(monkeypatch):
+def test_bcd_fp64_ksets_equal_oracle_and_any_workspace():
     """The float64 modes run on the compiled K-sets too (what `bcd.py` uses on reference-written files).  They equal
-    the first implementation (bcd.cu, K-sets re-evaluated at every step; FLOWB200_BCD_LEGACY) after every sweep, with
-    every record stored, none (dense steps) or some, on the reference's unquantised costs."""
+    the C oracle after every sweep, with every record stored, none (dense steps) or some, on the reference's
+    unquantised costs."""
+    from oracle import cport
     ops, ioc, lib = pkg("ops"), pkg("io_contract"), pkg("_lib")
     z = load_case("pair_b")
     sweeps = 2
@@ -354,12 +363,12 @@ def test_bcd_fp64_ksets_equal_legacy_and_any_workspace(monkeypatch):
     lo, hi = L.flowb200_bcd_min_workspace_bytes(H, W, K), L.flowb200_bcd_workspace_bytes(H, W, K)
     for mode, cost in ((lib.BCD_FP64_F32COST, dev(z["b0_lcosts"], torch.float32)),
                        (lib.BCD_FP64_F64COST, dev(z["b0_lcosts"] * 1.0000001, torch.float64))):
-        monkeypatch.setenv("FLOWB200_BCD_LEGACY", "1")
-        want = ops.bcd(pvec, cost, nprop, lab0.clone(), sweeps, mode=mode, per_sweep=True)
-        monkeypatch.delenv("FLOWB200_BCD_LEGACY")
+        # the oracle gets the same costs in float64 (float32 costs widened exactly)
+        want = np.stack(cport.ceo_bcd(z["b0_proposals"], cost.double().cpu().numpy(), z["b0_nprop"], z["b0_labels00"],
+                                      sweeps))
         for nb in (None, lo, lo + (hi - lo) // 7):
             got = ops.bcd(pvec, cost, nprop, lab0.clone(), sweeps, mode=mode, per_sweep=True, workspace_bytes=nb)
-            assert torch.equal(got, want), (mode, nb)
+            assert np.array_equal(got.cpu().numpy(), want), (mode, nb)
 
 
 def test_bcd_int32_on_float_costs_equals_quantise_then_int32():

@@ -19,25 +19,23 @@ with tempfile.TemporaryDirectory() as tmp:
                    stdout=subprocess.DEVNULL)
     t1 = time.time()
     out = {}
-    for name, extra in (("ksets", {}), ("legacy", {"FLOWB200_BCD_LEGACY": "1"})):
-        code = (f"import sys, time, torch; sys.path.insert(0, {ROOT!r}); import importlib;"
-                f"st = importlib.import_module('{P}.stage2'); ops = importlib.import_module('{P}.ops');"
-                "orig = ops.bcd\n"
-                "def timed(*a, **k):\n"
-                "    torch.cuda.synchronize(); e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)\n"
-                "    e0.record(); r = orig(*a, **k); e1.record(); torch.cuda.synchronize()\n"
-                "    print('BCD_MS', e0.elapsed_time(e1), 'MODE', k.get('mode')); return r\n"
-                "ops.bcd = timed\n"
-                f"t = time.time(); st.run('6', '0', {sweeps}, log=lambda *a: None); print('RUN_S', time.time() - t)")
-        r = subprocess.run([sys.executable, "-c", code], cwd=work, env=dict(os.environ, **extra), capture_output=True,
-                           text=True, check=True)
-        for line in r.stdout.splitlines():
-            f = line.split()
-            if f and f[0] == "BCD_MS":
-                out[name + "_bcd_ms"] = round(float(f[1]), 2)
-                out["bcd_mode"] = int(f[3])
-            if f and f[0] == "RUN_S":
-                out[name + "_script_s"] = round(float(f[1]), 2)
+    code = (f"import sys, time, torch; sys.path.insert(0, {ROOT!r}); import importlib;"
+            f"st = importlib.import_module('{P}.stage2'); ops = importlib.import_module('{P}.ops');"
+            "orig = ops.bcd\n"
+            "def timed(*a, **k):\n"
+            "    torch.cuda.synchronize(); e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)\n"
+            "    e0.record(); r = orig(*a, **k); e1.record(); torch.cuda.synchronize()\n"
+            "    print('BCD_MS', e0.elapsed_time(e1), 'MODE', k.get('mode')); return r\n"
+            "ops.bcd = timed\n"
+            f"t = time.time(); st.run('6', '0', {sweeps}, log=lambda *a: None); print('RUN_S', time.time() - t)")
+    r = subprocess.run([sys.executable, "-c", code], cwd=work, capture_output=True, text=True, check=True)
+    for line in r.stdout.splitlines():
+        f = line.split()
+        if f and f[0] == "BCD_MS":
+            out["ksets_bcd_ms"] = round(float(f[1]), 2)
+            out["bcd_mode"] = int(f[3])
+        if f and f[0] == "RUN_S":
+            out["ksets_script_s"] = round(float(f[1]), 2)
     out.update(H=H, W=W, K=150, bcd_times=sweeps, stage1_script_s=round(t1 - t0, 2),
                note="bcd_mode 0 = FP64_F32COST (reference-written costs are float32 sums); script time includes np.load "
                     "of 1.7 GB of int64/float64 files and the np.save calls after every sweep")
