@@ -45,8 +45,10 @@ constexpr int kTilesPerItem = 1;                        // MMA tiles (x-adjacent
 constexpr int kChunkN = 128;       // targets per accumulator stage
 // Two passes over a cell's targets (the GEMM is recomputed; the tensor pipe is mostly idle anyway): pass 0 only
 // tracks the k smallest group minima (tau), pass 1 compares every score with the FINAL bound tau + 2 eps and
-// writes the few survivors straight to the candidate array.  No shared-memory lists, no compaction, ~3.6 issue slots
-// per score (a single-pass streaming selection with per-row lists in shared memory was built first: ~6.5).
+// writes the few survivors straight to the candidate array.  No shared-memory lists, no compaction; per 32 scores
+// pass 0 issues ~36 instructions (group minimum + list insert) and pass 1 ~54 (16 packed subtractions, 32 sign-bit
+// shifts, the mask assembly, one hit test per 128 columns) (a single-pass streaming selection with per-row lists in
+// shared memory was built first: ~6.5 issue slots per score).
 constexpr int kPasses = 2;
 #ifndef FLOWB200_KNN_CTAS
 #define FLOWB200_KNN_CTAS 3
@@ -212,6 +214,12 @@ __device__ __forceinline__ void list_insert(float (&lst)[KC], float v) {
   }
 }
 
+// bb - {x0, x1} as one packed fp32 subtraction (FADD2 on sm_100); bb holds the bound twice
+__device__ __forceinline__ void sub_f32x2(uint64_t bb, uint32_t x0, uint32_t x1, uint32_t& d0, uint32_t& d1) {
+  asm("{\n\t.reg .b64 x, d;\n\tmov.b64 x, {%2, %3};\n\tsub.rn.f32x2 d, %4, x;\n\tmov.b64 {%0, %1}, d;\n\t}"
+      : "=r"(d0), "=r"(d1) : "r"(x0), "r"(x1), "l"(bb));
+}
+
 // decode a work item; returns false when the tile lies outside the cell's query band
 __device__ __forceinline__ bool decode_item(const KnnTcGeom& g, int item, int& cell, int& qx0, int& qy0, int& x1,
                                             int& y1) {
@@ -358,7 +366,7 @@ knn_select_kernel(const __grid_constant__ CUtensorMap tmap_q, const __half* __re
         float lst[KC];
 #pragma unroll
         for (int j = 0; j < KC; ++j) lst[j] = CUDART_INF_F;
-        float bound = 0.f;
+        uint64_t bound2 = 0;   // the pass-1 bound, twice
         int ns = 0;
 
         // pass 0: one group = 32 consecutive score columns of this row; the k smallest group minima are k distinct
@@ -384,20 +392,35 @@ knn_select_kernel(const __grid_constant__ CUtensorMap tmap_q, const __half* __re
             list_insert<KC>(lst, gm);
           }
         };
-        // pass 1: every score <= the final bound is a candidate for the exact re-rank
-        auto pick = [&](const uint32_t (&r)[32], int pos0) {
-          uint32_t mask = 0;
+        // pass 1: every score x <= the final bound b is a candidate for the exact re-rank.  b is finite and not -0
+        // (the list is seeded with 16 pair minima of the first group, T >= 32 >= KC, scores are finite: padding rows
+        // score ~6e4, and eps2 >= +0), so x <= b exactly when the sign bit of RN(b - x) is clear: b - x = +0 when
+        // they are equal, rounding and overflow to +-inf keep the sign, and without .ftz nothing is flushed (the
+        // difference of two floats is never rounded to zero).  Returns bit 31 - j set when column j is ABOVE b.
+        // Four independent chains of funnel shifts gather the sign bits of 8 consecutive columns each.
+        auto above = [&](const uint32_t (&r)[32]) -> uint32_t {
+          uint32_t m[4] = {0u, 0u, 0u, 0u};
 #pragma unroll
-          for (int j = 0; j < 32; ++j) {   // set.le gives all ones / zero: one compare + one logic op per score
-            uint32_t d;
-            asm("set.le.u32.f32 %0, %1, %2;" : "=r"(d) : "f"(__uint_as_float(r[j])), "f"(bound));
-            mask |= d & (1u << j);
+          for (int j = 0; j < 32; j += 2) {
+            uint32_t d0, d1;
+            sub_f32x2(bound2, r[j], r[j + 1], d0, d1);
+            m[j >> 3] = __funnelshift_l(d0, m[j >> 3], 1);
+            m[j >> 3] = __funnelshift_l(d1, m[j >> 3], 1);
           }
-          while (mask) {
-            const int j = __ffs((int)mask) - 1;
-            mask &= mask - 1;
-            if (valid && ns < kCand) cand_row[ns] = (uint16_t)(pos0 + j);   // position; knn_rerank maps it to the index
-            ++ns;
+          return (m[0] << 24) | (m[1] << 16) | (m[2] << 8) | m[3];
+        };
+        // the candidates of one 128-column chunk, in ascending position
+        auto pick = [&](const uint32_t (&ab)[4], int cpos) {
+          if ((ab[0] & ab[1] & ab[2] & ab[3]) == 0xffffffffu) return;
+#pragma unroll
+          for (int q = 0; q < 4; ++q) {
+            uint32_t mask = __brev(~ab[q]);
+            while (mask) {
+              const int j = __ffs((int)mask) - 1;
+              mask &= mask - 1;
+              if (valid && ns < kCand) cand_row[ns] = (uint16_t)(cpos + 32 * q + j);   // position; knn_rerank maps
+              ++ns;                                                                    // it to the index
+            }
           }
         };
 
@@ -410,14 +433,14 @@ knn_select_kernel(const __grid_constant__ CUtensorMap tmap_q, const __half* __re
             ptx::tc_fence_after();
             const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (acc * kTilesPerItem + mt) * kChunkN;
             const int cpos = c * kChunkN;
-            uint32_t r0[32], r1[32];
+            uint32_t r0[32], r1[32], ab[4];
             ptx::tmem_ld_32x32(taddr, r0);
             ptx::tmem_ld_wait();
-#pragma unroll 1
+#pragma unroll
             for (int h = 0; h < kChunkN / 64; ++h) {
               ptx::tmem_ld_32x32(taddr + 64 * h + 32, r1);      // in flight while r0 is processed
               if (pass == 0) track(r0, cpos + 64 * h, c == 0 && h == 0);
-              else pick(r0, cpos + 64 * h);
+              else ab[2 * h] = above(r0);
               ptx::tmem_ld_wait();
               if (h + 1 < kChunkN / 64) {
                 ptx::tmem_ld_32x32(taddr + 64 * h + 64, r0);
@@ -427,11 +450,13 @@ knn_select_kernel(const __grid_constant__ CUtensorMap tmap_q, const __half* __re
                 if (lane == 0) ptx::mbar_arrive(&ss->t_empty[acc]);
               }
               if (pass == 0) track(r1, cpos + 64 * h + 32, false);
-              else pick(r1, cpos + 64 * h + 32);
+              else ab[2 * h + 1] = above(r1);
               ptx::tmem_ld_wait();
             }
+            if (pass == 1) pick(ab, cpos);
           }
-          bound = lst[KC - 1] + eps2;
+          const float bound = lst[KC - 1] + eps2;
+          asm("mov.b64 %0, {%1, %1};" : "=l"(bound2) : "f"(bound));
         }
         int ns_stat = 0;
         if (valid) {
