@@ -20,9 +20,9 @@
 //                      label's entry list of (dp[k] + (L1 << S), k), add the unary term, publish the new dp, one block
 //                      barrier.  dp is a uint32 in units of 2^-S; (dp, label) pairs order like np.argmin does
 //                      (python bcd.py:155/:175/:234: smallest value, lowest index on ties).
-//   kset_chain_kernel  the generic variant (64-bit keys dp << 32 | label, steps without a stored record evaluated
-//                      densely): runs only the chains that have such a step (flagged by the first kernel).
-//   kset_chainf64_kernel  the float64 programme (FLOWB200_BCD_FP64_*) on the same records.
+//   kset_chainf64_kernel  the float64 programme (FLOWB200_BCD_FP64_*) on the same records, steps without a stored
+//                      record evaluated densely.  Its integer variant runs the int32 programme, exactly, on the chains
+//                      the 32-bit kernel cannot (a step without a stored record, K = 512), which it flags.
 //
 // A record that does not fit (arena exhausted, staging or slot too small, list longer than 124, data cost out of 16
 // bits) gets descriptor 0 and
@@ -446,24 +446,6 @@ kset_build_kernel(const int32_t* __restrict__ pvec, const CostT* __restrict__ co
 // ------------------------------------------------------------------------------------------------
 // chains
 // ------------------------------------------------------------------------------------------------
-// 64-bit keys of the generic kernel: dp << 32 | label, so that "smallest dp, lowest label on ties" (np.argmin, python
-// bcd.py:155/:175/:234) is one unsigned minimum; never saturates (make_plan bounds dp below 2^32).  The 32-bit keys of
-// the main kernel are described in the header of this file.
-using Key = unsigned long long;
-constexpr Key kKeyInf = ~0ull;
-__device__ __forceinline__ Key make_key(uint32_t dp, uint32_t label) { return ((Key)dp << 32) | label; }
-__device__ __forceinline__ uint32_t key_label(Key k) { return (uint32_t)k; }
-__device__ __forceinline__ Key key_scaled(uint32_t units, int shift) { return (Key)(units << shift) << 32; }
-__device__ __forceinline__ Key key_min(Key a, Key b) { return a < b ? a : b; }
-__device__ __forceinline__ Key warp_min_key(Key k) {
-  const uint32_t hi = (uint32_t)(k >> 32), lo = (uint32_t)k;
-  const uint32_t mh = __reduce_min_sync(0xffffffffu, hi);
-  const uint32_t ml = __reduce_min_sync(0xffffffffu, hi == mh ? lo : 0xffffffffu);
-  return ((Key)mh << 32) | ml;
-}
-// byte offset of the key pair of the label an entry names, + the buffer select
-__device__ __forceinline__ uint32_t key_off64(uint32_t e, uint32_t par_off) { return ((e & 0xFF8u) << 1) | par_off; }
-
 struct ChainArgs {
   const int32_t* pvec;
   const void* cost;
@@ -472,10 +454,10 @@ struct ChainArgs {
   uint16_t* bp;
   const unsigned long long* desc;
   const unsigned char* arena;
-  int32_t* flags;     // per chain of the launch: the 32-bit kernel sets 1 when it cannot certify its result
+  int32_t* flags;     // per chain of the launch: the 32-bit kernel sets 1 when it leaves the chain to the fallback
   int H, W, K, Kpad, phase, chain0, tpsi, shift, slot_shift;   // chain = chain0 + blockIdx.x; 1 << slot_shift slots
   uint32_t slot_bytes;
-  int force_generic;  // (tests) leave every chain to the generic kernel
+  int force_generic;  // (tests) leave every chain to the fallback, the integer variant of the float64 kernel
   double lamda;
 };
 
@@ -486,7 +468,7 @@ constexpr int kMaxWarps = 16;   // T <= 512
 __host__ __device__ inline uint32_t kset_slot_bytes(int Kpad) {
   return (uint32_t)((kRecHeader + 2 * (size_t)Kpad + 8 * (size_t)Kpad + 2 * (size_t)kSlotPerLabel * Kpad + 127) & ~(size_t)127);
 }
-// dynamic shared memory of the generic kernel: oldvec int32[len] | vprev int32[Kpad] | path uint16[len] | the record
+// dynamic shared memory of the float64 kernel: oldvec int32[len] | vprev int32[Kpad] | path uint16[len] | the record
 // slots, 128-aligned
 __host__ __device__ inline size_t chain_fixed_smem(int Kpad, int len) {
   return (4 * (size_t)len + 4 * (size_t)Kpad + 2 * (size_t)len + 127) & ~(size_t)127;
@@ -527,177 +509,14 @@ __device__ __forceinline__ void backtrack(const ChainArgs& a, const ChainGeom& g
   for (int i = t; i < g.len; i += T) a.labels[(g.sy + i * g.ystep) * a.W + (g.sx + i * g.xstep)] = (int)path[i];
 }
 
-// The generic kernel (64-bit keys, steps whose record was not stored evaluated densely): runs only the chains the
-// 32-bit kernel flagged.
-template <typename CostT, int T>
-__device__ __forceinline__ void chain64_body(const ChainArgs& a) {
-  constexpr int NW = T / 32;
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  // rep_s[2 * k + b]: key of label k of the pixel visited at a step of parity b (the two buffers are interleaved so
-  // that an entry's byte offset and the buffer select combine in one logic operation)
-  __shared__ __align__(16) Key rep_s[2 * 512];
-  __shared__ Key wred[2][kMaxWarps];           // warp minima of a step (infinite for warps without labels)
-  __shared__ uint32_t present_s[4];
-  __shared__ __align__(8) uint64_t mbar[4];
-  if (a.flags[blockIdx.x] == 0) return;   // (uniform) done by the 32-bit kernel
-
-  const ChainGeom g = chain_geom(a.phase, a.chain0 + (int)blockIdx.x, a.H, a.W);
-  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
-  const int K = a.K, Kpad = a.Kpad, shift = a.shift, tpsi = a.tpsi;
-  const int S = 1 << a.slot_shift, smask = S - 1;
-  const int orient = a.phase & 1;
-  const unsigned long long* dsc = a.desc + (size_t)orient * a.H * a.W;
-  const CostT* cost = static_cast<const CostT*>(a.cost);
-
-  int32_t* oldvec = reinterpret_cast<int32_t*>(smem_raw);
-  int32_t* vprev = oldvec + g.len;
-  uint16_t* path = reinterpret_cast<uint16_t*>(vprev + Kpad);
-  unsigned char* slots = smem_raw + chain_fixed_smem(Kpad, g.len);
-
-  auto pixel = [&](int i) { return (g.sy + i * g.ystep) * a.W + (g.sx + i * g.xstep); };
-
-  for (int i = t; i < g.len; i += T) {
-    const int p = pixel(i);
-    oldvec[i] = a.pvec[(size_t)p * K + a.labels[p]];
-  }
-  if (t == 0) {
-    for (int s = 0; s < S; ++s) ptx::mbar_init(&mbar[s], 1);
-    ptx::fence_barrier_init();
-  }
-  __syncthreads();
-
-  // producer (thread 0): record i goes to slot i % S; absent records complete their barrier phase without bytes
-  unsigned long long d_next = 0;
-  auto issue = [&](int i, unsigned long long d) {
-    const int slot = i & smask;
-    const uint32_t bytes = (uint32_t)(d >> 40) << 4;
-    present_s[slot] = bytes;
-    if (bytes) {
-      ptx::mbar_arrive_expect_tx(&mbar[slot], bytes);
-      ptx::bulk_load(slots + (size_t)slot * a.slot_bytes, a.arena + ((d & ((1ull << 40) - 1)) << 4), bytes, &mbar[slot]);
-    } else {
-      ptx::mbar_arrive(&mbar[slot]);
-    }
-  };
-  if (t == 0) {
-    for (int i = 0; i < S && i < g.len; ++i) issue(i, dsc[pixel(i)]);
-    if (S < g.len) d_next = dsc[pixel(S)];
-  }
-
-  // Block minimum of a step's keys: every warp leaves the minimum of its keys in wred[parity][warp] (no atomics).  It
-  // serves the truncation candidate min_k(tpsi + dp_prev[k]), lowest k on ties (:152-157) -- read only by the labels
-  // with an empty K-set -- and the final label.
-  const Key tpsi_key = key_scaled((uint32_t)tpsi, shift);
-  auto block_min = [&](int step) -> Key {
-    const Key* w = wred[step & 1];
-    Key m = kKeyInf;
-#pragma unroll
-    for (int k = 0; k < NW; ++k) m = key_min(m, w[k]);
-    return m;
-  };
-  uint16_t* bp_row = a.bp + (size_t)blockIdx.x * g.len * Kpad;   // row of step i (advanced every step)
-  const unsigned char* rpb = reinterpret_cast<const unsigned char*>(rep_s);
-
-  for (int i = 0; i < g.len; ++i, bp_row += Kpad) {
-    const int slot = i & smask;
-    ptx::mbar_wait(&mbar[slot], (uint32_t)(i >> a.slot_shift) & 1u);
-    const uint32_t present = present_s[slot];
-    const uint32_t prv_off = (uint32_t)((i & 1) ^ 1) * (uint32_t)sizeof(Key);
-    Key* rc = rep_s + (i & 1);
-    Key key = kKeyInf;
-    const int32_t ov_a = i + 1 < g.len ? oldvec[i + 1] : 0, ov_b = i > 0 ? oldvec[i - 1] : 0;
-    // data cost + the two side terms (sidepsi :84-88: the chain's own neighbours with their labels from before this
-    // call), in units of 2^-shift
-    auto unary = [&](int dy, int dx, uint32_t m) -> uint32_t {
-      uint32_t psi = 0;
-      if (i + 1 < g.len) psi += (uint32_t)min(tpsi, l1_vec(dy, dx, ov_a));
-      if (i > 0) psi += (uint32_t)min(tpsi, l1_vec(dy, dx, ov_b));
-      return m + (psi << shift);
-    };
-    // key of this step from the minimum `acc` over the previous step's candidates
-    auto next_key = [&](Key acc, uint32_t U, uint32_t orig) -> Key {
-      return acc - key_label(acc) + ((Key)U << 32) + orig;
-    };
-    if (present) {
-      const unsigned char* rec = slots + (size_t)slot * a.slot_bytes;
-      const uint4 hdr = *reinterpret_cast<const uint4*>(rec);
-      const int n = (int)hdr.x;
-      if (t < n) {
-        const uint2 st = *reinterpret_cast<const uint2*>(rec + hdr.z + 8 * t);
-        const uint32_t pk = st.y;
-        const uint32_t orig = (pk >> 16) & 511u;
-        const uint32_t U = unary(vec_dy((int32_t)st.x), vec_dx((int32_t)st.x), pk & 0xFFFFu);
-        if (i > 0) {
-          const int ng = (int)(pk >> 25);
-          const uint32_t g0 = *reinterpret_cast<const uint16_t*>(rec + kRecHeader + 2 * t);
-          const uint2* eg = reinterpret_cast<const uint2*>(rec + hdr.w) + g0;
-          // quirk Q1: the truncation candidate only when the K-set is empty
-          Key acc = ng ? kKeyInf : block_min(i - 1) + tpsi_key;
-          for (int gi = 0; gi < ng; ++gi) {
-            const uint2 w = eg[gi];
-            const uint32_t e[4] = {w.x & 0xFFFFu, w.x >> 16, w.y & 0xFFFFu, w.y >> 16};
-#pragma unroll
-            for (int j = 0; j < 4; ++j)
-              if (!(e[j] & 0x8000u))   // (not a padding entry)
-                acc = key_min(acc, *reinterpret_cast<const Key*>(rpb + key_off64(e[j], prv_off)) + key_scaled((e[j] >> 12) & 7u, shift));
-          }
-          bp_row[orig] = (uint16_t)key_label(acc);
-          key = next_key(acc, U, orig);
-        } else {
-          key = make_key(U, orig);
-        }
-        rc[2 * orig] = key;
-      }
-    } else {
-      // dense step: the record was not stored; evaluate the K-set from the proposal arrays
-      const int p = pixel(i);
-      const int n = a.nprop[p];
-      int nq = 0;
-      if (i > 0) {
-        const int q = pixel(i - 1);
-        nq = a.nprop[q];
-        for (int k = t; k < nq; k += T) vprev[k] = a.pvec[(size_t)q * K + k];
-      }
-      __syncthreads();
-      if (t < n) {
-        const int32_t v = a.pvec[(size_t)p * K + t];
-        const int dy = vec_dy(v), dx = vec_dx(v);
-        const uint32_t U = unary(dy, dx, (uint32_t)quant_cost<CostT>(cost[(size_t)p * K + t], a.lamda, shift));
-        if (i > 0) {
-          Key acc = kKeyInf;
-          const Key* rp = rep_s + ((i & 1) ^ 1);
-          for (int k = 0; k < nq; ++k) {
-            const int l1 = l1_vec(dy, dx, vprev[k]);
-            if (l1 < tpsi) acc = key_min(acc, rp[2 * k] + key_scaled((uint32_t)l1, shift));
-          }
-          if (acc == kKeyInf) acc = block_min(i - 1) + tpsi_key;
-          bp_row[t] = (uint16_t)key_label(acc);
-          key = next_key(acc, U, (uint32_t)t);
-        } else {
-          key = make_key(U, (uint32_t)t);
-        }
-        rc[2 * t] = key;
-      }
-    }
-    {
-      const Key wmin = warp_min_key(key);
-      if (lane == 0) wred[i & 1][warp] = wmin;
-    }
-    __syncthreads();
-    if (t == 0 && i + S < g.len) {
-      issue(i + S, d_next);
-      if (i + S + 1 < g.len) d_next = dsc[pixel(i + S + 1)];
-    }
-  }
-
-  // final label: lowest-index argmin of dp_last (:231-237) = label field of the last block minimum
-  backtrack<T>(a, g, (int)key_label(block_min(g.len - 1)), path, slots, S);
-}
-
 // The float64 programme on the same records (FLOWB200_BCD_FP64_*: arbitrary data costs, the reference's own arithmetic
 // and operation order, python bcd.py:118-120, :152-176): dp is a double per label, candidates are compared as
 // (value, label) pairs -- np.argmin takes the lowest label among equal values --, and the data cost comes from the
 // cost array (the record's 16-bit cost field is unused).  One thread per label position, every chain of the launch.
+// QUANT: the int32 modes' programme on the chains the 32-bit kernel flagged (its other blocks return at once).  Every
+// term is then an integer in units of 2^-shift -- the quantised data cost (what a record's cost field holds), L1 << shift,
+// min(tpsi, L1) << shift, tpsi << shift -- and make_plan keeps dp below 2^32, so the double arithmetic is exact in any
+// order and the (value, label) compares order as the 32-bit kernel's lexicographic ones do.
 __device__ __forceinline__ void warp_argmin_f64(double& val, int& idx) {
 #pragma unroll
   for (int off = 16; off > 0; off >>= 1) {
@@ -710,7 +529,7 @@ __device__ __forceinline__ void warp_argmin_f64(double& val, int& idx) {
   }
 }
 
-template <typename CostT, int T>
+template <typename CostT, int T, bool QUANT>
 __device__ __forceinline__ void chainf64_body(const ChainArgs& a) {
   constexpr int NW = T / 32;
   constexpr int kNone = 0x7fffffff;
@@ -720,6 +539,14 @@ __device__ __forceinline__ void chainf64_body(const ChainArgs& a) {
   __shared__ int red_idx[2][kMaxWarps];             // (the sum is what the reference minimises, :152-157: it can tie where dp does not)
   __shared__ uint32_t present_s[4];
   __shared__ __align__(8) uint64_t mbar[4];
+  if constexpr (QUANT) {
+    if (a.flags[blockIdx.x] == 0) return;   // (uniform) done by the 32-bit kernel
+  }
+  // an L1 distance or tpsi in the units of dp
+  auto units = [&](auto x) {
+    if constexpr (QUANT) return x << a.shift;
+    else return x;
+  };
 
   const ChainGeom g = chain_geom(a.phase, a.chain0 + (int)blockIdx.x, a.H, a.W);
   const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
@@ -794,9 +621,11 @@ __device__ __forceinline__ void chainf64_body(const ChainArgs& a) {
     const int32_t ov_p = has_p ? oldvec[ip] : 0, ov_m = has_m ? oldvec[im] : 0;
     // dp of label `orig` (vector dy, dx) from the minimum (best, arg) over the previous step's candidates
     auto finish = [&](int dy, int dx, int orig, double best, int arg, const int p) {
-      const int psi_p = has_p ? min(tpsi, l1_vec(dy, dx, ov_p)) : 0;
-      const int psi_m = has_m ? min(tpsi, l1_vec(dy, dx, ov_m)) : 0;
-      const double lc = __dmul_rn(lamda, (double)cost[(size_t)p * K + orig]);
+      const int psi_p = has_p ? units(min(tpsi, l1_vec(dy, dx, ov_p))) : 0;
+      const int psi_m = has_m ? units(min(tpsi, l1_vec(dy, dx, ov_m))) : 0;
+      double lc;
+      if constexpr (QUANT) lc = (double)quant_cost<CostT>(cost[(size_t)p * K + orig], lamda, a.shift);
+      else lc = __dmul_rn(lamda, (double)cost[(size_t)p * K + orig]);
       if (i == 0) {   // (psi+ + psi-) + lamda*lcost   (:118-120)
         dpv = __dadd_rn((double)(psi_p + psi_m), lc);
       } else {        // (lamda*lcost + psi+) + psi-, then m + that   (:161-162, :176)
@@ -826,7 +655,7 @@ __device__ __forceinline__ void chainf64_body(const ChainArgs& a) {
             for (int j = 0; j < 4; ++j)
               if (!(e[j] & 0x8000u)) {   // (not a padding entry)
                 const int k = (int)((e[j] >> 3) & 511u);
-                const double cand = __dadd_rn(rep_s[2 * k + prv], (double)((e[j] >> 12) & 7u));
+                const double cand = __dadd_rn(rep_s[2 * k + prv], (double)units((e[j] >> 12) & 7u));
                 if (cand < best || (cand == best && k < arg)) {   // np.argmin: lowest k wins ties
                   best = cand;
                   arg = k;
@@ -855,7 +684,7 @@ __device__ __forceinline__ void chainf64_body(const ChainArgs& a) {
         for (int k = 0; k < nq; ++k) {
           const int l1 = l1_vec(dy, dx, vprev[k]);
           if (l1 < tpsi) {
-            const double cand = __dadd_rn(rep_s[2 * k + prv], (double)l1);
+            const double cand = __dadd_rn(rep_s[2 * k + prv], (double)units(l1));
             if (cand < best) {   // (k ascending: the first minimum is the lowest k)
               best = cand;
               arg = k;
@@ -868,7 +697,7 @@ __device__ __forceinline__ void chainf64_body(const ChainArgs& a) {
     last_dp = dpv;
     last_label = mine;
     {
-      double wv = __dadd_rn((double)tpsi, dpv);
+      double wv = __dadd_rn((double)units(tpsi), dpv);
       int wi = mine;
       warp_argmin_f64(wv, wi);
       if (lane == 0) {
@@ -907,7 +736,7 @@ __device__ __forceinline__ void chainf64_body(const ChainArgs& a) {
 // that the shared-memory address of an entry's dp is one logic operation on the packed entry word (mask | base |
 // buffer); the cost shift is a template parameter (12 is what the scripts and the benchmark use; 0 = run time); the
 // last warp, which has no labels or the shortest lists, streams the records.  Chains with a record that was not stored
-// are left to the generic kernel (flags[chain] = 1), which evaluates such steps densely.
+// are left to the integer variant of kset_chainf64_kernel (flags[chain] = 1), which evaluates such steps densely.
 // (Keys of (dp relative to the running minimum) << 9 | label, one unsigned minimum per entry, were built first and are
 // NOT exact: because of quirk Q1 -- no truncation candidate for a non-empty K-set, :170-176 -- whole families of labels
 // fall behind the minimum by ~16 units per step, overflow any 22-bit field within ~64 steps, and now and then catch up
@@ -1080,19 +909,23 @@ __device__ __forceinline__ void chain32_body(const ChainArgs& a) {
   backtrack<T>(a, g, (int)lab, path, slots, S);
 }
 
-template <typename CostT, int T, int MINB>
-__global__ void __launch_bounds__(T, MINB) kset_chain_kernel(const ChainArgs a) {
-  chain64_body<CostT, T>(a);
-}
-
-template <typename CostT, int T, int MINB>
+template <typename CostT, int T, int MINB, bool QUANT>
 __global__ void __launch_bounds__(T, MINB) kset_chainf64_kernel(const ChainArgs a) {
-  chainf64_body<CostT, T>(a);
+  chainf64_body<CostT, T, QUANT>(a);
 }
 
 template <typename CostT, int T, int MINB, int SHIFT>
 __global__ void __launch_bounds__(T, MINB) kset_chain32_kernel(const ChainArgs a) {
   chain32_body<CostT, T, SHIFT>(a);
+}
+
+// the variant of kset_chainf64_kernel a mode runs: the float64 programme (shift < 0) or the integer one.  Only variants
+// a mode can run are compiled: int32 costs come only with the int32 modes, double costs only with the float64 modes.
+template <typename CostT, int T>
+auto chainf64_kernel(int shift) {
+  if constexpr (std::is_integral<CostT>::value) return kset_chainf64_kernel<CostT, T, 1, true>;
+  else if constexpr (std::is_same<CostT, double>::value) return kset_chainf64_kernel<CostT, T, 1, false>;
+  else return shift < 0 ? kset_chainf64_kernel<CostT, T, 1, false> : kset_chainf64_kernel<CostT, T, 1, true>;
 }
 
 struct KsetLayout {
@@ -1143,8 +976,7 @@ struct KsetPlan {
   void (*kern32)(const ChainArgs) = nullptr;   // every chain, 32-bit dp
   void (*kern32_lo)(const ChainArgs) = nullptr;  // the same compiled for one chain per SM fewer (more registers): used
                                                  // for the orientation whose shared memory does not admit more anyway
-  void (*kern64)(const ChainArgs) = nullptr;   // the chains the first could not certify
-  void (*kernf64)(const ChainArgs) = nullptr;  // the float64 programme (every chain)
+  void (*kernf64)(const ChainArgs) = nullptr;  // float64 modes: every chain; int32 modes: the chains kern32 flagged
   int T = 0, bshift = 0, slot_shift = 2, minb = 1;
   bool records = false;   // false: no record is built, every step is evaluated densely
   uint32_t slot_bytes = 0;
@@ -1173,8 +1005,7 @@ static int make_plan(int H, int W, int K, int tpsi, int shift, size_t workspace_
     P->kern32_lo = shift == 12 ? kset_chain32_kernel<CostT, TT, (MB > 4 ? 4 : MB) - (MB >= 4 ? 1 : 0), 12>   \
                                : kset_chain32_kernel<CostT, TT, (MB > 4 ? 4 : MB) - (MB >= 4 ? 1 : 0), 0>;   \
     P->minb = MB > 4 ? 4 : MB;                                                                               \
-    P->kern64 = kset_chain_kernel<CostT, TT, 1>;                                                             \
-    P->kernf64 = kset_chainf64_kernel<CostT, TT, 1>;                                                         \
+    P->kernf64 = chainf64_kernel<CostT, TT>(shift);                                                          \
     P->T = TT;                                                                                               \
     minb = MB;                                                                                               \
   }
@@ -1187,7 +1018,7 @@ static int make_plan(int H, int W, int K, int tpsi, int shift, size_t workspace_
   const size_t fixed32 = 4096 + chain32_fixed_smem(maxlen);   // (4096: worst case of the run-time alignment pad)
   const size_t fixed64 = chain_fixed_smem(Kpad, maxlen);
   P->slot_bytes = kset_slot_bytes(Kpad);
-  // + static shared memory (32-bit kernel 0.2 KB, 64-bit kernel 8.5 KB) + the driver's 1 KB per CTA
+  // + static shared memory (32-bit kernel 0.2 KB, float64 kernel 8.5 KB) + the driver's 1 KB per CTA
   const size_t budget = (size_t)(227 * 1024) / minb - 1024 - 512;
   if (4096 + chain32_fixed_smem(H < W ? H : W) + 4 * (size_t)P->slot_bytes > budget) P->slot_shift = 1;
   // long chains (large images): fewer resident chains rather than smaller slots
@@ -1199,7 +1030,6 @@ static int make_plan(int H, int W, int K, int tpsi, int shift, size_t workspace_
     return FLOWB200_EUNSUPPORTED;
   FB_CUDA_CHECK(cudaFuncSetAttribute(P->kern32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(fixed32 + ((size_t)P->slot_bytes << P->slot_shift))));
   FB_CUDA_CHECK(cudaFuncSetAttribute(P->kern32_lo, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(fixed32 + ((size_t)P->slot_bytes << P->slot_shift))));
-  FB_CUDA_CHECK(cudaFuncSetAttribute(P->kern64, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P->smem64));
   FB_CUDA_CHECK(cudaFuncSetAttribute(P->kernf64, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P->smem64));
   return FLOWB200_OK;
 }
@@ -1269,16 +1099,14 @@ int ksets_phase(const int32_t* pvec, const CostT* cost, const int32_t* nprop, in
   a.chain0 = c0;
   a.flags = reinterpret_cast<int32_t*>(ws + L.flags);
   a.force_generic = getenv("FLOWB200_KSET_FORCE_GENERIC") != nullptr;   // read at every call (tests)
-  if (shift < 0) {   // float64 programme
-    P.kernf64<<<c1 - c0, P.T, P.smem64, stream>>>(a);
+  if (shift >= 0) {
+    // (1300: static shared memory + the driver's 1 KB per CTA)
+    const bool fits = (size_t)P.minb * (P.smem32[phase & 1] + 1300) <= (size_t)227 * 1024;
+    (fits ? P.kern32 : P.kern32_lo)<<<c1 - c0, P.T, P.smem32[phase & 1], stream>>>(a);
     FB_LAUNCH_CHECK();
-    return FLOWB200_OK;
   }
-  // (1300: static shared memory + the driver's 1 KB per CTA)
-  const bool fits = (size_t)P.minb * (P.smem32[phase & 1] + 1300) <= (size_t)227 * 1024;
-  (fits ? P.kern32 : P.kern32_lo)<<<c1 - c0, P.T, P.smem32[phase & 1], stream>>>(a);
-  FB_LAUNCH_CHECK();
-  P.kern64<<<c1 - c0, P.T, P.smem64, stream>>>(a);   // blocks of certified chains return at once
+  // int32 modes: the blocks of the chains kern32 did not flag return at once
+  P.kernf64<<<c1 - c0, P.T, P.smem64, stream>>>(a);
   FB_LAUNCH_CHECK();
   return FLOWB200_OK;
 }

@@ -36,8 +36,8 @@ def test_two_gloo_ranks(tmp_path):
         n = d.sum_over_ranks(len(units))
         json.dump({{"rank": rank, "ws": ws, "units": units, "t": t, "n": n}}, open(os.path.join({str(tmp_path)!r}, f"r{{rank}}.json"), "w"))
     """))
-    r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2",
-                        "--master-addr", "127.0.0.1", "--master-port", "29533", str(script)],
+    # --standalone: the rendezvous takes a free local port, so runs of the suite that overlap on one host do not collide
+    r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--standalone", "--nproc-per-node=2", str(script)],
                        capture_output=True, text=True, timeout=300, env=dict(os.environ, OMP_NUM_THREADS="1"))
     assert r.returncode == 0, r.stderr[-3000:]
     import json

@@ -318,12 +318,22 @@ def test_bcd_int32_any_workspace_size(extra):
 
 
 def test_bcd_int32_generic_kernel(monkeypatch):
-    """Chains that have a step without a stored record are left by the 32-bit kernel to the generic one (64-bit keys,
-    dense steps).  FLOWB200_KSET_FORCE_GENERIC sends every chain that way: the labels stay the reference's (bcd_q12
-    fixture) and the oracle's on random proposal sets with large integer costs."""
+    """Chains that have a step without a stored record are left by the 32-bit kernel to the fallback, the integer
+    variant of the float64 kernel (exact double arithmetic on the int32 terms, dense steps).
+    FLOWB200_KSET_FORCE_GENERIC sends every chain that way: the labels stay the reference's (bcd_q12 fixture); on the
+    float32 costs of pair_a they equal the unforced run's and BCD_INT32's on the quantised costs (the fallback reads
+    the data costs from the cost array, the 32-bit kernel from the records); and they are the oracle's on random
+    proposal sets with large integer costs at cost shifts 12 and 8."""
     from oracle import bcd as obcd
     ops, ioc, lib = pkg("ops"), pkg("io_contract"), pkg("_lib")
-    monkeypatch.setenv("FLOWB200_KSET_FORCE_GENERIC", "1")
+
+    def force_generic(on):
+        if on:
+            monkeypatch.setenv("FLOWB200_KSET_FORCE_GENERIC", "1")
+        else:
+            monkeypatch.delenv("FLOWB200_KSET_FORCE_GENERIC", raising=False)
+
+    force_generic(True)
     z = load_npz("bcd_q12")
     sweeps, shift = int(z["meta"][5]), int(z["meta"][6])
     labels = dev(z["labels00"], torch.int32)
@@ -331,20 +341,33 @@ def test_bcd_int32_generic_kernel(monkeypatch):
                     labels, sweeps, mode=lib.BCD_INT32, cost_shift=shift, per_sweep=True).cpu().numpy()
     for w in range(sweeps):
         assert np.array_equal(snaps[w], z[f"labels{w + 1:02d}"]), w
+
+    z = load_case("pair_a")
+    pvec = dev(ioc.pack_proposals(z["b0_proposals"]))
+    nprop = dev(z["b0_nprop"], torch.int32)
+    lc = dev(z["b0_lcosts"], torch.float32)
+    lab0 = dev(z["b0_labels00"], torch.int32)
+    forced = ops.bcd(pvec, lc, nprop, lab0.clone(), 2, mode=lib.BCD_INT32_F32COST, cost_shift=12, per_sweep=True)
+    force_generic(False)
+    unforced = ops.bcd(pvec, lc, nprop, lab0.clone(), 2, mode=lib.BCD_INT32_F32COST, cost_shift=12, per_sweep=True)
+    quantised = ops.bcd(pvec, ops.quantise_costs(lc, 0.05, 12), nprop, lab0.clone(), 2, mode=lib.BCD_INT32,
+                        cost_shift=12, per_sweep=True)
+    assert torch.equal(forced, unforced) and torch.equal(forced, quantised)
+
     rng = np.random.default_rng(5)
     H, W, K = 38, 45, 96
     prop = rng.integers(-14, 15, (H, W, K, 2)).astype(np.int64)
     nprop = rng.integers(K // 2, K + 1, (H, W)).astype(np.int64)
     m = rng.integers(0, 60000, (H, W, K)).astype(np.int64)          # near the 16-bit limit of the data cost
     lab0 = (rng.integers(0, 1 << 30, (H, W)) % nprop).astype(np.int64)
-    want = obcd.ceo_bcd(prop, 20.0 * m / 4096.0, nprop, lab0, 2)
-    for force in (True, False):
-        if not force:
-            monkeypatch.delenv("FLOWB200_KSET_FORCE_GENERIC")
-        labels = dev(lab0, torch.int32)
-        snaps = ops.bcd(dev(ioc.pack_proposals(prop)), dev(m, torch.int32), dev(nprop, torch.int32), labels, 2,
-                        mode=lib.BCD_INT32, cost_shift=12, per_sweep=True).cpu().numpy()
-        assert np.array_equal(snaps[0], want[0]) and np.array_equal(snaps[1], want[1]), force
+    for shift in (12, 8):
+        want = obcd.ceo_bcd(prop, 20.0 * m / float(1 << shift), nprop, lab0, 2)
+        for force in (True, False):
+            force_generic(force)
+            labels = dev(lab0, torch.int32)
+            snaps = ops.bcd(dev(ioc.pack_proposals(prop)), dev(m, torch.int32), dev(nprop, torch.int32), labels, 2,
+                            mode=lib.BCD_INT32, cost_shift=shift, per_sweep=True).cpu().numpy()
+            assert np.array_equal(snaps[0], want[0]) and np.array_equal(snaps[1], want[1]), (shift, force)
 
 
 def test_bcd_fp64_ksets_equal_oracle_and_any_workspace():

@@ -1,6 +1,8 @@
 """BCD stage on the bench workload, piece by piece: CUDA-event time of the K-set preparation (sort + build) and of
-every phase launch (32-bit chain kernel + the 64-bit fix-up launch behind it), and a full-size regression check of the
-labels against the C oracle (oracle/flow_oracle.c) on costs quantised to 20*m/2^S.
+every phase launch (32-bit chain kernel + the fallback launch behind it, whose blocks return at once when no chain is
+flagged), and a full-size regression check of the labels against the C oracle (oracle/flow_oracle.c) on costs quantised
+to 20*m/2^S.  Then the time of the whole call with every chain forced through the fallback (FLOWB200_KSET_FORCE_GENERIC;
+its labels must equal the unforced run's), and of the float64 programme.
    python tests/tools/bcd_phase_time.py [K] [sweeps] [H] [W]"""
 import importlib, json, os, sys
 import numpy as np, torch
@@ -24,6 +26,16 @@ kw = dict(mode=lib.BCD_INT32_F32COST, cost_shift=p.cost_shift)
 
 def ev():
     return torch.cuda.Event(enable_timing=True)
+
+
+def bcd_ms(labels, **k):
+    torch.cuda.synchronize()
+    e0, e1 = ev(), ev()
+    e0.record()
+    ops.bcd(pv, lc, npr, labels, sweeps, **k)
+    e1.record()
+    torch.cuda.synchronize()
+    return round(e0.elapsed_time(e1), 3)
 
 
 res = {}
@@ -56,12 +68,14 @@ ref = cport.ceo_bcd(ioc.unpack_proposals(pv.cpu().numpy()), lq.cpu().numpy(), np
 ok = np.array_equal(ref, l2.cpu().numpy())
 print("labels equal to the C oracle:", ok, "| moved", float((l2 != lab).float().mean()))
 assert ok
+# every chain through the int32 fallback (the variable is read at every phase call); the second run is reported
+os.environ["FLOWB200_KSET_FORCE_GENERIC"] = "1"
+for rep in range(2):
+    forced = lab.clone()
+    forced_ms = bcd_ms(forced, **kw)
+del os.environ["FLOWB200_KSET_FORCE_GENERIC"]
+assert torch.equal(forced, whole), "the forced fallback differs from the unforced run"
+print(json.dumps({"forced_fallback_total_ms": forced_ms, "sweeps": sweeps, "labels_equal_unforced": True}))
 # the float64 programme on the K-set records (what bcd.py runs on reference-written files)
 f64 = lab.clone()
-torch.cuda.synchronize()
-e0, e1 = ev(), ev()
-e0.record()
-ops.bcd(pv, lc, npr, f64, sweeps, mode=lib.BCD_FP64_F32COST)
-e1.record()
-torch.cuda.synchronize()
-print(json.dumps({"fp64_ksets_total_ms": round(e0.elapsed_time(e1), 3), "sweeps": sweeps}))
+print(json.dumps({"fp64_ksets_total_ms": bcd_ms(f64, mode=lib.BCD_FP64_F32COST), "sweeps": sweeps}))
