@@ -277,7 +277,9 @@ def test_bcd_int32_golden():
     # other tpsi and cost shifts; tpsi 0 and 9..32 and cost shifts below 4 run without K-set records
     (37, 41, 150, 0, 12), (20, 24, 300, 3, 12), (24, 20, 500, 12, 12), (37, 41, 150, 32, 12), (20, 24, 300, 8, 2)])
 def test_bcd_vs_oracle_random(H, W, K, tpsi, shift):
-    """Random proposal sets incl. degenerate shapes, ragged nprop, heavy ties (int costs), K up to 500, tpsi 0..32."""
+    """Random proposal sets incl. degenerate shapes, ragged nprop, heavy ties (int costs), K up to 500, tpsi 0..32.
+    The vectors come from a small square, so nearly every label's candidates overflow the build kernel's staging and
+    most records are not stored: this tests the dense fallback.  test_gpu_bcd_records.py tests the record path."""
     from oracle import bcd as obcd
     ops, ioc, lib = pkg("ops"), pkg("io_contract"), pkg("_lib")
     rng = np.random.default_rng(H * 1000 + W + K)
