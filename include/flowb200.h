@@ -96,8 +96,9 @@ int flowb200_daisy(const uint8_t* bgr, int H, int W, float* desc, void* workspac
  *   pvec int32 [H][W][K], lcost float32 [H][W][K], nprop int32 [H][W], labels int32 [H][W]
  *   knn_idx (optional, may be NULL): int32 [H][W][(2r+1)^2][k_cell] target index inside the cell
  *       (idx = row*cellw + col, :147-148), -1 for cells out of range; block order = slot order.
- *   stats (optional): int32[8] device counters of the tcgen05 path {tasks redone by brute force, collect-list
- *       overflows, candidate-list overflows, 0, sum of candidates handed to the re-rank, sum of collected scores}. */
+ *   stats (optional): int32[8] device counters of the tcgen05 path; slots 0..5 are written: {tasks redone by brute
+ *       force, 0, tasks whose candidate list overflowed, 0, then slots 4-5 as one uint64 (low word first): the sum of
+ *       the candidates handed to the re-rank by the tasks that did not overflow}. */
 size_t flowb200_knn_workspace_bytes(const flowb200_params* p);
 int flowb200_knn_proposals(const float* desc_src, const float* desc_tgt, const flowb200_params* p,
                            int32_t* pvec, float* lcost, int32_t* nprop, int32_t* labels, int32_t* knn_idx,

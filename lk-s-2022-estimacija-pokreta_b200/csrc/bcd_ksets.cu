@@ -218,10 +218,7 @@ __host__ __device__ inline size_t build_smem_bytes(int Kpad) {
          (size_t)kStagePerLabel * Kpad * 2;
 }
 
-#ifndef FLOWB200_BUILD_THREADS
-#define FLOWB200_BUILD_THREADS 128
-#endif
-constexpr int kBuildThreads = FLOWB200_BUILD_THREADS;
+constexpr int kBuildThreads = 128;   // 256 threads per record measured slower (DESIGN section 6)
 
 template <typename CostT>
 __global__ void __launch_bounds__(kBuildThreads)
@@ -973,7 +970,7 @@ static inline void owned_chains(int phase, int H, int W, int part, int nparts, i
 template <typename CostT>
 struct KsetPlan {
   KsetLayout L;
-  void (*kern32)(const ChainArgs) = nullptr;   // every chain, 32-bit dp
+  void (*kern32)(const ChainArgs) = nullptr;   // int32 modes: every chain, 32-bit dp; nullptr in the float64 modes
   void (*kern32_lo)(const ChainArgs) = nullptr;  // the same compiled for one chain per SM fewer (more registers): used
                                                  // for the orientation whose shared memory does not admit more anyway
   void (*kernf64)(const ChainArgs) = nullptr;  // float64 modes: every chain; int32 modes: the chains kern32 flagged
@@ -983,7 +980,9 @@ struct KsetPlan {
   size_t smem32[2] = {0, 0}, smem64 = 0;   // smem32: by chain orientation (column chains are H long, row chains W)
 };
 
-// shift < 0 selects the float64 programme (kset_chainf64_kernel): the records then carry no data costs
+// shift < 0 selects the float64 programme (kset_chainf64_kernel): the records then carry no data costs, and no 32-bit
+// chain kernel is compiled (double costs) or set up.  Dropping the 32-bit kernel's shared-memory check there changes
+// nothing: the float64 kernel's check is stricter, its left side is 4*Kpad + 128 bytes larger at every chain length
 template <typename CostT>
 static int make_plan(int H, int W, int K, int tpsi, int shift, size_t workspace_bytes, KsetPlan<CostT>* P) {
   if (K > 512 || tpsi < 0 || tpsi > 32) return FLOWB200_EUNSUPPORTED;
@@ -999,12 +998,16 @@ static int make_plan(int H, int W, int K, int tpsi, int shift, size_t workspace_
   // one thread per label position; MB = chains per SM aimed at (registers and shared memory)
   int minb = 1;
 #define FB_KS_CASE(TT, MB)                                                                                   \
-  if (!P->kern32 && K <= TT) {                                                                               \
-    P->kern32 = shift == 12 ? kset_chain32_kernel<CostT, TT, (MB > 4 ? 4 : MB), 12>                          \
-                            : kset_chain32_kernel<CostT, TT, (MB > 4 ? 4 : MB), 0>;                          \
-    P->kern32_lo = shift == 12 ? kset_chain32_kernel<CostT, TT, (MB > 4 ? 4 : MB) - (MB >= 4 ? 1 : 0), 12>   \
-                               : kset_chain32_kernel<CostT, TT, (MB > 4 ? 4 : MB) - (MB >= 4 ? 1 : 0), 0>;   \
-    P->minb = MB > 4 ? 4 : MB;                                                                               \
+  if (!P->kernf64 && K <= TT) {                                                                              \
+    constexpr int mb = MB > 4 ? 4 : MB, mb_lo = mb - (MB >= 4 ? 1 : 0);                                      \
+    if constexpr (!std::is_same<CostT, double>::value) {                                                     \
+      if (shift >= 0) {                                                                                      \
+        P->kern32 = shift == 12 ? kset_chain32_kernel<CostT, TT, mb, 12> : kset_chain32_kernel<CostT, TT, mb, 0>;\
+        P->kern32_lo = shift == 12 ? kset_chain32_kernel<CostT, TT, mb_lo, 12>                               \
+                                   : kset_chain32_kernel<CostT, TT, mb_lo, 0>;                               \
+      }                                                                                                      \
+    }                                                                                                        \
+    P->minb = mb;                                                                                            \
     P->kernf64 = chainf64_kernel<CostT, TT>(shift);                                                          \
     P->T = TT;                                                                                               \
     minb = MB;                                                                                               \
@@ -1012,24 +1015,25 @@ static int make_plan(int H, int W, int K, int tpsi, int shift, size_t workspace_
   FB_KS_CASE(64, 8) FB_KS_CASE(128, 6) FB_KS_CASE(192, 5) FB_KS_CASE(256, 4) FB_KS_CASE(320, 4)
   FB_KS_CASE(384, 3) FB_KS_CASE(512, 2)
 #undef FB_KS_CASE
-  if (!P->kern32) return FLOWB200_EUNSUPPORTED;
+  if (!P->kernf64) return FLOWB200_EUNSUPPORTED;
   // ring of record slots: as many (<= 4) as keep `minb` chains per SM resident
   const int maxlen = H > W ? H : W;
-  const size_t fixed32 = 4096 + chain32_fixed_smem(maxlen);   // (4096: worst case of the run-time alignment pad)
-  const size_t fixed64 = chain_fixed_smem(Kpad, maxlen);
   P->slot_bytes = kset_slot_bytes(Kpad);
   // + static shared memory (32-bit kernel 0.2 KB, float64 kernel 8.5 KB) + the driver's 1 KB per CTA
   const size_t budget = (size_t)(227 * 1024) / minb - 1024 - 512;
   if (4096 + chain32_fixed_smem(H < W ? H : W) + 4 * (size_t)P->slot_bytes > budget) P->slot_shift = 1;
   // long chains (large images): fewer resident chains rather than smaller slots
-  P->smem32[0] = 4096 + chain32_fixed_smem(H) + ((size_t)P->slot_bytes << P->slot_shift);
-  P->smem32[1] = 4096 + chain32_fixed_smem(W) + ((size_t)P->slot_bytes << P->slot_shift);
-  P->smem64 = fixed64 + ((size_t)P->slot_bytes << P->slot_shift);
-  if (fixed32 + ((size_t)P->slot_bytes << P->slot_shift) + 1536 > (size_t)227 * 1024 ||
-      P->smem64 + 1024 + 9216 > (size_t)227 * 1024)
-    return FLOWB200_EUNSUPPORTED;
-  FB_CUDA_CHECK(cudaFuncSetAttribute(P->kern32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(fixed32 + ((size_t)P->slot_bytes << P->slot_shift))));
-  FB_CUDA_CHECK(cudaFuncSetAttribute(P->kern32_lo, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(fixed32 + ((size_t)P->slot_bytes << P->slot_shift))));
+  const size_t slots = (size_t)P->slot_bytes << P->slot_shift;
+  P->smem32[0] = 4096 + chain32_fixed_smem(H) + slots;
+  P->smem32[1] = 4096 + chain32_fixed_smem(W) + slots;
+  P->smem64 = chain_fixed_smem(Kpad, maxlen) + slots;
+  if (P->smem64 + 1024 + 9216 > (size_t)227 * 1024) return FLOWB200_EUNSUPPORTED;
+  if (P->kern32) {   // int32 modes
+    const size_t smem32 = 4096 + chain32_fixed_smem(maxlen) + slots;   // (4096: worst case of the run-time pad)
+    if (smem32 + 1536 > (size_t)227 * 1024) return FLOWB200_EUNSUPPORTED;
+    FB_CUDA_CHECK(cudaFuncSetAttribute(P->kern32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem32));
+    FB_CUDA_CHECK(cudaFuncSetAttribute(P->kern32_lo, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem32));
+  }
   FB_CUDA_CHECK(cudaFuncSetAttribute(P->kernf64, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P->smem64));
   return FLOWB200_OK;
 }

@@ -38,10 +38,10 @@ namespace flowb200 {
 constexpr int kKP = 80;            // padded contraction depth (5 x k16)
 constexpr int kKB = 5;             // k16 blocks
 constexpr float kScale = 64.0f;    // descriptors are < ~0.5: keeps fp16 values far from subnormals
-constexpr int kTileW = 16, kTileH = 8, kTileM = 128;   // one MMA tile: 16 x 8 query pixels
-constexpr int kTilesPerItem = 1;                        // MMA tiles (x-adjacent) per work item; 2 halves the target
-                                                         // stream but leaves one CTA per SM (measured slower: the
-                                                         // selection epilogue, not the stream, bounds the kernel)
+constexpr int kTileW = 16, kTileH = 8, kTileM = 128;   // one MMA tile = one work item: 16 x 8 query pixels (two
+                                                         // tiles per item halve the target stream but leave one CTA
+                                                         // per SM: measured slower, the selection epilogue, not the
+                                                         // stream, bounds the kernel)
 constexpr int kChunkN = 128;       // targets per accumulator stage
 // Two passes over a cell's targets (the GEMM is recomputed; the tensor pipe is mostly idle anyway): pass 0 only
 // tracks the k smallest group minima (tau), pass 1 compares every score with the FINAL bound tau + 2 eps and
@@ -50,23 +50,16 @@ constexpr int kChunkN = 128;       // targets per accumulator stage
 // shifts, the mask assembly, one hit test per 128 columns) (a single-pass streaming selection with per-row lists in
 // shared memory was built first: ~6.5 issue slots per score).
 constexpr int kPasses = 2;
-#ifndef FLOWB200_KNN_CTAS
-#define FLOWB200_KNN_CTAS 3
-#endif
-#ifndef FLOWB200_KNN_BSTAGES
-#define FLOWB200_KNN_BSTAGES 2
-#endif
 // The two-pass selection needs no shared-memory lists, so more CTAs fit an SM: with ONE accumulator stage (128 TMEM
-// columns) three or four CTAs are resident and it is the other CTAs' epilogues, not a second accumulator stage of the
-// same CTA, that overlap a CTA's MMAs.
-constexpr int kCtasPerSM = FLOWB200_KNN_CTAS;
-constexpr int kBStages = FLOWB200_KNN_BSTAGES;
-constexpr int kAccStages = 1;
-constexpr int kTmemCols = kAccStages * kTilesPerItem * kChunkN;   // 128 (256 single-pass: two CTAs per SM)
+// columns) three CTAs are resident and it is the other CTAs' epilogues, not a second accumulator stage of the same
+// CTA, that overlap a CTA's MMAs (four CTAs per SM measured slower, DESIGN section 4.2).
+constexpr int kCtasPerSM = 3;
+constexpr int kBStages = 2;                              // target chunk stages in shared memory
+constexpr int kTmemCols = kChunkN;                       // the one accumulator stage: 128 columns
 constexpr int kSlabBytes = kTileM * 32;                  // one k16 block of 128 rows: 4096 B
 constexpr int kTileBytes = kKB * kSlabBytes;             // 20480 B
 constexpr int kCand = 32;          // candidates handed to the exact re-rank per (query, cell)
-constexpr int kSelThreads = 64 + 128 * kTilesPerItem;     // TMA warp, MMA warp, 4 epilogue warps per tile
+constexpr int kSelThreads = 64 + 128;                    // TMA warp, MMA warp, 4 epilogue warps
 constexpr float kPadNorm = 60000.0f;   // n_hi of padding target rows: their score can never be selected
 
 struct KnnTcGeom {
@@ -193,7 +186,7 @@ __global__ void knn_prep_target_kernel(const float* __restrict__ desc, KnnTcGeom
 struct SelSmem {
   uint64_t a_full, a_empty;
   uint64_t b_full[kBStages], b_empty[kBStages];
-  uint64_t t_full[kAccStages], t_empty[kAccStages];
+  uint64_t t_full, t_empty;   // the accumulator stage
   uint32_t tmem_base;
 };
 
@@ -234,7 +227,7 @@ __device__ __forceinline__ bool decode_item(const KnnTcGeom& g, int item, int& c
   const int x0 = max(0, g.cellw * (ci - g.R)), y0 = max(0, g.cellh * (cj - g.R));
   x1 = min(g.W, g.cellw * (ci + g.R + 1));
   y1 = min(g.H, g.cellh * (cj + g.R + 1));
-  qx0 = x0 + txi * kTileW * kTilesPerItem;
+  qx0 = x0 + txi * kTileW;
   qy0 = y0 + tyi * kTileH;
   return qx0 < x1 && qy0 < y1;
 }
@@ -247,9 +240,9 @@ knn_select_kernel(const __grid_constant__ CUtensorMap tmap_q, const __half* __re
                   int counters_on, float* __restrict__ dbg_scores) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  uint8_t* sA = smem;                                                                     // [tile][5 slabs]
-  uint8_t* sB = smem + kTileBytes * kTilesPerItem;                                         // [stage][5 slabs]
-  SelSmem* ss = reinterpret_cast<SelSmem*>(smem + kTileBytes * (kTilesPerItem + kBStages));
+  uint8_t* sA = smem;                                                                     // [5 slabs]
+  uint8_t* sB = smem + kTileBytes;                                                         // [stage][5 slabs]
+  SelSmem* ss = reinterpret_cast<SelSmem*>(smem + kTileBytes * (1 + kBStages));
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int nchunks = g.Tpad / kChunkN;
@@ -262,10 +255,8 @@ knn_select_kernel(const __grid_constant__ CUtensorMap tmap_q, const __half* __re
       ptx::mbar_init(&ss->b_full[i], 1);
       ptx::mbar_init(&ss->b_empty[i], 1);
     }
-    for (int i = 0; i < kAccStages; ++i) {
-      ptx::mbar_init(&ss->t_full[i], 1);
-      ptx::mbar_init(&ss->t_empty[i], 4 * kTilesPerItem);      // one arrival per epilogue warp
-    }
+    ptx::mbar_init(&ss->t_full, 1);
+    ptx::mbar_init(&ss->t_empty, 4);      // one arrival per epilogue warp
     ptx::fence_barrier_init();
   }
   if (warp == 1) ptx::tmem_alloc<kTmemCols>(&ss->tmem_base);
@@ -282,24 +273,17 @@ knn_select_kernel(const __grid_constant__ CUtensorMap tmap_q, const __half* __re
         int cell, qx0, qy0, x1, y1;
         if (!decode_item(g, item, cell, qx0, qy0, x1, y1)) continue;
         ptx::mbar_wait_backoff(&ss->a_empty, (it & 1) ^ 1, 2000);
-        ptx::mbar_arrive_expect_tx(&ss->a_full, kTileBytes * kTilesPerItem);
+        ptx::mbar_arrive_expect_tx(&ss->a_full, kTileBytes);
 #pragma unroll
-        for (int m = 0; m < kTilesPerItem; ++m)
-#pragma unroll
-          for (int kb = 0; kb < kKB; ++kb)
-            ptx::tma_load_3d(sA + m * kTileBytes + kb * kSlabBytes, &tmap_q, &ss->a_full, kb * 16, qx0 + m * kTileW, qy0);
+        for (int kb = 0; kb < kKB; ++kb)
+          ptx::tma_load_3d(sA + kb * kSlabBytes, &tmap_q, &ss->a_full, kb * 16, qx0, qy0);
         for (int cc = 0; cc < kPasses * nchunks; ++cc, ++bcount) {
           const int c = cc % nchunks;
           const uint32_t st = bcount % kBStages, ph = (bcount / kBStages) & 1;
           ptx::mbar_wait_backoff(&ss->b_empty[st], ph ^ 1, 100);
           ptx::mbar_arrive_expect_tx(&ss->b_full[st], kTileBytes);
-          // several smaller copies per chunk: the TMA engine overlaps independent copies but moves a single one
-          // with limited memory-level parallelism
-          constexpr int kSplit = 1, kPiece = kTileBytes / kSplit;
-          const __half* src = t16 + ((size_t)cell * nchunks + c) * (kTileBytes / 2);
-#pragma unroll
-          for (int q = 0; q < kSplit; ++q)
-            ptx::bulk_load(sB + st * kTileBytes + q * kPiece, src + q * (kPiece / 2), kPiece, &ss->b_full[st]);
+          ptx::bulk_load(sB + st * kTileBytes, t16 + ((size_t)cell * nchunks + c) * (kTileBytes / 2), kTileBytes,
+                         &ss->b_full[st]);
         }
         ++it;
       }
@@ -315,20 +299,17 @@ knn_select_kernel(const __grid_constant__ CUtensorMap tmap_q, const __half* __re
         ptx::mbar_wait_backoff(&ss->a_full, it & 1, 1000);
         for (int cc = 0; cc < kPasses * nchunks; ++cc, ++bcount) {
           const uint32_t st = bcount % kBStages, ph = (bcount / kBStages) & 1;
-          const uint32_t acc = bcount % kAccStages, aph = (bcount / kAccStages) & 1;
           ptx::mbar_wait_backoff(&ss->b_full[st], ph, 100);
-          ptx::mbar_wait_backoff(&ss->t_empty[acc], aph ^ 1, 100);
+          ptx::mbar_wait_backoff(&ss->t_empty, (bcount & 1) ^ 1, 100);
           ptx::tc_fence_after();
 #pragma unroll
-          for (int m = 0; m < kTilesPerItem; ++m)
-#pragma unroll
-            for (int kb = 0; kb < kKB; ++kb) {
-              const uint64_t da = ptx::umma_desc_k_sw32(ptx::smem_u32(sA + m * kTileBytes + kb * kSlabBytes));
-              const uint64_t db = ptx::umma_desc_k_sw32(ptx::smem_u32(sB + st * kTileBytes + kb * kSlabBytes));
-              ptx::mma_f16_ss(tmem_base + (acc * kTilesPerItem + m) * kChunkN, da, db, idesc, kb > 0 ? 1u : 0u);
-            }
+          for (int kb = 0; kb < kKB; ++kb) {
+            const uint64_t da = ptx::umma_desc_k_sw32(ptx::smem_u32(sA + kb * kSlabBytes));
+            const uint64_t db = ptx::umma_desc_k_sw32(ptx::smem_u32(sB + st * kTileBytes + kb * kSlabBytes));
+            ptx::mma_f16_ss(tmem_base, da, db, idesc, kb > 0 ? 1u : 0u);
+          }
           ptx::mma_commit(&ss->b_empty[st]);     // B stage reusable once these MMAs have read it
-          ptx::mma_commit(&ss->t_full[acc]);     // accumulator stage complete
+          ptx::mma_commit(&ss->t_full);          // accumulator stage complete
         }
         ptx::mma_commit(&ss->a_empty);           // A tile reusable
         ++it;
@@ -338,13 +319,12 @@ knn_select_kernel(const __grid_constant__ CUtensorMap tmap_q, const __half* __re
     // ===================== selection epilogue =====================
     {
       const int quad = warp & 3;                   // TMEM lane quadrant this warp may access
-      const int mt = (warp - 2) >> 2;              // which of the item's tiles this warp serves
       const int row = quad * 32 + lane;            // query row of the tile = TMEM lane
       uint32_t bcount = 0;
       for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
         int cell, qx0, qy0, x1, y1;
         if (!decode_item(g, item, cell, qx0, qy0, x1, y1)) continue;
-        const int px = qx0 + mt * kTileW + (row & (kTileW - 1)), py = qy0 + (row >> 4);
+        const int px = qx0 + (row & (kTileW - 1)), py = qy0 + (row >> 4);
         const bool valid = px < x1 && py < y1;
         const int pix = valid ? py * g.W + px : 0;
         // eps >= |a - exact score| for every target of the cell (see file header)
@@ -375,7 +355,7 @@ knn_select_kernel(const __grid_constant__ CUtensorMap tmap_q, const __half* __re
           if constexpr (DBG) {
 #pragma unroll
             for (int j = 0; j < 32; ++j)
-              dbg_scores[((size_t)(item * kTilesPerItem + mt) * kTileM + row) * g.Tpad + pos0 + j] = __uint_as_float(r[j]);
+              dbg_scores[((size_t)item * kTileM + row) * g.Tpad + pos0 + j] = __uint_as_float(r[j]);
           }
           if (first) {   // first group of the cell: 16 pair minima (distinct elements) seed the list
 #pragma unroll
@@ -425,13 +405,12 @@ knn_select_kernel(const __grid_constant__ CUtensorMap tmap_q, const __half* __re
         };
 
 #pragma unroll 1
-        for (int pass = 0; pass < 2; ++pass) {
+        for (int pass = 0; pass < kPasses; ++pass) {
 #pragma unroll 1
           for (int c = 0; c < nchunks; ++c, ++bcount) {
-            const uint32_t acc = bcount % kAccStages, aph = (bcount / kAccStages) & 1;
-            ptx::mbar_wait_backoff(&ss->t_full[acc], aph, 100);
+            ptx::mbar_wait_backoff(&ss->t_full, bcount & 1, 100);
             ptx::tc_fence_after();
-            const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (acc * kTilesPerItem + mt) * kChunkN;
+            const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16);
             const int cpos = c * kChunkN;
             uint32_t r0[32], r1[32], ab[4];
             ptx::tmem_ld_32x32(taddr, r0);
@@ -447,7 +426,7 @@ knn_select_kernel(const __grid_constant__ CUtensorMap tmap_q, const __half* __re
               } else {
                 ptx::tc_fence_before();                          // all TMEM reads of this stage are done
                 __syncwarp();
-                if (lane == 0) ptx::mbar_arrive(&ss->t_empty[acc]);
+                if (lane == 0) ptx::mbar_arrive(&ss->t_empty);
               }
               if (pass == 0) track(r1, cpos + 64 * h + 32, false);
               else ab[2 * h + 1] = above(r1);
@@ -929,7 +908,7 @@ static KnnTcGeom make_tc_geom(const flowb200_params* p) {
   g.rcp_T = g.T > 1 ? (uint32_t)((1ull << 32) / (uint64_t)g.T) : 0xffffffffu;
   g.rcp_cellw = g.cellw > 1 ? (uint32_t)((1ull << 32) / (uint64_t)g.cellw) : 0xffffffffu;
   const int r = 2 * g.R + 1;
-  g.tiles_x = (min(g.W, r * g.cellw) + kTileW * kTilesPerItem - 1) / (kTileW * kTilesPerItem);
+  g.tiles_x = (min(g.W, r * g.cellw) + kTileW - 1) / kTileW;
   g.tiles_y = (min(g.H, r * g.cellh) + kTileH - 1) / kTileH;
   g.nblk = r * r;
   g.cx0 = 0;
@@ -1003,8 +982,7 @@ static int run_tc(const float* desc_src, const float* desc_tgt, const flowb200_p
   CUtensorMap mq;
   if (!make_map(&mq, q16, (uint64_t)g.W, (uint64_t)g.H, kTileW, kTileH)) return FLOWB200_ECUDA;
   const int n_items = ncell * g.tiles_x * g.tiles_y;
-  const size_t smem = (size_t)kTileBytes * (kTilesPerItem + kBStages) +
-                      sizeof(SelSmem) + 1024;
+  const size_t smem = (size_t)kTileBytes * (1 + kBStages) + sizeof(SelSmem) + 1024;
   auto kern = dbg_scores ? knn_select_kernel<KC, true> : knn_select_kernel<KC, false>;
   FB_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int grid = min(L.grid, n_items);
@@ -1023,7 +1001,7 @@ static int run_tc(const float* desc_src, const float* desc_tgt, const flowb200_p
   FB_LAUNCH_CHECK();
   labels_from_best_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(best64, labels, (int)n);
   FB_LAUNCH_CHECK();
-  // stats: {fallback tasks, collect-list overflows, candidate-list overflows, -, sum candidates, sum collected}
+  // stats: {fallback tasks, 0, candidate-list overflows, 0, sum of candidates as one uint64 in slots 4-5}
   if (stats) FB_CUDA_CHECK(cudaMemcpyAsync(stats, fb_count, 6 * sizeof(int32_t), cudaMemcpyDeviceToDevice, stream));
   (void)p;
   return FLOWB200_OK;
@@ -1056,7 +1034,7 @@ int knn_tc_debug_scores(const float* desc_src, const float* desc_tgt, const flow
   if (geom_out_host) {
     geom_out_host[0] = g.Tpad; geom_out_host[1] = g.stride_s; geom_out_host[2] = g.tiles_x;
     geom_out_host[3] = g.tiles_y; geom_out_host[4] = g.ncellx * g.ncelly * g.tiles_x * g.tiles_y;
-    geom_out_host[5] = kTileW * kTilesPerItem; geom_out_host[6] = kTileH; geom_out_host[7] = kCand;
+    geom_out_host[5] = kTileW; geom_out_host[6] = kTileH; geom_out_host[7] = kCand;
   }
   if (!scores) return FLOWB200_OK;
   if (workspace_bytes < L.total) return FLOWB200_EWORKSPACE;

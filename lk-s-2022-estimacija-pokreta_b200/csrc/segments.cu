@@ -7,12 +7,11 @@
 //   seg_union_kernel    union-find over "valid 4-neighbours whose float32 L1 flow difference is <= tresh"
 //                       (lock-free: atomicMin on the larger root, roots are minimal scan indices)
 //   seg_flatten_kernel  root per pixel, pixels per root
-//   seg_replay_kernel   ONE warp walks the reference's scan: 32 or 128 pixels of a column per step (coalesced, ballot
-//                       for the unvisited ones), lane 0 handles the seed events in order (seg_process_seed)
+//   seg_prefilter_*     settle the seed events that cannot have an effect (segments_core.cuh)
+//   seg_replay_kernel   ONE warp walks the reference's scan: 32 pixels of a column per step (coalesced, ballot for
+//                       the unvisited ones), lane 0 handles the seed events in order (seg_process_seed)
 // HBM bound in the first three (36 B/pixel), latency bound in the replay (two dependent loads per 32 pixels and per
 // seed event); the replay is what the reference's semantics leave sequential.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "segments_core.cuh"
 #include "unionfind.cuh"
@@ -37,13 +36,6 @@ SegLayout seg_layout(int A, int B) {
   L.touch = o; o = align_up(o + n);
   L.total = o;
   return L;
-}
-
-// FLOWB200_SEG_SCAN=1|4 selects the replay's scan width (diagnostics; both give the same field and, measured, the
-// same time: the seed events bound the replay, not the scan - profiles/r01_segments_time.json)
-int seg_scan_width() {
-  const char* e = getenv("FLOWB200_SEG_SCAN");
-  return e && e[0] == '4' ? 4 : 1;
 }
 
 __global__ void seg_init_kernel(const float* __restrict__ flow, int A, int B, float2* __restrict__ fT,
@@ -78,14 +70,8 @@ __global__ void seg_flatten_kernel(int n, int32_t* parent, int32_t* __restrict__
   atomicAdd(&size[r], 1);
 }
 
-// Settle the seed events that cannot have an effect before the replay (segments_core.cuh): on by default (8.4 instead
-// of 29.7 ms on the bench workload's checked field, same valid flags: profiles/r02_segments_prefilter{0,1}.json);
-// FLOWB200_SEG_PREFILTER=0 switches it off.
-bool seg_prefilter_enabled() {
-  const char* e = getenv("FLOWB200_SEG_PREFILTER");
-  return !(e && e[0] == '0');
-}
-
+// Settle the seed events that cannot have an effect before the replay (segments_core.cuh): 8.4 instead of 29.7 ms on
+// the bench workload's checked field, same valid flags (profiles/r02_segments_prefilter{0,1}.json).
 __global__ void seg_prefilter_invalid_kernel(SegState S) {
   const int s = blockIdx.x * blockDim.x + threadIdx.x;
   if (s >= S.A * S.B) return;
@@ -100,42 +86,33 @@ __global__ void seg_prefilter_component_kernel(SegState S) {
   if (seg_component_inert(S, s)) S.cchk[s] = 1;
 }
 
-// kWide = 1: 32 pixels of the column per step.  kWide = 4: 128 pixels per step, their state loads in flight together;
-// the four ballot masks may be stale by the time a bit is reached (an earlier seed of the same step took that pixel's
-// component), so lane 0 re-tests every candidate - pixels only ever go from unvisited to visited, so a pixel absent
-// from the mask stays skipped rightly.  A removal that moves the scan to another column restarts the step there.
-template <int kWide>
+// 32 pixels of the column per step: one ballot marks the unvisited ones.  The mask may be stale by the time a bit is
+// reached (an earlier seed of the same step took that pixel's component), so lane 0 re-tests every candidate - pixels
+// only ever go from unvisited to visited, so a pixel absent from the mask stays skipped rightly.  A removal that moves
+// the scan to another column restarts the step there.  The seed events, not the scan, bound the replay: 128 pixels
+// per step measured the same time (profiles/r01_segments_time.json).
 __global__ void __launch_bounds__(32, 1) seg_replay_kernel(SegState S) {
   const unsigned lane = threadIdx.x;
   for (int bo = 0; bo < S.B; ++bo) {
     int b = bo;      // :36; may be rebound by a removal until the column scan ends (:74)
     int a = 0;       // :37
     while (a < S.A) {
-      bool open[kWide];
-#pragma unroll
-      for (int j = 0; j < kWide; ++j) {
-        const int pa = a + 32 * j + (int)lane;
-        open[j] = pa < S.A && seg_unchecked(S, b * S.A + pa);
-      }
-      unsigned m[kWide];
-#pragma unroll
-      for (int j = 0; j < kWide; ++j) m[j] = __ballot_sync(0xffffffffu, open[j]);
-      int next_a = a + 32 * kWide;
+      const int pa = a + (int)lane;
+      const bool open = pa < S.A && seg_unchecked(S, b * S.A + pa);
+      unsigned m = __ballot_sync(0xffffffffu, open);
+      int next_a = a + 32;
       bool moved = false;
-#pragma unroll
-      for (int j = 0; j < kWide; ++j) {
-        while (m[j] != 0 && !moved) {
-          const int sa = a + 32 * j + __ffs(m[j]) - 1;
-          m[j] &= m[j] - 1;
-          int nb = b;
-          if (lane == 0 && seg_unchecked(S, b * S.A + sa)) nb = seg_process_seed(S, b * S.A + sa, b);
-          __syncwarp();   // lane 0's flag updates are ordered before the next loads of all lanes
-          nb = __shfl_sync(0xffffffffu, nb, 0);
-          if (nb != b) {
-            b = nb;
-            next_a = sa + 1;
-            moved = true;
-          }
+      while (m != 0 && !moved) {
+        const int sa = a + __ffs(m) - 1;
+        m &= m - 1;
+        int nb = b;
+        if (lane == 0 && seg_unchecked(S, b * S.A + sa)) nb = seg_process_seed(S, b * S.A + sa, b);
+        __syncwarp();   // lane 0's flag updates are ordered before the next loads of all lanes
+        nb = __shfl_sync(0xffffffffu, nb, 0);
+        if (nb != b) {
+          b = nb;
+          next_a = sa + 1;
+          moved = true;
         }
       }
       a = next_a;
@@ -182,18 +159,11 @@ extern "C" int flowb200_remove_small_segments(float* flow, int A, int B, float t
   seg_init_kernel<<<G, T, 0, stream>>>(flow, A, B, fT, root, size, reinterpret_cast<uint8_t*>(ws + L.cchk), S.vis);
   seg_union_kernel<<<G, T, 0, stream>>>(fT, A, B, tresh, root);
   seg_flatten_kernel<<<G, T, 0, stream>>>(n, root, size);
-  if (seg_prefilter_enabled()) {
-    FB_CUDA_CHECK(cudaMemsetAsync(S.touch, 0, (size_t)n, stream));
-    seg_prefilter_invalid_kernel<<<G, T, 0, stream>>>(S);
-    seg_prefilter_component_kernel<<<G, T, 0, stream>>>(S);
-    FB_LAUNCH_CHECK_N(2);
-  }
-  if (seg_scan_width() == 1) {
-    seg_replay_kernel<1><<<1, 32, 0, stream>>>(S);
-  } else {
-    seg_replay_kernel<4><<<1, 32, 0, stream>>>(S);
-  }
-  FB_LAUNCH_CHECK_N(4);
+  FB_CUDA_CHECK(cudaMemsetAsync(S.touch, 0, (size_t)n, stream));
+  seg_prefilter_invalid_kernel<<<G, T, 0, stream>>>(S);
+  seg_prefilter_component_kernel<<<G, T, 0, stream>>>(S);
+  seg_replay_kernel<<<1, 32, 0, stream>>>(S);
+  FB_LAUNCH_CHECK_N(6);
   return FLOWB200_OK;
 }
 

@@ -63,7 +63,7 @@ SEG_HD void seg_neighbours(const SegState& S, int s, int nb[4]) {
   nb[3] = b + 1 < S.B ? s + S.A : -1;
 }
 
-// ---- optional prefilter: seed events that cannot have any effect are settled before the replay ----
+// ---- prefilter: seed events that cannot have any effect are settled before the replay ----
 // An invalid pixel none of whose valid 4-neighbours is near can never absorb anything: its event only marks itself.
 // A component that no invalid pixel can absorb (no near invalid 4-neighbour) and that is not removable (one pixel, or
 // min_size and more) has an event that only sets its own flag, which nobody else ever reads.  Both are marked visited

@@ -1,5 +1,5 @@
 """Times removeSmallSegments (flowb200_remove_small_segments) on the checked forward field of the bench workload
-(1024x436, K=300, 4 sweeps) and on a synthetic island field, for both scan widths of the replay kernel; checks every
+(1024x436, K=300, 4 sweeps), on a synthetic island field and on noise, all through the one replay path; checks every
 result against the C oracle.  Writes gpurun_out/segments_time.json.  (The oracle is used as the checker only.)"""
 import importlib, json, os, sys, time
 import numpy as np, torch
@@ -27,21 +27,19 @@ for name, f in fields.items():
     cpu_ms = (time.perf_counter() - t0) * 1e3
     rec = {"segments_removed": nrem, "valid_before": int(f[..., 2].sum()), "valid_after": int(want[..., 2].sum()),
            "oracle_cpu_ms_1_thread": round(cpu_ms, 3)}
-    for width in (1, 4):
-        os.environ["FLOWB200_SEG_SCAN"] = str(width)
-        src = torch.from_numpy(f).cuda()
-        ws = torch.empty(int(lib.load().flowb200_segments_workspace_bytes(H, W)), dtype=torch.uint8, device="cuda")
-        ts = []
-        for it in range(4):
-            t = src.clone()
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            ops.remove_small_segments(t, 10, 100, workspace=ws)
-            e1.record()
-            torch.cuda.synchronize()
-            ts.append(e0.elapsed_time(e1))
-        rec[f"gpu_ms_scan{width}"] = round(min(ts[1:]), 3)
-        rec[f"equal_to_oracle_scan{width}"] = bool(np.array_equal(t.cpu().numpy(), want))
+    src = torch.from_numpy(f).cuda()
+    ws = torch.empty(int(lib.load().flowb200_segments_workspace_bytes(H, W)), dtype=torch.uint8, device="cuda")
+    ts = []
+    for it in range(4):
+        t = src.clone()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        ops.remove_small_segments(t, 10, 100, workspace=ws)
+        e1.record()
+        torch.cuda.synchronize()
+        ts.append(e0.elapsed_time(e1))
+    rec["gpu_ms"] = round(min(ts[1:]), 3)
+    rec["equal_to_oracle"] = bool(np.array_equal(t.cpu().numpy(), want))
     if name == "bench_checked_forward":
         rec["epe_before"] = ops.epe(torch.from_numpy(f).cuda(), gt)[:2]
         rec["epe_after"] = ops.epe(torch.from_numpy(want).cuda(), gt)[:2]
