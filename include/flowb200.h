@@ -47,9 +47,17 @@ enum {
  *       (lamda*lcost*2^S == m, 0 <= m < 65536, 0 <= cost_shift <= 14); bit-exact with the reference whenever
  *       lcost == 20*m/2^S;
  *   INT32_F32COST: the same int32 programme fed with float32 costs, m = rint(lamda*lcost*2^S) on the fly
- *       (what flowb200_quantise_costs computes, without the extra array). */
+ *       (what flowb200_quantise_costs computes, without the extra array).
+ * Without a flag every mode reproduces the reference programme, which does not minimise the MRF energy (side terms
+ * along the chain, quirk Q1).  FLOWB200_BCD_MRF, OR'd into any mode, runs block coordinate descent on
+ *     E(l) = lamda * sum_p lcost(p, l_p) + sum over 4-connected pairs (p, q) of min(L1(v_p, v_q), tpsi):
+ * the side terms of a chain step are the two neighbours ACROSS the chain ((y, x+1) then (y, x-1) for a column chain,
+ * (y+1, x) then (y-1, x) for a row chain) with their current labels, and every step takes the smaller of the K-set
+ * candidate and the truncation candidate min_k dp(k) + tpsi (lowest k on ties).  Every chain is then an exact
+ * minimisation of E over its pixels with the rest fixed: in the int32 modes E (units of 2^-S) never rises from one
+ * phase to the next; in the float64 modes up to rounding.  Labels differ from the reference's by design. */
 enum { FLOWB200_BCD_FP64_F32COST = 0, FLOWB200_BCD_FP64_F64COST = 1, FLOWB200_BCD_INT32 = 2,
-       FLOWB200_BCD_INT32_F32COST = 3 };
+       FLOWB200_BCD_INT32_F32COST = 3, FLOWB200_BCD_MRF = 16 };
 
 /* how the per-cell nearest-neighbour search is carried out (all give the exact answer) */
 enum { FLOWB200_KNN_EXACT_FP64 = 0,   /* brute force, float64 CUDA cores                              */
@@ -152,13 +160,23 @@ int flowb200_bcd(const int32_t* pvec, const void* cost, const int32_t* nprop, in
  * a contiguous range of every phase's chains.  flowb200_bcd_prepare compiles the K-sets of the owned chains (once per
  * proposal set); flowb200_bcd_phase runs the owned chains of one phase (0 even columns down, 1 even rows right to
  * left, 2 odd columns up, 3 odd rows left to right; python bcd.py:265-277) in place on labels.
- * flowb200_bcd(sweeps) == prepare(0,1) + sweeps x phases 0..3 (0,1).  INT32 / INT32_F32COST modes only. */
+ * flowb200_bcd(sweeps) == prepare(0,1) + sweeps x phases 0..3 (0,1).  INT32 / INT32_F32COST modes only, with or
+ * without FLOWB200_BCD_MRF (whose across-chain labels are then those of the previous phase's exchange). */
 int flowb200_bcd_prepare(const int32_t* pvec, const void* cost, const int32_t* nprop, int H, int W, int K,
                          int bcd_mode, double lamda, int tpsi, int cost_shift, int part, int nparts,
                          void* workspace, size_t workspace_bytes, flowb200_stream_t stream);
 int flowb200_bcd_phase(const int32_t* pvec, const void* cost, const int32_t* nprop, int32_t* labels, int H, int W,
                        int K, int bcd_mode, double lamda, int tpsi, int cost_shift, int phase, int part, int nparts,
                        void* workspace, size_t workspace_bytes, flowb200_stream_t stream);
+
+/* The MRF energy E(labels) (see FLOWB200_BCD_MRF) in the arithmetic of bcd_mode (the MRF flag is ignored).
+ * out4: device double[4] = {data term, pairwise term, total, number of pixels whose label is outside [0, nprop)};
+ * such pixels, and every pair they belong to, are left out.  Int32 modes: sum of m (INT32_F32COST: m =
+ * rint(lamda*lcost*2^S) as the chains quantise it) + sum of min(L1, tpsi) << S, scaled by 2^-S: exact.  Float64
+ * modes: sum of lamda*lcost in double.  The summation order is fixed: repeated calls give the same bits. */
+int flowb200_energy(const int32_t* pvec, const void* cost, const int32_t* nprop, const int32_t* labels, int H, int W,
+                    int K, int bcd_mode, double lamda, int tpsi, int cost_shift, double* out4,
+                    flowb200_stream_t stream);
 
 /* bestlabels as generisi leaves them (daisy i flann.py:181-184): first strict minimum of the data costs of the first
  * nprop slots (0 where nprop is 0).  flowb200_knn_proposals computes them itself; this entry point serves callers that

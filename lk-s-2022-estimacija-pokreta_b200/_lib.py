@@ -12,6 +12,7 @@ LIB_PATH = os.path.join(_HERE, "libflowb200.so")
 
 OK, EINVAL, EWORKSPACE, ECUDA, EUNSUPPORTED = 0, -1, -2, -3, -4
 BCD_FP64_F32COST, BCD_FP64_F64COST, BCD_INT32, BCD_INT32_F32COST = 0, 1, 2, 3
+BCD_MRF = 16   # OR'd into a BCD mode: block coordinate descent on the MRF energy (include/flowb200.h)
 KNN_EXACT_FP64, KNN_TCGEN05 = 0, 1
 
 
@@ -54,6 +55,8 @@ SYMBOLS = {
                                        C.c_int, C.c_int, _P, C.c_size_t, _P]),
     "flowb200_bcd_phase": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_int,
                                      C.c_int, C.c_int, C.c_int, _P, C.c_size_t, _P]),
+    "flowb200_energy": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_int,
+                                  _P, _P]),
     "flowb200_best_labels": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P]),
     "flowb200_slot_copy": (C.c_int, [_P, C.c_int, _P, _P, C.c_int, C.c_int, _P, C.c_int, _P]),
     "flowb200_flow_from_labels": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P, _P]),

@@ -90,6 +90,73 @@ __device__ __forceinline__ int32_t quant_cost(CostT c, double lamda, int shift) 
 }
 
 // ------------------------------------------------------------------------------------------------
+// energy (SURVEY 8a): E = lamda * sum_p lcost(p, l_p) + sum over 4-connected pairs of min(L1(v_p, v_q), tpsi), in the
+// arithmetic of the mode: QUANT (int32 modes) sums quant_cost and min(L1, tpsi) << shift as integers (exact);
+// otherwise the data term is a float64 sum of lamda * lcost.  One CTA: every thread sums a fixed set of pixels, then
+// a fixed tree, so that repeated calls give the same bits.  Pixels whose label is outside [0, nprop) are counted and
+// left out, with every pair they belong to.
+// ------------------------------------------------------------------------------------------------
+constexpr int kEnergyThreads = 1024;
+
+template <typename CostT, bool QUANT>
+__global__ void __launch_bounds__(kEnergyThreads)
+energy_kernel(const int32_t* __restrict__ pvec, const CostT* __restrict__ cost, const int32_t* __restrict__ nprop,
+              const int32_t* __restrict__ labels, int H, int W, int K, double lamda, int tpsi, int shift,
+              double* __restrict__ out4) {
+  __shared__ double fd_s[kEnergyThreads];
+  __shared__ long long qd_s[kEnergyThreads], pw_s[kEnergyThreads], bad_s[kEnergyThreads];
+  const int t = threadIdx.x;
+  const int npix = H * W;
+  auto valid = [&](int p, int l) { return l >= 0 && l < nprop[p]; };
+  double fd = 0.0;
+  long long qd = 0, pw = 0, bad = 0;
+  for (int p = t; p < npix; p += kEnergyThreads) {
+    const int l = labels[p];
+    if (!valid(p, l)) {
+      ++bad;
+      continue;
+    }
+    const CostT c = cost[(size_t)p * K + l];
+    if constexpr (QUANT) qd += quant_cost<CostT>(c, lamda, shift);
+    else fd = __dadd_rn(fd, __dmul_rn(lamda, (double)c));
+    const int32_t v = pvec[(size_t)p * K + l];
+    const int y = p / W, x = p - y * W;
+    if (x + 1 < W && valid(p + 1, labels[p + 1]))
+      pw += min(tpsi, l1_vec(vec_dy(v), vec_dx(v), pvec[(size_t)(p + 1) * K + labels[p + 1]]));
+    if (y + 1 < H && valid(p + W, labels[p + W]))
+      pw += min(tpsi, l1_vec(vec_dy(v), vec_dx(v), pvec[(size_t)(p + W) * K + labels[p + W]]));
+  }
+  fd_s[t] = fd;
+  qd_s[t] = qd;
+  pw_s[t] = pw;
+  bad_s[t] = bad;
+  __syncthreads();
+  for (int s = kEnergyThreads / 2; s > 0; s >>= 1) {
+    if (t < s) {
+      fd_s[t] = __dadd_rn(fd_s[t], fd_s[t + s]);
+      qd_s[t] += qd_s[t + s];
+      pw_s[t] += pw_s[t + s];
+      bad_s[t] += bad_s[t + s];
+    }
+    __syncthreads();
+  }
+  if (t == 0) {
+    const double pair = (double)pw_s[0];
+    if constexpr (QUANT) {   // in units of 2^-shift: every sum below 2^53, so exact
+      const double unit = 1.0 / (double)(1 << shift);
+      out4[0] = (double)qd_s[0] * unit;
+      out4[1] = pair;
+      out4[2] = (double)(qd_s[0] + (pw_s[0] << shift)) * unit;
+    } else {
+      out4[0] = fd_s[0];
+      out4[1] = pair;
+      out4[2] = __dadd_rn(fd_s[0], pair);
+    }
+    out4[3] = (double)bad_s[0];
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
 // sort: one warp per pixel, counting sort of the label indices by bucket key (order inside a bucket is arbitrary)
 // ------------------------------------------------------------------------------------------------
 constexpr int kSortWarps = 8;
@@ -465,15 +532,40 @@ constexpr int kMaxWarps = 16;   // T <= 512
 __host__ __device__ inline uint32_t kset_slot_bytes(int Kpad) {
   return (uint32_t)((kRecHeader + 2 * (size_t)Kpad + 8 * (size_t)Kpad + 2 * (size_t)kSlotPerLabel * Kpad + 127) & ~(size_t)127);
 }
-// dynamic shared memory of the float64 kernel: oldvec int32[len] | vprev int32[Kpad] | path uint16[len] | the record
-// slots, 128-aligned
-__host__ __device__ inline size_t chain_fixed_smem(int Kpad, int len) {
-  return (4 * (size_t)len + 4 * (size_t)Kpad + 2 * (size_t)len + 127) & ~(size_t)127;
+// dynamic shared memory of the float64 kernel: side vectors int32[nside * len] | vprev int32[Kpad] | path uint16[len] |
+// the record slots, 128-aligned.  nside = 1: the reference's side terms read the chain's own old vectors (oldvec);
+// nside = 2 (FLOWB200_BCD_MRF): the labels' vectors of the two across-chain neighbours of every step
+__host__ __device__ inline size_t chain_fixed_smem(int Kpad, int len, int nside = 1) {
+  return (4 * (size_t)nside * len + 4 * (size_t)Kpad + 2 * (size_t)len + 127) & ~(size_t)127;
 }
 // ... of the 32-bit kernel, behind the (run-time) pad that aligns it to 4 KB: dp 4 KB | control 384 B |
-// oldvec int32[len] | path uint16[len] | the record slots, 128-aligned
-__host__ __device__ inline size_t chain32_fixed_smem(int len) {
-  return (4096 + 384 + 4 * (size_t)len + 2 * (size_t)len + 127) & ~(size_t)127;
+// side vectors int32[nside * len] | path uint16[len] | the record slots, 128-aligned
+__host__ __device__ inline size_t chain32_fixed_smem(int len, int nside = 1) {
+  return (4096 + 384 + 4 * (size_t)nside * len + 2 * (size_t)len + 127) & ~(size_t)127;
+}
+
+// FLOWB200_BCD_MRF: the side neighbours of a chain step lie ACROSS the chain axis -- (y, x + 1) and (y, x - 1) of a
+// column chain, (y + 1, x) and (y - 1, x) of a row chain, in that order.  They belong to lines of the other parity,
+// which no chain of the phase writes, so their labels are read once when the chain starts.  Whether they exist
+// depends on the chain's line only.
+struct AcrossChain {
+  bool has_p, has_m;
+  int off;   // pixel index offset of the + neighbour (the - neighbour is at -off)
+};
+__device__ __forceinline__ AcrossChain across_chain(const ChainGeom& g, int H, int W) {
+  if (g.ystep != 0) return {g.sx + 1 < W, g.sx > 0, 1};
+  return {g.sy + 1 < H, g.sy > 0, W};
+}
+// side[i] / side[len + i]: vector of the label of the + / - neighbour of step i (0 where it does not exist)
+template <int T>
+__device__ __forceinline__ void load_across(const ChainArgs& a, const ChainGeom& g, int32_t* side) {
+  const AcrossChain ac = across_chain(g, a.H, a.W);
+  for (int i = threadIdx.x; i < g.len; i += T) {
+    const int p = (g.sy + i * g.ystep) * a.W + (g.sx + i * g.xstep);
+    const int pp = p + ac.off, pm = p - ac.off;
+    side[i] = ac.has_p ? a.pvec[(size_t)pp * a.K + a.labels[pp]] : 0;
+    side[g.len + i] = ac.has_m ? a.pvec[(size_t)pm * a.K + a.labels[pm]] : 0;
+  }
 }
 
 // backtrack (:238-253) through the back-pointers of the chain of this block, staged through shared memory (the record
@@ -526,7 +618,9 @@ __device__ __forceinline__ void warp_argmin_f64(double& val, int& idx) {
   }
 }
 
-template <typename CostT, int T, bool QUANT>
+// MRF (FLOWB200_BCD_MRF): side terms across the chain (AcrossChain) and, at every step, the smaller of the K-set
+// candidate and the truncation candidate (DESIGN 4.4).
+template <typename CostT, int T, bool QUANT, bool MRF>
 __device__ __forceinline__ void chainf64_body(const ChainArgs& a) {
   constexpr int NW = T / 32;
   constexpr int kNone = 0x7fffffff;
@@ -553,15 +647,20 @@ __device__ __forceinline__ void chainf64_body(const ChainArgs& a) {
   const CostT* cost = static_cast<const CostT*>(a.cost);
   const double lamda = a.lamda;
 
-  int32_t* oldvec = reinterpret_cast<int32_t*>(smem_raw);
-  int32_t* vprev = oldvec + g.len;
+  constexpr int kSide = MRF ? 2 : 1;
+  int32_t* oldvec = reinterpret_cast<int32_t*>(smem_raw);   // MRF: the across-chain vectors, 2 x len
+  int32_t* vprev = oldvec + kSide * g.len;
   uint16_t* path = reinterpret_cast<uint16_t*>(vprev + Kpad);
-  unsigned char* slots = smem_raw + chain_fixed_smem(Kpad, g.len);
+  unsigned char* slots = smem_raw + chain_fixed_smem(Kpad, g.len, kSide);
   auto pixel = [&](int i) { return (g.sy + i * g.ystep) * a.W + (g.sx + i * g.xstep); };
 
-  for (int i = t; i < g.len; i += T) {
-    const int p = pixel(i);
-    oldvec[i] = a.pvec[(size_t)p * K + a.labels[p]];
+  if constexpr (MRF) {
+    load_across<T>(a, g, oldvec);
+  } else {
+    for (int i = t; i < g.len; i += T) {
+      const int p = pixel(i);
+      oldvec[i] = a.pvec[(size_t)p * K + a.labels[p]];
+    }
   }
   if (t == 0) {
     for (int s = 0; s < S; ++s) ptx::mbar_init(&mbar[s], 1);
@@ -613,9 +712,21 @@ __device__ __forceinline__ void chainf64_body(const ChainArgs& a) {
     double dpv = CUDART_INF;
     int mine = kNone;
     // side terms (sidepsi :84-88): the neighbour on the +1 side of the chain axis first, as the reference adds them
-    const int ip = i + sgn, im = i - sgn;
-    const bool has_p = ip >= 0 && ip < g.len, has_m = im >= 0 && im < g.len;
-    const int32_t ov_p = has_p ? oldvec[ip] : 0, ov_m = has_m ? oldvec[im] : 0;
+    bool has_p, has_m;
+    int32_t ov_p, ov_m;
+    if constexpr (MRF) {
+      const AcrossChain ac = across_chain(g, a.H, a.W);
+      has_p = ac.has_p;
+      has_m = ac.has_m;
+      ov_p = oldvec[i];
+      ov_m = oldvec[g.len + i];
+    } else {
+      const int ip = i + sgn, im = i - sgn;
+      has_p = ip >= 0 && ip < g.len;
+      has_m = im >= 0 && im < g.len;
+      ov_p = has_p ? oldvec[ip] : 0;
+      ov_m = has_m ? oldvec[im] : 0;
+    }
     // dp of label `orig` (vector dy, dx) from the minimum (best, arg) over the previous step's candidates
     auto finish = [&](int dy, int dx, int orig, double best, int arg, const int p) {
       const int psi_p = has_p ? units(min(tpsi, l1_vec(dy, dx, ov_p))) : 0;
@@ -626,8 +737,18 @@ __device__ __forceinline__ void chainf64_body(const ChainArgs& a) {
       if (i == 0) {   // (psi+ + psi-) + lamda*lcost   (:118-120)
         dpv = __dadd_rn((double)(psi_p + psi_m), lc);
       } else {        // (lamda*lcost + psi+) + psi-, then m + that   (:161-162, :176)
-        if (arg == kNone) block_argmin(i - 1, best, arg);   // quirk Q1: min_k (tpsi + dp_prev[k]), lowest k (:152-157),
-                                                           // only for an empty K-set
+        if constexpr (MRF) {   // the truncation candidate at every step: the smaller (value, label) of the two
+          double tv;
+          int tk;
+          block_argmin(i - 1, tv, tk);
+          if (tv < best || (tv == best && tk < arg)) {
+            best = tv;
+            arg = tk;
+          }
+        } else if (arg == kNone) {
+          block_argmin(i - 1, best, arg);   // quirk Q1: min_k (tpsi + dp_prev[k]), lowest k (:152-157), only for an
+                                            // empty K-set
+        }
         dpv = __dadd_rn(best, __dadd_rn(__dadd_rn(lc, (double)psi_p), (double)psi_m));
         bp_row[orig] = (uint16_t)arg;
       }
@@ -742,7 +863,7 @@ __device__ __forceinline__ void chainf64_body(const ChainArgs& a) {
 constexpr int kKeyBytes = 4096;   // dp of labels 0..510 in two buffers; the slot of label 511 stays infinite (null entries)
 constexpr int kCtlBytes = 384;    // warp minima [2][16] x 2, four mbarriers
 
-template <typename CostT, int T, int SHIFT>
+template <typename CostT, int T, int SHIFT, bool MRF>
 __device__ __forceinline__ void chain32_body(const ChainArgs& a) {
   constexpr int NW = T / 32;
   constexpr uint32_t kInf = 0xFFFFFFFFu;
@@ -767,18 +888,20 @@ __device__ __forceinline__ void chain32_body(const ChainArgs& a) {
   uint32_t (*wred_v)[kMaxWarps] = reinterpret_cast<uint32_t (*)[kMaxWarps]>(smem_raw + pad + kKeyBytes);         // [2][16]: per warp,
   uint32_t (*wred_l)[kMaxWarps] = reinterpret_cast<uint32_t (*)[kMaxWarps]>(smem_raw + pad + kKeyBytes + 128);   // min dp of a step and the lowest label that has it
   uint64_t* mbar = reinterpret_cast<uint64_t*>(smem_raw + pad + kKeyBytes + 256);                                // [4]
-  int32_t* oldvec = reinterpret_cast<int32_t*>(smem_raw + pad + kKeyBytes + kCtlBytes);
-  uint16_t* path = reinterpret_cast<uint16_t*>(oldvec + len);
-  unsigned char* slots = smem_raw + pad + chain32_fixed_smem(len);
+  constexpr int kSide = MRF ? 2 : 1;
+  int32_t* oldvec = reinterpret_cast<int32_t*>(smem_raw + pad + kKeyBytes + kCtlBytes);   // MRF: across-chain, 2 x len
+  uint16_t* path = reinterpret_cast<uint16_t*>(oldvec + kSide * len);
+  unsigned char* slots = smem_raw + pad + chain32_fixed_smem(len, kSide);
   auto pixel = [&](int i) { return (g.sy + i * g.ystep) * a.W + (g.sx + i * g.xstep); };
 
   if (t == 0) absent_s = 0;
   __syncthreads();
   {
     bool absent = false;
+    if constexpr (MRF) load_across<T>(a, g, oldvec);
     for (int i = t; i < len; i += T) {
       const int p = pixel(i);
-      oldvec[i] = a.pvec[(size_t)p * K + a.labels[p]];
+      if constexpr (!MRF) oldvec[i] = a.pvec[(size_t)p * K + a.labels[p]];
       absent |= (dsc[p] >> 40) == 0;
     }
     if (absent || K > 511 || a.force_generic) absent_s = 1;   // (label 511's slot is the padding entries' infinity)
@@ -833,8 +956,14 @@ __device__ __forceinline__ void chain32_body(const ChainArgs& a) {
       // before this call), in units of 2^-shift
       const int dy = vec_dy((int32_t)st.x), dx = vec_dx((int32_t)st.x);
       uint32_t psi = 0;
-      if (i + 1 < len) psi += (uint32_t)min(tpsi, l1_vec(dy, dx, oldvec[i + 1]));
-      if (i > 0) psi += (uint32_t)min(tpsi, l1_vec(dy, dx, oldvec[i - 1]));
+      if constexpr (MRF) {
+        const AcrossChain ac = across_chain(g, a.H, a.W);
+        if (ac.has_p) psi += (uint32_t)min(tpsi, l1_vec(dy, dx, oldvec[i]));
+        if (ac.has_m) psi += (uint32_t)min(tpsi, l1_vec(dy, dx, oldvec[len + i]));
+      } else {
+        if (i + 1 < len) psi += (uint32_t)min(tpsi, l1_vec(dy, dx, oldvec[i + 1]));
+        if (i > 0) psi += (uint32_t)min(tpsi, l1_vec(dy, dx, oldvec[i - 1]));
+      }
       dp = (st.y & 0xFFFFu) + (psi << shift);   // dp_0 = unary (:118-120)
       if (i > 0) {
         const uint32_t ng = st.y >> 25;
@@ -868,8 +997,14 @@ __device__ __forceinline__ void chain32_body(const ChainArgs& a) {
           lex_min(v1, k1, cd, kd);
         }
         lex_min(v0, k0, v1, k1);
+        if constexpr (MRF) {   // the truncation candidate at every step, label field << 3 like the entries'
+          uint32_t tv = kInf, tk = kInf;
+#pragma unroll
+          for (int k = 0; k < NW; ++k) lex_min(tv, tk, wred_v[(i - 1) & 1][k], wred_l[(i - 1) & 1][k]);
+          lex_min(v0, k0, tv + tpsi_dp, tk << 3);
+        }
         uint32_t arg = k0 >> 3;
-        if (ng == 0) {   // quirk Q1: the truncation candidate min_k (tpsi + dp_prev[k]), lowest k (:152-157), only for an
+        if (!MRF && ng == 0) {   // quirk Q1: the truncation candidate min_k (tpsi + dp_prev[k]), lowest k (:152-157), only for an
                          // empty K-set (last warps: labels are stored by decreasing list length)
           v0 = kInf;
           arg = kInf;
@@ -908,12 +1043,23 @@ __device__ __forceinline__ void chain32_body(const ChainArgs& a) {
 
 template <typename CostT, int T, int MINB, bool QUANT>
 __global__ void __launch_bounds__(T, MINB) kset_chainf64_kernel(const ChainArgs a) {
-  chainf64_body<CostT, T, QUANT>(a);
+  chainf64_body<CostT, T, QUANT, false>(a);
 }
 
 template <typename CostT, int T, int MINB, int SHIFT>
 __global__ void __launch_bounds__(T, MINB) kset_chain32_kernel(const ChainArgs a) {
-  chain32_body<CostT, T, SHIFT>(a);
+  chain32_body<CostT, T, SHIFT, false>(a);
+}
+
+// the FLOWB200_BCD_MRF programme: kernels of their own, so that the reference programme's stay as they are
+template <typename CostT, int T, int MINB, bool QUANT>
+__global__ void __launch_bounds__(T, MINB) kset_chainf64_mrf_kernel(const ChainArgs a) {
+  chainf64_body<CostT, T, QUANT, true>(a);
+}
+
+template <typename CostT, int T, int MINB, int SHIFT>
+__global__ void __launch_bounds__(T, MINB) kset_chain32_mrf_kernel(const ChainArgs a) {
+  chain32_body<CostT, T, SHIFT, true>(a);
 }
 
 // the variant of kset_chainf64_kernel a mode runs: the float64 programme (shift < 0) or the integer one.  Only variants
@@ -923,6 +1069,12 @@ auto chainf64_kernel(int shift) {
   if constexpr (std::is_integral<CostT>::value) return kset_chainf64_kernel<CostT, T, 1, true>;
   else if constexpr (std::is_same<CostT, double>::value) return kset_chainf64_kernel<CostT, T, 1, false>;
   else return shift < 0 ? kset_chainf64_kernel<CostT, T, 1, false> : kset_chainf64_kernel<CostT, T, 1, true>;
+}
+template <typename CostT, int T>
+auto chainf64_mrf_kernel(int shift) {
+  if constexpr (std::is_integral<CostT>::value) return kset_chainf64_mrf_kernel<CostT, T, 1, true>;
+  else if constexpr (std::is_same<CostT, double>::value) return kset_chainf64_mrf_kernel<CostT, T, 1, false>;
+  else return shift < 0 ? kset_chainf64_mrf_kernel<CostT, T, 1, false> : kset_chainf64_mrf_kernel<CostT, T, 1, true>;
 }
 
 struct KsetLayout {
@@ -983,9 +1135,12 @@ struct KsetPlan {
 // shift < 0 selects the float64 programme (kset_chainf64_kernel): the records then carry no data costs, and no 32-bit
 // chain kernel is compiled (double costs) or set up.  Dropping the 32-bit kernel's shared-memory check there changes
 // nothing: the float64 kernel's check is stricter, its left side is 4*Kpad + 128 bytes larger at every chain length
+// mrf: the FLOWB200_BCD_MRF kernels, whose side vectors take 2 x len int32 of shared memory instead of len (the dp
+// bound holds as it is: a step adds at most the smaller of the two candidates, so at most tpsi over the minimum)
 template <typename CostT>
-static int make_plan(int H, int W, int K, int tpsi, int shift, size_t workspace_bytes, KsetPlan<CostT>* P) {
+static int make_plan(int H, int W, int K, int tpsi, int shift, bool mrf, size_t workspace_bytes, KsetPlan<CostT>* P) {
   if (K > 512 || tpsi < 0 || tpsi > 32) return FLOWB200_EUNSUPPORTED;
+  const int nside = mrf ? 2 : 1;
   P->records = tpsi >= 1 && tpsi <= 8 && (shift < 0 || shift >= 4);
   if (shift >= 0) {   // dp is a uint32
     const unsigned long long per_step = ((unsigned long long)(3 * tpsi) << shift) + 65535ull;
@@ -1001,14 +1156,18 @@ static int make_plan(int H, int W, int K, int tpsi, int shift, size_t workspace_
   if (!P->kernf64 && K <= TT) {                                                                              \
     constexpr int mb = MB > 4 ? 4 : MB, mb_lo = mb - (MB >= 4 ? 1 : 0);                                      \
     if constexpr (!std::is_same<CostT, double>::value) {                                                     \
-      if (shift >= 0) {                                                                                      \
+      if (shift >= 0 && mrf) {   /* one instantiation per width: no variant for fewer chains per SM */       \
+        P->kern32 = shift == 12 ? kset_chain32_mrf_kernel<CostT, TT, mb, 12>                                 \
+                                : kset_chain32_mrf_kernel<CostT, TT, mb, 0>;                                 \
+        P->kern32_lo = P->kern32;                                                                            \
+      } else if (shift >= 0) {                                                                               \
         P->kern32 = shift == 12 ? kset_chain32_kernel<CostT, TT, mb, 12> : kset_chain32_kernel<CostT, TT, mb, 0>;\
         P->kern32_lo = shift == 12 ? kset_chain32_kernel<CostT, TT, mb_lo, 12>                               \
                                    : kset_chain32_kernel<CostT, TT, mb_lo, 0>;                               \
       }                                                                                                      \
     }                                                                                                        \
     P->minb = mb;                                                                                            \
-    P->kernf64 = chainf64_kernel<CostT, TT>(shift);                                                          \
+    P->kernf64 = mrf ? chainf64_mrf_kernel<CostT, TT>(shift) : chainf64_kernel<CostT, TT>(shift);            \
     P->T = TT;                                                                                               \
     minb = MB;                                                                                               \
   }
@@ -1021,15 +1180,15 @@ static int make_plan(int H, int W, int K, int tpsi, int shift, size_t workspace_
   P->slot_bytes = kset_slot_bytes(Kpad);
   // + static shared memory (32-bit kernel 0.2 KB, float64 kernel 8.5 KB) + the driver's 1 KB per CTA
   const size_t budget = (size_t)(227 * 1024) / minb - 1024 - 512;
-  if (4096 + chain32_fixed_smem(H < W ? H : W) + 4 * (size_t)P->slot_bytes > budget) P->slot_shift = 1;
+  if (4096 + chain32_fixed_smem(H < W ? H : W, nside) + 4 * (size_t)P->slot_bytes > budget) P->slot_shift = 1;
   // long chains (large images): fewer resident chains rather than smaller slots
   const size_t slots = (size_t)P->slot_bytes << P->slot_shift;
-  P->smem32[0] = 4096 + chain32_fixed_smem(H) + slots;
-  P->smem32[1] = 4096 + chain32_fixed_smem(W) + slots;
-  P->smem64 = chain_fixed_smem(Kpad, maxlen) + slots;
+  P->smem32[0] = 4096 + chain32_fixed_smem(H, nside) + slots;
+  P->smem32[1] = 4096 + chain32_fixed_smem(W, nside) + slots;
+  P->smem64 = chain_fixed_smem(Kpad, maxlen, nside) + slots;
   if (P->smem64 + 1024 + 9216 > (size_t)227 * 1024) return FLOWB200_EUNSUPPORTED;
   if (P->kern32) {   // int32 modes
-    const size_t smem32 = 4096 + chain32_fixed_smem(maxlen) + slots;   // (4096: worst case of the run-time pad)
+    const size_t smem32 = 4096 + chain32_fixed_smem(maxlen, nside) + slots;   // (4096: worst case of the run-time pad)
     if (smem32 + 1536 > (size_t)227 * 1024) return FLOWB200_EUNSUPPORTED;
     FB_CUDA_CHECK(cudaFuncSetAttribute(P->kern32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem32));
     FB_CUDA_CHECK(cudaFuncSetAttribute(P->kern32_lo, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem32));
@@ -1041,11 +1200,11 @@ static int make_plan(int H, int W, int K, int tpsi, int shift, size_t workspace_
 // sort + record build for the chains this part owns
 template <typename CostT>
 int ksets_prepare(const int32_t* pvec, const CostT* cost, const int32_t* nprop, int H, int W, int K, double lamda,
-                  int tpsi, int shift, int part, int nparts, void* workspace, size_t workspace_bytes,
+                  int tpsi, int shift, bool mrf, int part, int nparts, void* workspace, size_t workspace_bytes,
                   cudaStream_t stream) {
   if (nparts < 1 || part < 0 || part >= nparts) return FLOWB200_EINVAL;
   KsetPlan<CostT> P;
-  const int rc = make_plan<CostT>(H, W, K, tpsi, shift, workspace_bytes, &P);
+  const int rc = make_plan<CostT>(H, W, K, tpsi, shift, mrf, workspace_bytes, &P);
   if (rc) return rc;
   const KsetLayout& L = P.L;
   char* ws = static_cast<char*>(workspace);
@@ -1077,11 +1236,11 @@ int ksets_prepare(const int32_t* pvec, const CostT* cost, const int32_t* nprop, 
 // one phase, the chains this part owns, in place on labels
 template <typename CostT>
 int ksets_phase(const int32_t* pvec, const CostT* cost, const int32_t* nprop, int32_t* labels, int H, int W, int K,
-                double lamda, int tpsi, int shift, int phase, int part, int nparts, void* workspace,
+                double lamda, int tpsi, int shift, bool mrf, int phase, int part, int nparts, void* workspace,
                 size_t workspace_bytes, cudaStream_t stream) {
   if (nparts < 1 || part < 0 || part >= nparts || phase < 0 || phase > 3) return FLOWB200_EINVAL;
   KsetPlan<CostT> P;
-  const int rc = make_plan<CostT>(H, W, K, tpsi, shift, workspace_bytes, &P);
+  const int rc = make_plan<CostT>(H, W, K, tpsi, shift, mrf, workspace_bytes, &P);
   if (rc) return rc;
   const KsetLayout& L = P.L;
   char* ws = static_cast<char*>(workspace);
@@ -1117,17 +1276,18 @@ int ksets_phase(const int32_t* pvec, const CostT* cost, const int32_t* nprop, in
 
 template <typename CostT>
 int launch_sweeps_ksets(const int32_t* pvec, const CostT* cost, const int32_t* nprop, int32_t* labels, int H, int W,
-                        int K, double lamda, int tpsi, int shift, int sweeps, int32_t* labels_per_sweep,
+                        int K, double lamda, int tpsi, int shift, bool mrf, int sweeps, int32_t* labels_per_sweep,
                         void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   if (sweeps <= 0) {
     KsetPlan<CostT> P;
-    return make_plan<CostT>(H, W, K, tpsi, shift, workspace_bytes, &P);
+    return make_plan<CostT>(H, W, K, tpsi, shift, mrf, workspace_bytes, &P);
   }
-  int rc = ksets_prepare<CostT>(pvec, cost, nprop, H, W, K, lamda, tpsi, shift, 0, 1, workspace, workspace_bytes, stream);
+  int rc = ksets_prepare<CostT>(pvec, cost, nprop, H, W, K, lamda, tpsi, shift, mrf, 0, 1, workspace, workspace_bytes,
+                                stream);
   if (rc) return rc;
   for (int w = 0; w < sweeps; ++w) {
     for (int phase = 0; phase < 4; ++phase) {
-      rc = ksets_phase<CostT>(pvec, cost, nprop, labels, H, W, K, lamda, tpsi, shift, phase, 0, 1, workspace,
+      rc = ksets_phase<CostT>(pvec, cost, nprop, labels, H, W, K, lamda, tpsi, shift, mrf, phase, 0, 1, workspace,
                               workspace_bytes, stream);
       if (rc) return rc;
     }
@@ -1184,11 +1344,13 @@ extern "C" int flowb200_bcd(const int32_t* pvec, const void* cost, const int32_t
   if (!pvec || !cost || !nprop || !labels || !workspace) return FLOWB200_EINVAL;
   if (H <= 0 || W <= 0 || K <= 0 || K > 512 || sweeps < 0 || tpsi < 0) return FLOWB200_EINVAL;
   if (H > 16384 || W > 16384) return FLOWB200_EINVAL;
+  const bool mrf = (bcd_mode & FLOWB200_BCD_MRF) != 0;
+  bcd_mode &= ~FLOWB200_BCD_MRF;
   if (is_int_mode(bcd_mode) && (cost_shift < 0 || cost_shift > 14)) return FLOWB200_EINVAL;
   // any workspace that holds the fixed part is accepted: records that do not fit are evaluated densely
   return with_mode(bcd_mode, cost, cost_shift, [&](auto c, int shift) {
-    return launch_sweeps_ksets(pvec, c, nprop, labels, H, W, K, lamda, tpsi, shift, sweeps, labels_per_sweep, workspace,
-                               workspace_bytes, stream);
+    return launch_sweeps_ksets(pvec, c, nprop, labels, H, W, K, lamda, tpsi, shift, mrf, sweeps, labels_per_sweep,
+                               workspace, workspace_bytes, stream);
   });
 }
 
@@ -1199,9 +1361,12 @@ extern "C" int flowb200_bcd_prepare(const int32_t* pvec, const void* cost, const
   if (!pvec || !cost || !nprop || !workspace) return FLOWB200_EINVAL;
   if (H <= 0 || W <= 0 || K <= 0 || K > 512 || H > 16384 || W > 16384) return FLOWB200_EINVAL;
   if (cost_shift < 0 || cost_shift > 14) return FLOWB200_EINVAL;
+  const bool mrf = (bcd_mode & FLOWB200_BCD_MRF) != 0;
+  bcd_mode &= ~FLOWB200_BCD_MRF;
   if (!is_int_mode(bcd_mode)) return FLOWB200_EUNSUPPORTED;
   return with_mode(bcd_mode, cost, cost_shift, [&](auto c, int shift) {
-    return ksets_prepare(pvec, c, nprop, H, W, K, lamda, tpsi, shift, part, nparts, workspace, workspace_bytes, stream);
+    return ksets_prepare(pvec, c, nprop, H, W, K, lamda, tpsi, shift, mrf, part, nparts, workspace, workspace_bytes,
+                         stream);
   });
 }
 
@@ -1211,10 +1376,30 @@ extern "C" int flowb200_bcd_phase(const int32_t* pvec, const void* cost, const i
   if (!pvec || !cost || !nprop || !labels || !workspace) return FLOWB200_EINVAL;
   if (H <= 0 || W <= 0 || K <= 0 || K > 512 || H > 16384 || W > 16384) return FLOWB200_EINVAL;
   if (cost_shift < 0 || cost_shift > 14) return FLOWB200_EINVAL;
+  const bool mrf = (bcd_mode & FLOWB200_BCD_MRF) != 0;
+  bcd_mode &= ~FLOWB200_BCD_MRF;
   if (!is_int_mode(bcd_mode)) return FLOWB200_EUNSUPPORTED;
   return with_mode(bcd_mode, cost, cost_shift, [&](auto c, int shift) {
-    return ksets_phase(pvec, c, nprop, labels, H, W, K, lamda, tpsi, shift, phase, part, nparts, workspace,
+    return ksets_phase(pvec, c, nprop, labels, H, W, K, lamda, tpsi, shift, mrf, phase, part, nparts, workspace,
                        workspace_bytes, stream);
+  });
+}
+
+extern "C" int flowb200_energy(const int32_t* pvec, const void* cost, const int32_t* nprop, const int32_t* labels,
+                               int H, int W, int K, int bcd_mode, double lamda, int tpsi, int cost_shift, double* out4,
+                               flowb200_stream_t stream) {
+  if (!pvec || !cost || !nprop || !labels || !out4) return FLOWB200_EINVAL;
+  if (H <= 0 || W <= 0 || K <= 0 || tpsi < 0 || (long long)H * W > 0x7FFFFFFFll) return FLOWB200_EINVAL;
+  bcd_mode &= ~FLOWB200_BCD_MRF;   // the energy does not depend on the optimiser
+  if (is_int_mode(bcd_mode) && (cost_shift < 0 || cost_shift > 14)) return FLOWB200_EINVAL;
+  return with_mode(bcd_mode, cost, cost_shift, [&](auto c, int shift) {
+    using CostT = std::remove_const_t<std::remove_pointer_t<decltype(c)>>;
+    // (only the variants a mode can run, as for the chain kernels)
+    auto kern = energy_kernel<CostT, !std::is_same<CostT, double>::value>;
+    if constexpr (std::is_same<CostT, float>::value) kern = shift >= 0 ? energy_kernel<float, true> : energy_kernel<float, false>;
+    kern<<<1, kEnergyThreads, 0, stream>>>(pvec, c, nprop, labels, H, W, K, lamda, tpsi, shift < 0 ? 0 : shift, out4);
+    FB_LAUNCH_CHECK();
+    return FLOWB200_OK;
   });
 }
 

@@ -140,11 +140,14 @@ static int run_bcd(const flowb200_params* p, const PairLayout& L, char* ws, int 
   int32_t* nprop = reinterpret_cast<int32_t*>(ws + L.nprop[d]);
   int32_t* labels = reinterpret_cast<int32_t*>(ws + L.labels[d]);
   // the pipeline produces float32 costs: the int32 programme quantises them on the fly
-  int mode = p->bcd_mode;
+  // (FLOWB200_BCD_MRF passes through to the chains)
+  const int mrf = p->bcd_mode & FLOWB200_BCD_MRF;
+  int mode = p->bcd_mode & ~FLOWB200_BCD_MRF;
   if (mode == FLOWB200_BCD_INT32) mode = FLOWB200_BCD_INT32_F32COST;
   if (mode != FLOWB200_BCD_INT32_F32COST && mode != FLOWB200_BCD_FP64_F32COST) return FLOWB200_EINVAL;
-  int rc = flowb200_bcd(pvec, lcost, nprop, labels, p->H, p->W, p->maxnprop, mode, p->lamda, p->tpsi, p->cost_shift,
-                        sweeps, nullptr, ws + L.bcd_ws[d], flowb200_bcd_workspace_bytes(p->H, p->W, p->maxnprop), stream);
+  int rc = flowb200_bcd(pvec, lcost, nprop, labels, p->H, p->W, p->maxnprop, mode | mrf, p->lamda, p->tpsi,
+                        p->cost_shift, sweeps, nullptr, ws + L.bcd_ws[d],
+                        flowb200_bcd_workspace_bytes(p->H, p->W, p->maxnprop), stream);
   if (rc) return rc;
   return flowb200_flow_from_labels(pvec, labels, p->H, p->W, p->maxnprop, nullptr,
                                    reinterpret_cast<float*>(ws + L.uvv[d]), stream);

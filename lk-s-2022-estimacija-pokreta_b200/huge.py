@@ -314,10 +314,11 @@ def flow_pair_sharded(bgr0, bgr1, p: FlowParams, sweeps, directions, seed, bcd_m
         src, tgt = d[direction], d[1 - direction]
         pvec, lcost, nprop, labels = knn_proposals_sharded(src, tgt, p, rank, world, dist)
         ops.random_proposals(src, tgt, p, pvec, lcost, nprop, labels, seed=seed + direction)
-        if bcd_mode in (_lib.BCD_INT32, _lib.BCD_INT32_F32COST):
-            bcd_sharded(pvec, lcost, nprop, labels, sweeps, p, _lib.BCD_INT32_F32COST, rank, world, dist)
+        mrf = bcd_mode & _lib.BCD_MRF
+        if (bcd_mode & ~_lib.BCD_MRF) in (_lib.BCD_INT32, _lib.BCD_INT32_F32COST):
+            bcd_sharded(pvec, lcost, nprop, labels, sweeps, p, _lib.BCD_INT32_F32COST | mrf, rank, world, dist)
         else:   # the float64 programme is not split: replicated
-            ops.bcd(pvec, lcost, nprop, labels, sweeps, mode=_lib.BCD_FP64_F32COST, lamda=p.lamda, tpsi=p.tpsi,
+            ops.bcd(pvec, lcost, nprop, labels, sweeps, mode=_lib.BCD_FP64_F32COST | mrf, lamda=p.lamda, tpsi=p.tpsi,
                     cost_shift=p.cost_shift)
         uvv.append(ops.flow_from_labels(pvec, labels, want_yx=False)[1])
         del pvec, lcost

@@ -123,17 +123,51 @@ _BCD_COST_DTYPE = {_lib.BCD_FP64_F32COST: torch.float32, _lib.BCD_FP64_F64COST: 
                    _lib.BCD_INT32: torch.int32, _lib.BCD_INT32_F32COST: torch.float32}
 
 
+def _cost_dtype(mode):
+    """dtype of the cost array of a BCD mode (the BCD_MRF flag does not change it)"""
+    return _BCD_COST_DTYPE[mode & ~_lib.BCD_MRF]
+
+
+def energy(pvec, cost, nprop, labels, mode=_lib.BCD_FP64_F32COST, lamda=0.05, tpsi=8, cost_shift=12):
+    """The MRF energy of labels in the arithmetic of `mode` (flowb200_energy): (data, pairwise, total, n_bad), n_bad =
+    pixels whose label is outside [0, nprop), left out of both terms.  Exact in the int32 modes."""
+    lib = _lib.load()
+    H, W, K = pvec.shape
+    out = torch.empty(4, dtype=torch.float64, device=pvec.device)
+    _lib.check(lib.flowb200_energy(_ptr(pvec, torch.int32, "pvec"), _ptr(cost, _cost_dtype(mode), "cost"),
+                                   _ptr(nprop, torch.int32, "nprop"), _ptr(labels, torch.int32, "labels"), H, W, K,
+                                   int(mode), float(lamda), int(tpsi), int(cost_shift), _ptr(out), _stream()),
+               "flowb200_energy")
+    data, pair, total, bad = out.tolist()
+    return data, pair, total, int(bad)
+
+
 def bcd(pvec, cost, nprop, labels, sweeps, mode=_lib.BCD_FP64_F32COST, lamda=0.05, tpsi=8, cost_shift=12,
-        per_sweep=False, workspace_bytes=None):
+        per_sweep=False, workspace_bytes=None, energy_per_phase=False):
     """ceoBCD (python bcd.py:261-284): `sweeps` sweeps in place on labels.
 
-    Returns int32 (sweeps,H,W) snapshots after every sweep when per_sweep, else None."""
+    Returns int32 (sweeps,H,W) snapshots after every sweep when per_sweep, else None.
+    energy_per_phase (int32 modes, which bcd_prepare / bcd_phase run): returns (snapshots, energies) instead, with
+    energies the total energy (`energy`) before the first phase and after every phase, 1 + 4 * sweeps floats."""
     lib = _lib.load()
     H, W, K = pvec.shape
     snaps = torch.empty((sweeps, H, W), dtype=torch.int32, device=pvec.device) if per_sweep else None
     nb = lib.flowb200_bcd_workspace_bytes(H, W, K) if workspace_bytes is None else int(workspace_bytes)
     ws = _workspace(nb, pvec.device)[:nb]
-    rc = lib.flowb200_bcd(_ptr(pvec, torch.int32, "pvec"), _ptr(cost, _BCD_COST_DTYPE[mode], "cost"),
+    if energy_per_phase:
+        if (mode & ~_lib.BCD_MRF) not in (_lib.BCD_INT32, _lib.BCD_INT32_F32COST):
+            raise ValueError("energy_per_phase: int32 modes only (bcd_prepare / bcd_phase)")
+        kw = dict(mode=mode, lamda=lamda, tpsi=tpsi, cost_shift=cost_shift)
+        bcd_prepare(pvec, cost, nprop, ws, 0, 1, **kw)
+        energies = [energy(pvec, cost, nprop, labels, **kw)[2]]
+        for w in range(sweeps):
+            for phase in range(4):
+                bcd_phase(pvec, cost, nprop, labels, ws, phase, 0, 1, **kw)
+                energies.append(energy(pvec, cost, nprop, labels, **kw)[2])
+            if per_sweep:
+                snaps[w].copy_(labels)
+        return snaps, energies
+    rc = lib.flowb200_bcd(_ptr(pvec, torch.int32, "pvec"), _ptr(cost, _cost_dtype(mode), "cost"),
                           _ptr(nprop, torch.int32, "nprop"), _ptr(labels, torch.int32, "labels"), H, W, K, int(mode),
                           float(lamda), int(tpsi), int(cost_shift), int(sweeps), _ptr(snaps), _ptr(ws), ws.numel(),
                           _stream())
@@ -158,7 +192,7 @@ def bcd_prepare(pvec, cost, nprop, ws, part=0, nparts=1, mode=_lib.BCD_INT32_F32
     """Compile the K-sets of the chains part `part` of `nparts` owns into the workspace `ws` (int32 modes)."""
     lib = _lib.load()
     H, W, K = pvec.shape
-    _lib.check(lib.flowb200_bcd_prepare(_ptr(pvec, torch.int32, "pvec"), _ptr(cost, _BCD_COST_DTYPE[mode], "cost"),
+    _lib.check(lib.flowb200_bcd_prepare(_ptr(pvec, torch.int32, "pvec"), _ptr(cost, _cost_dtype(mode), "cost"),
                                         _ptr(nprop, torch.int32, "nprop"), H, W, K, int(mode), float(lamda), int(tpsi),
                                         int(cost_shift), int(part), int(nparts), _ptr(ws), ws.numel(), _stream()),
                "flowb200_bcd_prepare")
@@ -169,7 +203,7 @@ def bcd_phase(pvec, cost, nprop, labels, ws, phase, part=0, nparts=1, mode=_lib.
     """Run the owned chains of one phase in place on labels (after bcd_prepare with the same workspace and part)."""
     lib = _lib.load()
     H, W, K = pvec.shape
-    _lib.check(lib.flowb200_bcd_phase(_ptr(pvec, torch.int32, "pvec"), _ptr(cost, _BCD_COST_DTYPE[mode], "cost"),
+    _lib.check(lib.flowb200_bcd_phase(_ptr(pvec, torch.int32, "pvec"), _ptr(cost, _cost_dtype(mode), "cost"),
                                       _ptr(nprop, torch.int32, "nprop"), _ptr(labels, torch.int32, "labels"), H, W, K,
                                       int(mode), float(lamda), int(tpsi), int(cost_shift), int(phase), int(part),
                                       int(nparts), _ptr(ws), ws.numel(), _stream()), "flowb200_bcd_phase")

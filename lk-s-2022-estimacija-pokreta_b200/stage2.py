@@ -7,6 +7,8 @@ kernels evaluate the same predicate on the fly.
 Arithmetic mode is chosen from the data so that labels equal the reference's float64 programme bit for bit:
   float32-representable costs -> FP64 mode on float32 costs; anything else -> FP64 mode on float64 costs;
   FLOWB200_BCD_INT32=1 requests the int32 mode and is honoured only if lamda*lcost*2^S is integral.
+FLOWB200_BCD_MRF=1 runs block coordinate descent on the MRF energy (include/flowb200.h FLOWB200_BCD_MRF) in whichever
+mode was chosen: the files written then differ from the reference's by design.
 """
 import os
 import sys
@@ -43,6 +45,8 @@ def run(picindex, backward, bcd_times, in_dir=".", out_dir=".", lamda=0.05, tpsi
             mode, cost = _lib.BCD_FP64_F32COST, torch.from_numpy(f32).cuda()
         else:
             cost = torch.from_numpy(np.ascontiguousarray(lcosts, dtype=np.float64)).cuda()
+    if os.environ.get("FLOWB200_BCD_MRF") == "1":
+        mode |= _lib.BCD_MRF
     snaps = ops.bcd(pvec, cost, g_nprop, g_lab, bcd_times, mode=mode, lamda=lamda, tpsi=tpsi, cost_shift=cost_shift,
                     per_sweep=True)
     for w in range(1, bcd_times + 1):
