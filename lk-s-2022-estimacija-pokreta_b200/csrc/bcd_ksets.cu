@@ -163,7 +163,7 @@ constexpr int kSortWarps = 8;
 constexpr int kCntSize = kHashSize + kHashSize / 32;   // 1056, a multiple of 4
 
 // single-huge-image mode: line (column x or row y) `line` of `nlines` belongs to chain line >> 1 of its parity's
-// phase; part `part` of `nparts` runs a contiguous share of every phase's chains (owned_chains on the host)
+// phase; part `part` of `nparts` runs a contiguous share of every phase's chains (the range of ksets_phase on the host)
 __device__ __forceinline__ bool owns_line(int line, int nlines, int part, int nparts) {
   const long long nch = (line & 1) ? nlines / 2 : (nlines + 1) / 2;
   const int c = line >> 1;
@@ -1062,19 +1062,22 @@ __global__ void __launch_bounds__(T, MINB) kset_chain32_mrf_kernel(const ChainAr
   chain32_body<CostT, T, SHIFT, true>(a);
 }
 
-// the variant of kset_chainf64_kernel a mode runs: the float64 programme (shift < 0) or the integer one.  Only variants
-// a mode can run are compiled: int32 costs come only with the int32 modes, double costs only with the float64 modes.
-template <typename CostT, int T>
-auto chainf64_kernel(int shift) {
-  if constexpr (std::is_integral<CostT>::value) return kset_chainf64_kernel<CostT, T, 1, true>;
-  else if constexpr (std::is_same<CostT, double>::value) return kset_chainf64_kernel<CostT, T, 1, false>;
-  else return shift < 0 ? kset_chainf64_kernel<CostT, T, 1, false> : kset_chainf64_kernel<CostT, T, 1, true>;
+// the kernels a mode runs.  Only variants a mode can run are compiled: int32 costs come only with the int32 modes,
+// double costs only with the float64 modes (no 32-bit kernel)
+template <typename CostT, int T, int MINB, bool MRF>
+auto chain32_kernel(int shift) {
+  if constexpr (std::is_same<CostT, double>::value) return (void (*)(const ChainArgs)) nullptr;
+  else if constexpr (MRF) return shift == 12 ? kset_chain32_mrf_kernel<CostT, T, MINB, 12> : kset_chain32_mrf_kernel<CostT, T, MINB, 0>;
+  else return shift == 12 ? kset_chain32_kernel<CostT, T, MINB, 12> : kset_chain32_kernel<CostT, T, MINB, 0>;
 }
-template <typename CostT, int T>
-auto chainf64_mrf_kernel(int shift) {
-  if constexpr (std::is_integral<CostT>::value) return kset_chainf64_mrf_kernel<CostT, T, 1, true>;
-  else if constexpr (std::is_same<CostT, double>::value) return kset_chainf64_mrf_kernel<CostT, T, 1, false>;
-  else return shift < 0 ? kset_chainf64_mrf_kernel<CostT, T, 1, false> : kset_chainf64_mrf_kernel<CostT, T, 1, true>;
+// the float64 kernel runs the float64 programme, or (QUANT) the integer one: int32 costs, and float costs in the int32
+// modes (shift >= 0)
+template <typename CostT, int T, bool MRF, bool QUANT = !std::is_same<CostT, double>::value>
+auto chainf64_kernel(int shift) {
+  if constexpr (std::is_same<CostT, float>::value && QUANT)
+    if (shift < 0) return chainf64_kernel<CostT, T, MRF, false>(shift);
+  if constexpr (MRF) return kset_chainf64_mrf_kernel<CostT, T, 1, QUANT>;
+  else return kset_chainf64_kernel<CostT, T, 1, QUANT>;
 }
 
 struct KsetLayout {
@@ -1111,15 +1114,6 @@ KsetLayout kset_layout(int H, int W, int K, size_t workspace_bytes) {
   return L;
 }
 
-// chains [c0, c1) of `phase` that part `part` of `nparts` owns (single-huge-image mode: a phase's independent chains
-// are split over the GPUs, python bcd.py:265-277 makes every chain of a phase independent of the others)
-static inline void owned_chains(int phase, int H, int W, int part, int nparts, int* c0, int* c1) {
-  const long long n = phase_chains(phase, H, W);
-  *c0 = (int)(n * part / nparts);
-  *c1 = (int)(n * (part + 1) / nparts);
-}
-
-template <typename CostT>
 struct KsetPlan {
   KsetLayout L;
   void (*kern32)(const ChainArgs) = nullptr;   // int32 modes: every chain, 32-bit dp; nullptr in the float64 modes
@@ -1132,15 +1126,49 @@ struct KsetPlan {
   size_t smem32[2] = {0, 0}, smem64 = 0;   // smem32: by chain orientation (column chains are H long, row chains W)
 };
 
+template <typename CostT>
+struct BcdProblem {   // the problem a BCD call solves, as the entry points receive it (cost typed for the mode)
+  const int32_t* pvec;
+  const CostT* cost;
+  const int32_t* nprop;
+  int H, W, K;
+  double lamda;
+  int tpsi, shift;   // shift -1: the float64 programme
+  bool mrf;          // FLOWB200_BCD_MRF
+};
+
+// the chain widths: T threads, one per label position, and the chains per SM aimed at (registers and shared memory)
+constexpr int kWidths[][2] = {{64, 8}, {128, 6}, {192, 5}, {256, 4}, {320, 4}, {384, 3}, {512, 2}};
+
+// the kernels of the first width that holds K; returns the chains per SM aimed at, 0 if no width holds K
+template <bool MRF, size_t I = 0, typename CostT>
+int pick_kernels(const BcdProblem<CostT>& pb, KsetPlan* P) {
+  constexpr int T = kWidths[I][0], MB = kWidths[I][1];
+  const int K = pb.K, shift = pb.shift;
+  if constexpr (I + 1 < sizeof(kWidths) / sizeof(kWidths[0]))
+    if (K > T) return pick_kernels<MRF, I + 1>(pb, P);
+  if (K > T) return 0;
+  constexpr int mb = MB > 4 ? 4 : MB;
+  constexpr int mb_lo = MRF ? mb : mb - (MB >= 4 ? 1 : 0);   // MRF: no variant for fewer chains per SM
+  if (shift >= 0) {
+    P->kern32 = chain32_kernel<CostT, T, mb, MRF>(shift);
+    P->kern32_lo = chain32_kernel<CostT, T, mb_lo, MRF>(shift);
+  }
+  P->minb = mb;
+  P->kernf64 = chainf64_kernel<CostT, T, MRF>(shift);
+  P->T = T;
+  return MB;
+}
+
 // shift < 0 selects the float64 programme (kset_chainf64_kernel): the records then carry no data costs, and no 32-bit
 // chain kernel is compiled (double costs) or set up.  Dropping the 32-bit kernel's shared-memory check there changes
 // nothing: the float64 kernel's check is stricter, its left side is 4*Kpad + 128 bytes larger at every chain length
 // mrf: the FLOWB200_BCD_MRF kernels, whose side vectors take 2 x len int32 of shared memory instead of len (the dp
 // bound holds as it is: a step adds at most the smaller of the two candidates, so at most tpsi over the minimum)
 template <typename CostT>
-static int make_plan(int H, int W, int K, int tpsi, int shift, bool mrf, size_t workspace_bytes, KsetPlan<CostT>* P) {
+static int make_plan(const BcdProblem<CostT>& pb, size_t workspace_bytes, KsetPlan* P) {
+  const int H = pb.H, W = pb.W, K = pb.K, tpsi = pb.tpsi, shift = pb.shift, nside = pb.mrf ? 2 : 1;
   if (K > 512 || tpsi < 0 || tpsi > 32) return FLOWB200_EUNSUPPORTED;
-  const int nside = mrf ? 2 : 1;
   P->records = tpsi >= 1 && tpsi <= 8 && (shift < 0 || shift >= 4);
   if (shift >= 0) {   // dp is a uint32
     const unsigned long long per_step = ((unsigned long long)(3 * tpsi) << shift) + 65535ull;
@@ -1150,30 +1178,7 @@ static int make_plan(int H, int W, int K, int tpsi, int shift, bool mrf, size_t 
   if (workspace_bytes < P->L.arena) return FLOWB200_EWORKSPACE;
   const int Kpad = P->L.Kpad;
   while ((1 << P->bshift) < tpsi) ++P->bshift;
-  // one thread per label position; MB = chains per SM aimed at (registers and shared memory)
-  int minb = 1;
-#define FB_KS_CASE(TT, MB)                                                                                   \
-  if (!P->kernf64 && K <= TT) {                                                                              \
-    constexpr int mb = MB > 4 ? 4 : MB, mb_lo = mb - (MB >= 4 ? 1 : 0);                                      \
-    if constexpr (!std::is_same<CostT, double>::value) {                                                     \
-      if (shift >= 0 && mrf) {   /* one instantiation per width: no variant for fewer chains per SM */       \
-        P->kern32 = shift == 12 ? kset_chain32_mrf_kernel<CostT, TT, mb, 12>                                 \
-                                : kset_chain32_mrf_kernel<CostT, TT, mb, 0>;                                 \
-        P->kern32_lo = P->kern32;                                                                            \
-      } else if (shift >= 0) {                                                                               \
-        P->kern32 = shift == 12 ? kset_chain32_kernel<CostT, TT, mb, 12> : kset_chain32_kernel<CostT, TT, mb, 0>;\
-        P->kern32_lo = shift == 12 ? kset_chain32_kernel<CostT, TT, mb_lo, 12>                               \
-                                   : kset_chain32_kernel<CostT, TT, mb_lo, 0>;                               \
-      }                                                                                                      \
-    }                                                                                                        \
-    P->minb = mb;                                                                                            \
-    P->kernf64 = mrf ? chainf64_mrf_kernel<CostT, TT>(shift) : chainf64_kernel<CostT, TT>(shift);            \
-    P->T = TT;                                                                                               \
-    minb = MB;                                                                                               \
-  }
-  FB_KS_CASE(64, 8) FB_KS_CASE(128, 6) FB_KS_CASE(192, 5) FB_KS_CASE(256, 4) FB_KS_CASE(320, 4)
-  FB_KS_CASE(384, 3) FB_KS_CASE(512, 2)
-#undef FB_KS_CASE
+  const int minb = pb.mrf ? pick_kernels<true>(pb, P) : pick_kernels<false>(pb, P);
   if (!P->kernf64) return FLOWB200_EUNSUPPORTED;
   // ring of record slots: as many (<= 4) as keep `minb` chains per SM resident
   const int maxlen = H > W ? H : W;
@@ -1199,16 +1204,15 @@ static int make_plan(int H, int W, int K, int tpsi, int shift, bool mrf, size_t 
 
 // sort + record build for the chains this part owns
 template <typename CostT>
-int ksets_prepare(const int32_t* pvec, const CostT* cost, const int32_t* nprop, int H, int W, int K, double lamda,
-                  int tpsi, int shift, bool mrf, int part, int nparts, void* workspace, size_t workspace_bytes,
+int ksets_prepare(const BcdProblem<CostT>& pb, int part, int nparts, void* workspace, size_t workspace_bytes,
                   cudaStream_t stream) {
   if (nparts < 1 || part < 0 || part >= nparts) return FLOWB200_EINVAL;
-  KsetPlan<CostT> P;
-  const int rc = make_plan<CostT>(H, W, K, tpsi, shift, mrf, workspace_bytes, &P);
+  KsetPlan P;
+  const int rc = make_plan(pb, workspace_bytes, &P);
   if (rc) return rc;
   const KsetLayout& L = P.L;
   char* ws = static_cast<char*>(workspace);
-  const int npix = H * W;
+  const int H = pb.H, W = pb.W, K = pb.K, shift = pb.shift, npix = H * W;
   if (!P.records) {   // every descriptor 0: the chain kernels evaluate every step densely
     FB_CUDA_CHECK(cudaMemsetAsync(ws + L.desc, 0, 2 * (size_t)npix * sizeof(unsigned long long), stream));
     return FLOWB200_OK;
@@ -1218,51 +1222,45 @@ int ksets_prepare(const int32_t* pvec, const CostT* cost, const int32_t* nprop, 
   FB_CUDA_CHECK(cudaMemsetAsync(cursor, 0, sizeof(unsigned long long), stream));
   int32_t* svec = reinterpret_cast<int32_t*>(ws + L.svec);
   kset_sort_kernel<<<min((npix + kSortWarps - 1) / kSortWarps, 8 * kNumSMs), kSortWarps * 32, 0, stream>>>(
-      pvec, nprop, npix, K, L.Kst, P.bshift, sorig, svec, H, W, part, nparts);
+      pb.pvec, pb.nprop, npix, K, L.Kst, P.bshift, sorig, svec, H, W, part, nparts);
   FB_LAUNCH_CHECK();
   const size_t bsmem = build_smem_bytes(L.Kpad);
   auto bk = kset_build_kernel<CostT>;
   FB_CUDA_CHECK(cudaFuncSetAttribute(bk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem));
   const int bctas = std::min(16, (int)(227 * 1024 / (bsmem + 1024)));
   bk<<<min(2 * npix, max(1, bctas) * kNumSMs), kBuildThreads, bsmem, stream>>>(
-      pvec, cost, nprop, sorig, svec, H, W, K, L.Kst, L.Kpad, tpsi, P.bshift, shift < 0 ? 0 : shift, shift < 0 ? 0.0 : lamda,
-      P.slot_bytes,
-      reinterpret_cast<unsigned char*>(ws + L.arena), (unsigned long long)L.arena_bytes, cursor,
-      reinterpret_cast<unsigned long long*>(ws + L.desc), part, nparts);
+      pb.pvec, pb.cost, pb.nprop, sorig, svec, H, W, K, L.Kst, L.Kpad, pb.tpsi, P.bshift, shift < 0 ? 0 : shift,
+      shift < 0 ? 0.0 : pb.lamda, P.slot_bytes, reinterpret_cast<unsigned char*>(ws + L.arena),
+      (unsigned long long)L.arena_bytes, cursor, reinterpret_cast<unsigned long long*>(ws + L.desc), part, nparts);
   FB_LAUNCH_CHECK();
   return FLOWB200_OK;
 }
 
 // one phase, the chains this part owns, in place on labels
 template <typename CostT>
-int ksets_phase(const int32_t* pvec, const CostT* cost, const int32_t* nprop, int32_t* labels, int H, int W, int K,
-                double lamda, int tpsi, int shift, bool mrf, int phase, int part, int nparts, void* workspace,
+int ksets_phase(const BcdProblem<CostT>& pb, int32_t* labels, int phase, int part, int nparts, void* workspace,
                 size_t workspace_bytes, cudaStream_t stream) {
   if (nparts < 1 || part < 0 || part >= nparts || phase < 0 || phase > 3) return FLOWB200_EINVAL;
-  KsetPlan<CostT> P;
-  const int rc = make_plan<CostT>(H, W, K, tpsi, shift, mrf, workspace_bytes, &P);
+  KsetPlan P;
+  const int rc = make_plan(pb, workspace_bytes, &P);
   if (rc) return rc;
   const KsetLayout& L = P.L;
   char* ws = static_cast<char*>(workspace);
-  int c0, c1;
-  owned_chains(phase, H, W, part, nparts, &c0, &c1);
+  // this part's chains [c0, c1) (single-huge-image mode; the chains of a phase are independent, python bcd.py:265-277)
+  const long long nch = phase_chains(phase, pb.H, pb.W);
+  const int c0 = (int)(nch * part / nparts), c1 = (int)(nch * (part + 1) / nparts);
   if (c1 <= c0) return FLOWB200_OK;
   ChainArgs a{};
-  a.pvec = pvec;
-  a.cost = cost;
-  a.nprop = nprop;
-  a.labels = labels;
+  a.pvec = pb.pvec; a.cost = pb.cost; a.nprop = pb.nprop; a.labels = labels;
   a.bp = reinterpret_cast<uint16_t*>(ws + L.bp);
   a.desc = reinterpret_cast<const unsigned long long*>(ws + L.desc);
   a.arena = reinterpret_cast<const unsigned char*>(ws + L.arena);
-  a.H = H; a.W = W; a.K = K; a.Kpad = L.Kpad; a.tpsi = tpsi; a.shift = shift; a.slot_shift = P.slot_shift;
-  a.slot_bytes = P.slot_bytes;
-  a.lamda = lamda;
-  a.phase = phase;
-  a.chain0 = c0;
+  a.H = pb.H; a.W = pb.W; a.K = pb.K; a.Kpad = L.Kpad; a.tpsi = pb.tpsi; a.shift = pb.shift;
+  a.slot_shift = P.slot_shift; a.slot_bytes = P.slot_bytes;
+  a.lamda = pb.lamda; a.phase = phase; a.chain0 = c0;
   a.flags = reinterpret_cast<int32_t*>(ws + L.flags);
   a.force_generic = getenv("FLOWB200_KSET_FORCE_GENERIC") != nullptr;   // read at every call (tests)
-  if (shift >= 0) {
+  if (pb.shift >= 0) {
     // (1300: static shared memory + the driver's 1 KB per CTA)
     const bool fits = (size_t)P.minb * (P.smem32[phase & 1] + 1300) <= (size_t)227 * 1024;
     (fits ? P.kern32 : P.kern32_lo)<<<c1 - c0, P.T, P.smem32[phase & 1], stream>>>(a);
@@ -1275,30 +1273,38 @@ int ksets_phase(const int32_t* pvec, const CostT* cost, const int32_t* nprop, in
 }
 
 template <typename CostT>
-int launch_sweeps_ksets(const int32_t* pvec, const CostT* cost, const int32_t* nprop, int32_t* labels, int H, int W,
-                        int K, double lamda, int tpsi, int shift, bool mrf, int sweeps, int32_t* labels_per_sweep,
+int launch_sweeps_ksets(const BcdProblem<CostT>& pb, int32_t* labels, int sweeps, int32_t* labels_per_sweep,
                         void* workspace, size_t workspace_bytes, cudaStream_t stream) {
-  if (sweeps <= 0) {
-    KsetPlan<CostT> P;
-    return make_plan<CostT>(H, W, K, tpsi, shift, mrf, workspace_bytes, &P);
+  if (sweeps <= 0) {   // the plan only
+    KsetPlan P;
+    return make_plan(pb, workspace_bytes, &P);
   }
-  int rc = ksets_prepare<CostT>(pvec, cost, nprop, H, W, K, lamda, tpsi, shift, mrf, 0, 1, workspace, workspace_bytes,
-                                stream);
+  int rc = ksets_prepare(pb, 0, 1, workspace, workspace_bytes, stream);
   if (rc) return rc;
   for (int w = 0; w < sweeps; ++w) {
     for (int phase = 0; phase < 4; ++phase) {
-      rc = ksets_phase<CostT>(pvec, cost, nprop, labels, H, W, K, lamda, tpsi, shift, mrf, phase, 0, 1, workspace,
-                              workspace_bytes, stream);
+      rc = ksets_phase(pb, labels, phase, 0, 1, workspace, workspace_bytes, stream);
       if (rc) return rc;
     }
     if (labels_per_sweep)
-      FB_CUDA_CHECK(cudaMemcpyAsync(labels_per_sweep + (size_t)w * H * W, labels, sizeof(int32_t) * H * W,
+      FB_CUDA_CHECK(cudaMemcpyAsync(labels_per_sweep + (size_t)w * pb.H * pb.W, labels, sizeof(int32_t) * pb.H * pb.W,
                                     cudaMemcpyDeviceToDevice, stream));
   }
   return FLOWB200_OK;
 }
 
-bool is_int_mode(int bcd_mode) { return bcd_mode == FLOWB200_BCD_INT32 || bcd_mode == FLOWB200_BCD_INT32_F32COST; }
+// The checks the entry points share, after their null-pointer checks; splits the FLOWB200_BCD_MRF flag off *bcd_mode.
+// chains: K <= 512 and H, W <= 16384.  int_modes_only (prepare / phase): the cost shift checked in every mode, then
+// every other mode (stray bits too) unsupported; else the shift checked in the int32 modes, the mode by with_mode.
+int check_args(int H, int W, int K, int cost_shift, int* bcd_mode, bool* mrf, bool chains, bool int_modes_only) {
+  if (H <= 0 || W <= 0 || K <= 0) return FLOWB200_EINVAL;
+  if (chains && (K > 512 || H > 16384 || W > 16384)) return FLOWB200_EINVAL;
+  *mrf = (*bcd_mode & FLOWB200_BCD_MRF) != 0;
+  *bcd_mode &= ~FLOWB200_BCD_MRF;
+  const bool int_mode = *bcd_mode == FLOWB200_BCD_INT32 || *bcd_mode == FLOWB200_BCD_INT32_F32COST;
+  if ((int_mode || int_modes_only) && (cost_shift < 0 || cost_shift > 14)) return FLOWB200_EINVAL;
+  return int_modes_only && !int_mode ? FLOWB200_EUNSUPPORTED : FLOWB200_OK;
+}
 
 // run(cost, shift) with the cost array typed for bcd_mode; shift -1 selects the float64 programme
 template <typename Run>
@@ -1342,15 +1348,13 @@ extern "C" int flowb200_bcd(const int32_t* pvec, const void* cost, const int32_t
                             int32_t* labels_per_sweep, void* workspace, size_t workspace_bytes,
                             flowb200_stream_t stream) {
   if (!pvec || !cost || !nprop || !labels || !workspace) return FLOWB200_EINVAL;
-  if (H <= 0 || W <= 0 || K <= 0 || K > 512 || sweeps < 0 || tpsi < 0) return FLOWB200_EINVAL;
-  if (H > 16384 || W > 16384) return FLOWB200_EINVAL;
-  const bool mrf = (bcd_mode & FLOWB200_BCD_MRF) != 0;
-  bcd_mode &= ~FLOWB200_BCD_MRF;
-  if (is_int_mode(bcd_mode) && (cost_shift < 0 || cost_shift > 14)) return FLOWB200_EINVAL;
+  if (sweeps < 0 || tpsi < 0) return FLOWB200_EINVAL;   // (tpsi > 32: make_plan)
+  bool mrf;
+  if (const int rc = check_args(H, W, K, cost_shift, &bcd_mode, &mrf, true, false)) return rc;
   // any workspace that holds the fixed part is accepted: records that do not fit are evaluated densely
   return with_mode(bcd_mode, cost, cost_shift, [&](auto c, int shift) {
-    return launch_sweeps_ksets(pvec, c, nprop, labels, H, W, K, lamda, tpsi, shift, mrf, sweeps, labels_per_sweep,
-                               workspace, workspace_bytes, stream);
+    const BcdProblem<std::decay_t<decltype(*c)>> pb{pvec, c, nprop, H, W, K, lamda, tpsi, shift, mrf};
+    return launch_sweeps_ksets(pb, labels, sweeps, labels_per_sweep, workspace, workspace_bytes, stream);
   });
 }
 
@@ -1359,14 +1363,11 @@ extern "C" int flowb200_bcd_prepare(const int32_t* pvec, const void* cost, const
                                     int bcd_mode, double lamda, int tpsi, int cost_shift, int part, int nparts,
                                     void* workspace, size_t workspace_bytes, flowb200_stream_t stream) {
   if (!pvec || !cost || !nprop || !workspace) return FLOWB200_EINVAL;
-  if (H <= 0 || W <= 0 || K <= 0 || K > 512 || H > 16384 || W > 16384) return FLOWB200_EINVAL;
-  if (cost_shift < 0 || cost_shift > 14) return FLOWB200_EINVAL;
-  const bool mrf = (bcd_mode & FLOWB200_BCD_MRF) != 0;
-  bcd_mode &= ~FLOWB200_BCD_MRF;
-  if (!is_int_mode(bcd_mode)) return FLOWB200_EUNSUPPORTED;
+  bool mrf;
+  if (const int rc = check_args(H, W, K, cost_shift, &bcd_mode, &mrf, true, true)) return rc;
   return with_mode(bcd_mode, cost, cost_shift, [&](auto c, int shift) {
-    return ksets_prepare(pvec, c, nprop, H, W, K, lamda, tpsi, shift, mrf, part, nparts, workspace, workspace_bytes,
-                         stream);
+    const BcdProblem<std::decay_t<decltype(*c)>> pb{pvec, c, nprop, H, W, K, lamda, tpsi, shift, mrf};
+    return ksets_prepare(pb, part, nparts, workspace, workspace_bytes, stream);
   });
 }
 
@@ -1374,14 +1375,11 @@ extern "C" int flowb200_bcd_phase(const int32_t* pvec, const void* cost, const i
                                   int W, int K, int bcd_mode, double lamda, int tpsi, int cost_shift, int phase, int part,
                                   int nparts, void* workspace, size_t workspace_bytes, flowb200_stream_t stream) {
   if (!pvec || !cost || !nprop || !labels || !workspace) return FLOWB200_EINVAL;
-  if (H <= 0 || W <= 0 || K <= 0 || K > 512 || H > 16384 || W > 16384) return FLOWB200_EINVAL;
-  if (cost_shift < 0 || cost_shift > 14) return FLOWB200_EINVAL;
-  const bool mrf = (bcd_mode & FLOWB200_BCD_MRF) != 0;
-  bcd_mode &= ~FLOWB200_BCD_MRF;
-  if (!is_int_mode(bcd_mode)) return FLOWB200_EUNSUPPORTED;
+  bool mrf;
+  if (const int rc = check_args(H, W, K, cost_shift, &bcd_mode, &mrf, true, true)) return rc;
   return with_mode(bcd_mode, cost, cost_shift, [&](auto c, int shift) {
-    return ksets_phase(pvec, c, nprop, labels, H, W, K, lamda, tpsi, shift, mrf, phase, part, nparts, workspace,
-                       workspace_bytes, stream);
+    const BcdProblem<std::decay_t<decltype(*c)>> pb{pvec, c, nprop, H, W, K, lamda, tpsi, shift, mrf};
+    return ksets_phase(pb, labels, phase, part, nparts, workspace, workspace_bytes, stream);
   });
 }
 
@@ -1389,9 +1387,9 @@ extern "C" int flowb200_energy(const int32_t* pvec, const void* cost, const int3
                                int H, int W, int K, int bcd_mode, double lamda, int tpsi, int cost_shift, double* out4,
                                flowb200_stream_t stream) {
   if (!pvec || !cost || !nprop || !labels || !out4) return FLOWB200_EINVAL;
-  if (H <= 0 || W <= 0 || K <= 0 || tpsi < 0 || (long long)H * W > 0x7FFFFFFFll) return FLOWB200_EINVAL;
-  bcd_mode &= ~FLOWB200_BCD_MRF;   // the energy does not depend on the optimiser
-  if (is_int_mode(bcd_mode) && (cost_shift < 0 || cost_shift > 14)) return FLOWB200_EINVAL;
+  if (tpsi < 0 || (long long)H * W > 0x7FFFFFFFll) return FLOWB200_EINVAL;
+  bool mrf;   // (the energy does not depend on the optimiser)
+  if (const int rc = check_args(H, W, K, cost_shift, &bcd_mode, &mrf, false, false)) return rc;
   return with_mode(bcd_mode, cost, cost_shift, [&](auto c, int shift) {
     using CostT = std::remove_const_t<std::remove_pointer_t<decltype(c)>>;
     // (only the variants a mode can run, as for the chain kernels)

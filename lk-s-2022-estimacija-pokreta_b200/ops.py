@@ -128,16 +128,22 @@ def _cost_dtype(mode):
     return _BCD_COST_DTYPE[mode & ~_lib.BCD_MRF]
 
 
+def _bcd_args(pvec, cost, nprop, mode, lamda, tpsi, cost_shift, *labels):
+    """The arguments the BCD entry points begin with: pvec, cost, nprop[, labels], H, W, K, mode, lamda, tpsi,
+    cost_shift (flowb200_bcd_prepare takes no labels)."""
+    H, W, K = pvec.shape
+    ptrs = [_ptr(pvec, torch.int32, "pvec"), _ptr(cost, _cost_dtype(mode), "cost"), _ptr(nprop, torch.int32, "nprop")]
+    ptrs += [_ptr(t, torch.int32, "labels") for t in labels]
+    return (*ptrs, H, W, K, int(mode), float(lamda), int(tpsi), int(cost_shift))
+
+
 def energy(pvec, cost, nprop, labels, mode=_lib.BCD_FP64_F32COST, lamda=0.05, tpsi=8, cost_shift=12):
     """The MRF energy of labels in the arithmetic of `mode` (flowb200_energy): (data, pairwise, total, n_bad), n_bad =
     pixels whose label is outside [0, nprop), left out of both terms.  Exact in the int32 modes."""
     lib = _lib.load()
-    H, W, K = pvec.shape
     out = torch.empty(4, dtype=torch.float64, device=pvec.device)
-    _lib.check(lib.flowb200_energy(_ptr(pvec, torch.int32, "pvec"), _ptr(cost, _cost_dtype(mode), "cost"),
-                                   _ptr(nprop, torch.int32, "nprop"), _ptr(labels, torch.int32, "labels"), H, W, K,
-                                   int(mode), float(lamda), int(tpsi), int(cost_shift), _ptr(out), _stream()),
-               "flowb200_energy")
+    _lib.check(lib.flowb200_energy(*_bcd_args(pvec, cost, nprop, mode, lamda, tpsi, cost_shift, labels), _ptr(out),
+                                   _stream()), "flowb200_energy")
     data, pair, total, bad = out.tolist()
     return data, pair, total, int(bad)
 
@@ -167,11 +173,8 @@ def bcd(pvec, cost, nprop, labels, sweeps, mode=_lib.BCD_FP64_F32COST, lamda=0.0
             if per_sweep:
                 snaps[w].copy_(labels)
         return snaps, energies
-    rc = lib.flowb200_bcd(_ptr(pvec, torch.int32, "pvec"), _ptr(cost, _cost_dtype(mode), "cost"),
-                          _ptr(nprop, torch.int32, "nprop"), _ptr(labels, torch.int32, "labels"), H, W, K, int(mode),
-                          float(lamda), int(tpsi), int(cost_shift), int(sweeps), _ptr(snaps), _ptr(ws), ws.numel(),
-                          _stream())
-    _lib.check(rc, "flowb200_bcd")
+    _lib.check(lib.flowb200_bcd(*_bcd_args(pvec, cost, nprop, mode, lamda, tpsi, cost_shift, labels), int(sweeps),
+                                _ptr(snaps), _ptr(ws), ws.numel(), _stream()), "flowb200_bcd")
     return snaps
 
 
@@ -191,22 +194,16 @@ def bcd_workspace(pvec, nparts=1):
 def bcd_prepare(pvec, cost, nprop, ws, part=0, nparts=1, mode=_lib.BCD_INT32_F32COST, lamda=0.05, tpsi=8, cost_shift=12):
     """Compile the K-sets of the chains part `part` of `nparts` owns into the workspace `ws` (int32 modes)."""
     lib = _lib.load()
-    H, W, K = pvec.shape
-    _lib.check(lib.flowb200_bcd_prepare(_ptr(pvec, torch.int32, "pvec"), _ptr(cost, _cost_dtype(mode), "cost"),
-                                        _ptr(nprop, torch.int32, "nprop"), H, W, K, int(mode), float(lamda), int(tpsi),
-                                        int(cost_shift), int(part), int(nparts), _ptr(ws), ws.numel(), _stream()),
-               "flowb200_bcd_prepare")
+    _lib.check(lib.flowb200_bcd_prepare(*_bcd_args(pvec, cost, nprop, mode, lamda, tpsi, cost_shift), int(part),
+                                        int(nparts), _ptr(ws), ws.numel(), _stream()), "flowb200_bcd_prepare")
 
 
 def bcd_phase(pvec, cost, nprop, labels, ws, phase, part=0, nparts=1, mode=_lib.BCD_INT32_F32COST, lamda=0.05, tpsi=8,
               cost_shift=12):
     """Run the owned chains of one phase in place on labels (after bcd_prepare with the same workspace and part)."""
     lib = _lib.load()
-    H, W, K = pvec.shape
-    _lib.check(lib.flowb200_bcd_phase(_ptr(pvec, torch.int32, "pvec"), _ptr(cost, _cost_dtype(mode), "cost"),
-                                      _ptr(nprop, torch.int32, "nprop"), _ptr(labels, torch.int32, "labels"), H, W, K,
-                                      int(mode), float(lamda), int(tpsi), int(cost_shift), int(phase), int(part),
-                                      int(nparts), _ptr(ws), ws.numel(), _stream()), "flowb200_bcd_phase")
+    _lib.check(lib.flowb200_bcd_phase(*_bcd_args(pvec, cost, nprop, mode, lamda, tpsi, cost_shift, labels), int(phase),
+                                      int(part), int(nparts), _ptr(ws), ws.numel(), _stream()), "flowb200_bcd_phase")
 
 
 def best_labels(lcost, nprop):

@@ -67,7 +67,7 @@ def bucket_shift(tpsi):
 
 
 def chain_width(K):
-    """T of make_plan's FB_KS_CASE table and the chains per SM it aims at."""
+    """T of make_plan's width table (kWidths) and the chains per SM it aims at."""
     return next((T, mb) for T, mb in ((64, 8), (128, 6), (192, 5), (256, 4), (320, 4), (384, 3), (512, 2)) if K <= T)
 
 

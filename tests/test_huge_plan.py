@@ -186,7 +186,7 @@ class _OracleOps:
         geo = [(1, 0, [(0, x) for x in range(0, W, 2)]), (0, -1, [(y, W - 1) for y in range(0, H, 2)]),
                (-1, 0, [(H - 1, x) for x in range(1, W, 2)]), (0, 1, [(y, 0) for y in range(1, H, 2)])][phase]
         n = len(geo[2])
-        mine = geo[2][n * part // nparts:n * (part + 1) // nparts]     # owned_chains() of csrc/bcd_ksets.cu
+        mine = geo[2][n * part // nparts:n * (part + 1) // nparts]     # ksets_phase's chain range, csrc/bcd_ksets.cu
         if mine:
             lab = labels.numpy().astype(np.int64)
             obcd._phase(self.prop, self.lc, self.nprop, lab, 8, 0.05, geo[0], geo[1], mine)
