@@ -134,7 +134,8 @@ int flowb200_random_proposals(const float* desc_src, const float* desc_tgt, cons
 int flowb200_ksets_pack(const int32_t* pvec, const int32_t* nprop, int H, int W, int K, int tpsi,
                         uint8_t* packed, flowb200_stream_t stream);
 
-/* lamda*lcost -> integer units of 2^-S (rint), unused slots -> 0.  m: int32 [n] */
+/* lamda*lcost -> integer units of 2^-S (rint), unused slots -> 0.  m: int32 [n]; n = 0 does nothing (pointers may be
+ * null then) */
 int flowb200_quantise_costs(const float* lcost, int32_t* m, size_t n, double lamda, int shift,
                             flowb200_stream_t stream);
 
@@ -201,7 +202,8 @@ int flowb200_flow_from_labels(const int32_t* pvec, const int32_t* labels, int H,
 
 /* ---- A13/A14  consistencyCheck / fowardBackwardConsistency (postprocessing.py:79-117) ----
  * flow1 (in place) and flow2: float32 [A][B][3] = (dx, dy, valid).  Quirk Q5 (dx added to the row index)
- * is reproduced.  Only pixels a0<=a<a1, b0<=b<b1 are checked (whole image: 0,A,0,B). */
+ * is reproduced.  Only pixels a0<=a<a1, b0<=b<b1 are checked (whole image: 0,A,0,B).  A valid pixel whose target
+ * coordinate is NaN (the reference's int() would raise) counts as out of range and is zeroed, like +-inf. */
 int flowb200_consistency(float* flow1, const float* flow2, int A, int B, float tresh,
                          int a0, int a1, int b0, int b1, flowb200_stream_t stream);
 

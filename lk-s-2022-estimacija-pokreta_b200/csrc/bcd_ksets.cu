@@ -1403,8 +1403,9 @@ extern "C" int flowb200_energy(const int32_t* pvec, const void* cost, const int3
 
 extern "C" int flowb200_quantise_costs(const float* lcost, int32_t* m, size_t n, double lamda, int shift,
                                        flowb200_stream_t stream) {
-  if (!lcost || !m || shift < 0 || shift > 14) return FLOWB200_EINVAL;
-  if (n == 0) return FLOWB200_OK;
+  if (shift < 0 || shift > 14) return FLOWB200_EINVAL;
+  if (n == 0) return FLOWB200_OK;          // (an empty tensor's pointers are null)
+  if (!lcost || !m) return FLOWB200_EINVAL;
   quantise_costs_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(lcost, m, n, lamda, (double)(1 << shift));
   FB_LAUNCH_CHECK();
   return FLOWB200_OK;

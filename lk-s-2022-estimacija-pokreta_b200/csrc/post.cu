@@ -38,9 +38,12 @@ __global__ void consistency_kernel(float* __restrict__ f1, const float* __restri
   size_t o = 3 * ((size_t)a * B + b);
   float u = f1[o], v = f1[o + 1], val = f1[o + 2];
   if (!(val > 0.5f)) return;
-  int a2 = (int)__fadd_rn(u, (float)a);   // int() truncates toward zero
-  int b2 = (int)__fadd_rn(v, (float)b);
-  bool bad = (a2 < 0 || b2 < 0 || a2 >= A || b2 >= B);
+  const float fa = __fadd_rn(u, (float)a), fb = __fadd_rn(v, (float)b);
+  int a2 = (int)fa;   // int() truncates toward zero; +-inf saturates to INT_MAX / INT_MIN: out of range
+  int b2 = (int)fb;
+  // The conversion turns NaN into 0, a valid row / column.  The reference's int() raises on NaN and the oracle's cast
+  // gives INT64_MIN: a NaN coordinate is out of range, so the pixel is zeroed (deliberate difference, DESIGN section 1).
+  bool bad = (isnan(fa) || isnan(fb) || a2 < 0 || b2 < 0 || a2 >= A || b2 >= B);
   if (!bad) {
     size_t o2 = 3 * ((size_t)a2 * B + b2);
     float u2 = f2[o2], v2 = f2[o2 + 1], val2 = f2[o2 + 2];

@@ -4,6 +4,7 @@ Everything goes through the C ABI (libflowb200.so) via the package's ctypes laye
 bit-exact for labels, proposals, nprop, K-set bits, kNN indices, the consistency field and the
 float32 data costs; DAISY within 1e-4 relative to the per-descriptor maximum (north star).
 """
+import ctypes as C
 import os
 
 import numpy as np
@@ -16,6 +17,7 @@ pytestmark = pytest.mark.gpu
 
 KNN_MODES = [0, 1]    # 0 = float64 CUDA cores, 1 = tcgen05 prefilter + exact re-rank
 DAISY_RTOL = 1e-4      # BASELINE.json north_star: "DAISY must agree within 1e-4 relative"
+F32 = np.float32
 
 
 def dev(a, dtype=None):
@@ -419,6 +421,33 @@ def test_quantise_costs():
     assert np.array_equal(m, want)
 
 
+@pytest.mark.parametrize("shift", range(15))
+def test_quantise_costs_every_shift(shift):
+    """m = rint((lamda * c) * 2^S) in float64, 1000.0 (an unused slot) -> 0, at every shift: uniform costs, costs whose
+    product lands exactly half-way (lamda 0.5, c = (2j+1) / 2^S: rint rounds half to even), the float32 neighbours of
+    1000.0 (quantised), and n = 0, 1, 255, 257 (not a multiple of the block); shifts -1 and 15 are refused."""
+    ops, lib = pkg("ops"), pkg("_lib")
+    rng = np.random.default_rng(shift)
+    S = float(1 << shift)
+    c = rng.uniform(0, 2.5, (9, 11, 20)).astype(np.float32)
+    c[..., 15:] = 1000.0
+    ties = ((2 * np.arange(300) + 1) / S).astype(np.float32)
+    thousand = np.array([np.nextafter(F32(1000), F32(0)), 1000.0, np.nextafter(F32(1000), F32(np.inf))], np.float32)
+    arrays = [c, ties, thousand] + [rng.uniform(0, 3, n).astype(np.float32) for n in (0, 1, 255, 257)]
+    for lamda in (0.05, 0.5, 1.0):
+        for a in arrays:
+            want = np.where(a == 1000.0, 0, np.rint((lamda * a.astype(np.float64)) * S)).astype(np.int32)
+            m = ops.quantise_costs(dev(a), lamda, shift).cpu().numpy()
+            assert m.shape == a.shape and np.array_equal(m, want), (lamda, a.shape)
+    # j + 1/2 rounds to the even neighbour
+    assert np.array_equal(ops.quantise_costs(dev(ties), 0.5, shift).cpu().numpy(), 2 * ((np.arange(300) + 1) // 2))
+    m = torch.zeros(3, dtype=torch.int32, device="cuda")
+    for bad in (-1, 15):
+        rc = lib.load().flowb200_quantise_costs(C.c_void_p(dev(thousand).data_ptr()), C.c_void_p(m.data_ptr()), 3, 0.05,
+                                                bad, C.c_void_p(torch.cuda.current_stream().cuda_stream))
+        assert rc == lib.EINVAL
+
+
 def test_epe_metric_matches_error_image():
     from oracle import epe as oepe
     ops = pkg("ops")
@@ -639,3 +668,43 @@ def test_best_labels_kernel():
     d1, d2 = ops.daisy(dev(a)), ops.daisy(dev(b))
     pv, lcost, nprop, labels = ops.knn_proposals(d1, d2, p)
     assert torch.equal(ops.best_labels(lcost, nprop), labels)
+
+
+@pytest.mark.parametrize("K", [1, 31, 32, 33, 64, 65, 512])
+def test_best_labels_kernel_edges(K):
+    """flowb200_best_labels = the first strict minimum of the first nprop data costs (daisy i flann.py:181-184), ties and
+    empty pixels included, at K around the warp width: nprop 0, 1, 31, 32, 33 and K; equal minima 32 slots apart (one
+    lane) and 1 apart (two lanes); a smaller cost at slot nprop (ignored); costs 0, 1e-45 (subnormal), 1000 and +inf.
+    (Costs are >= 0 and not -0.0: the kernel orders them by their bits.)"""
+    ops = pkg("ops")
+    rng = np.random.default_rng(8 + K)
+    H, W = 37, 53
+    lc = rng.integers(0, 6, (H, W, K)).astype(np.float32) * 0.25          # many ties
+    npr = np.where(rng.random((H, W)) < 0.5, rng.choice([0, 1, 31, 32, 33, K], (H, W)),
+                   rng.integers(0, K + 1, (H, W))).clip(0, K).astype(np.int32)
+    special = np.array([0.0, 1e-45, 1000.0, np.inf], np.float32)
+    assert special[1] > 0                                                  # the smallest subnormal, not flushed
+    flat_c, flat_n = lc.reshape(H * W, K), npr.reshape(H * W)
+    for p in range(H * W):
+        n, kind = int(flat_n[p]), p % 5
+        if kind == 0 and n > 32:                     # equal minima at s and s + 32
+            s = int(rng.integers(0, n - 32))
+            flat_c[p, :n] = rng.uniform(1, 2, n)
+            flat_c[p, [s, s + 32]] = 0.5
+        elif kind == 1 and n > 1:                    # equal minima at s and s + 1
+            s = int(rng.integers(0, n - 1))
+            flat_c[p, :n] = rng.uniform(1, 2, n)
+            flat_c[p, [s, s + 1]] = 0.5
+        elif kind == 2 and n < K:                    # a smaller cost just past nprop
+            flat_c[p, :n] = rng.uniform(1, 2, n)
+            flat_c[p, n] = 0.0
+        elif kind == 3:                              # special values inside nprop
+            flat_c[p, :n] = special[rng.integers(0, 4, n)]
+        elif kind == 4:                              # mostly 1000 / +inf, one subnormal
+            flat_c[p, :n] = special[rng.integers(2, 4, n)]
+            if n:
+                flat_c[p, int(rng.integers(0, n))] = special[1]
+    want = np.array([int(np.argmin(flat_c[p, :flat_n[p]])) if flat_n[p] else 0 for p in range(H * W)],
+                    np.int32).reshape(H, W)
+    got = ops.best_labels(dev(lc), dev(npr)).cpu().numpy()
+    assert np.array_equal(got, want)
