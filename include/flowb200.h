@@ -123,7 +123,12 @@ int flowb200_knn_debug_scores(const float* desc_src, const float* desc_tgt, cons
 
 /* ---- A6  nasumicni  (daisy i flann.py:205-233), quirks Q4/Q6 reproduced ----
  * draws: optional int16 [H][W][n_gauss][2] accepted in-bounds (tgy,tgx) samples to replay (parity mode);
- * NULL -> Philox4x32-10 Gaussian draws from `seed` with the reference's rejection rules. */
+ * NULL -> Philox4x32-10 Gaussian draws from `seed` with the reference's rejection rules: counter (pixel, attempt, 0, 0),
+ * key (seed low word, seed high word), u = (r + 0.5) 2^-32, z = sqrt(-2 log u0) cospi(2 u1) for y (words 0, 1) and x
+ * (words 2, 3), target = trunc(pixel + sigma z); a target outside the frame redraws both coordinates.
+ * n_gauss > 0 with cell_radius 0 on a frame whose H or W is no multiple of cellh / cellw: FLOWB200_EUNSUPPORTED.
+ * The pixels of the remainder strips search no cell, so their first random proposal goes to slot 0, which is what
+ * other pixels read as their best vector; the reference then gives a result that depends on its x-major scan. */
 int flowb200_random_proposals(const float* desc_src, const float* desc_tgt, const flowb200_params* p,
                               int32_t* pvec, float* lcost, int32_t* nprop, const int32_t* labels,
                               const int16_t* draws, uint64_t seed, flowb200_stream_t stream);

@@ -176,7 +176,10 @@ __global__ void finish_nn_kernel(KnnGeom g, int KC, int32_t* __restrict__ pvec, 
 // ----------------------------------------------------------------------------------------------
 // nasumicni (:205-233).  One thread per pixel; the 25 draws of a pixel are sequential because each
 // accepted proposal changes the duplicate test of the next one.  Reads only NN slots of other
-// pixels (never rewritten here), so pixels are independent.
+// pixels (never rewritten here), so pixels are independent.  The one exception, refused by
+// flowb200_random_proposals: radius 0 on a frame that is no whole multiple of the cell, where the
+// remainder pixels have no NN slot and publish their first random proposal in slot 0, which the
+// reference's x-major scan shows to the pixels after them and not to those before.
 // ----------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t mulhilo(uint32_t a, uint32_t b, uint32_t* hi) {
   uint64_t p = (uint64_t)a * b;
@@ -408,6 +411,8 @@ extern "C" int flowb200_random_proposals(const float* desc_src, const float* des
   if (rc) return rc;
   if (!desc_src || !desc_tgt || !pvec || !lcost || !nprop || !labels) return FLOWB200_EINVAL;
   if (p->n_gauss == 0) return FLOWB200_OK;
+  // radius 0, ragged frame: the result depends on the reference's scan order (see random_proposals_kernel)
+  if (p->cell_radius == 0 && (p->H % p->cellh || p->W % p->cellw)) return FLOWB200_EUNSUPPORTED;
   const KnnGeom g = make_geom(p);
   const int n = g.H * g.W;
   random_proposals_kernel<<<(n + 127) / 128, 128, 0, stream>>>(desc_src, desc_tgt, g, p->k_cell, p->n_gauss, p->sigma,

@@ -328,7 +328,10 @@ static inline double gauss(uint64_t* s) {
 /* nasumicni (daisy i flann.py:205-233).  proposals int32 [H][W][K][2], lcosts f64, nprop int32 are updated
  * in place; bestlabels is read only.  draws: optional int16 [H][W][n_gauss][2] accepted in-bounds (tgy,tgx)
  * to replay; NULL -> Gaussian draws from `seed` with the reference's rejection rules (:216-222, :233).
- * Pixels are independent: only NN slots of other pixels are read, and those are never rewritten. */
+ * Pixels are independent: only NN slots of other pixels are read, and those are never rewritten.  The exception is
+ * radius 0 on a frame that is no whole multiple of the cell (flowb200_random_proposals refuses it): a remainder pixel
+ * has no NN slot, its first random proposal lands in slot 0 (its bestlabels), and the reference's x-major scan shows
+ * it to the pixels after it only; this row-major parallel loop does not reproduce that. */
 int fo_nasumicni(const float* desc1, const float* desc2, int H, int W, int cellw, int cellh, int kc, int K,
                  int n_gauss, double sigma, double tphi, int32_t* proposals, double* lcosts, int32_t* nprop,
                  const int32_t* bestlabels, const int16_t* draws, uint64_t seed) {

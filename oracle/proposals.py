@@ -138,10 +138,15 @@ def _in_slice(tv, arr, a, b):
     return bool((sl == tv).any())
 
 
-def nasumicni(desc1, desc2, proposals, lcosts, nprop, bestlabels, p, draws):
+def nasumicni(desc1, desc2, proposals, lcosts, nprop, bestlabels, p, draws, snapshot=False):
     """nasumicni (:205-233) with the accepted Gaussian draws replayed from `draws`
-    (int array (H,W,n_gauss,2) of in-bounds (tgy,tgx)); modifies proposals/lcosts/nprop in place."""
+    (int array (H,W,n_gauss,2) of in-bounds (tgy,tgx)); modifies proposals/lcosts/nprop in place.
+
+    The reference scans x-major and reads a neighbour's best vector from the array it is filling, so a pixel that
+    had no NN proposals (bestlabels 0 pointing at an unused slot) shows its first random proposal to the pixels
+    scanned after it.  snapshot=True reads every neighbour's vector as it was before the pass instead."""
     H, W = p.H, p.W
+    src = proposals.copy() if snapshot else proposals
     ngaussprop = np.zeros((H, W), dtype=np.int64)
     for x in range(W):
         for y in range(H):
@@ -151,7 +156,7 @@ def nasumicni(desc1, desc2, proposals, lcosts, nprop, bestlabels, p, draws):
             for i in range(p.n_gauss):
                 tgy, tgx = int(draws[y, x, i, 0]), int(draws[y, x, i, 1])
                 broj = p.k_cell * ((tgy // p.cellh - mincellyl) + (tgx // p.cellw - mincellxl) * ncellyl)
-                tv = proposals[tgy, tgx, bestlabels[tgy, tgx]]
+                tv = src[tgy, tgx, bestlabels[tgy, tgx]]
                 n = int(nprop[y, x])
                 if (not _in_slice(tv, proposals[y, x], broj, broj + p.k_cell)) and \
                         (not _in_slice(tv, proposals[y, x], n - int(ngaussprop[y, x]), n)):

@@ -109,8 +109,21 @@ GEOMETRIES = [
 ]
 
 
-@pytest.mark.parametrize("knn_mode", KNN_MODES)
-@pytest.mark.parametrize("geom", GEOMETRIES, ids=lambda g: "x".join(map(str, g)))
+# the float64 search's other compiled widths (knn_exact_dispatch: k = 1, 2, 3, 4, 8, 16; the tensor-core search has
+# only 5 / 10 / 12) on ragged frames: topk_insert<1> has no shift loop, <16> the longest
+FP64_GEOMETRIES = [
+    (43, 61, 8, 4, 2, 1),
+    (50, 71, 16, 8, 1, 2),
+    (61, 83, 13, 11, 2, 3),
+    (37, 53, 4, 4, 3, 4),          # k = T / 4
+    (101, 9, 1, 40, 2, 8),
+    (45, 70, 8, 2, 2, 16),         # k = T: every target of a cell is a neighbour
+    (60, 90, 12, 10, 1, 16),
+]
+SWEEP = [(g, m) for g in GEOMETRIES for m in KNN_MODES] + [(g, 0) for g in FP64_GEOMETRIES]
+
+
+@pytest.mark.parametrize("geom,knn_mode", SWEEP, ids=["x".join(map(str, g)) + f"-{m}" for g, m in SWEEP])
 def test_geometry_sweep(geom, knn_mode):
     H, W, cw, ch, R, k = geom
     rng = np.random.default_rng(H * 7 + W)
@@ -139,6 +152,17 @@ def test_unsupported_geometry_raises_in_tcgen05_mode(geom):
             gpu_search(d1, d2, p, 0)
     else:
         assert_search_equal(gpu_search(d1, d2, p, 0), oracle_search(d1, d2, p))
+
+
+@pytest.mark.parametrize("k", [6, 7, 9])
+def test_float64_search_refuses_widths_it_does_not_compile(k):
+    """k = 6, 7, 9 fit the cell but have no knn_exact_kernel instance: FLOWB200_EUNSUPPORTED in mode 0."""
+    lib = pkg("_lib")
+    rng = np.random.default_rng(k)
+    p = flow_params(24, 36, 4, 6, 1, k)
+    d1, d2 = random_desc(rng, p.H, p.W), random_desc(rng, p.H, p.W)
+    with pytest.raises(lib.FlowB200Error, match="unsupported"):
+        gpu_search(d1, d2, p, 0)
 
 
 # ---------------------------------------------------------------- ties and near-ties
