@@ -82,6 +82,8 @@ typedef struct flowb200_params {
                                 0, 0 = all.  For callers that shard the target cells (single-huge-image mode): the
                                 slots of the other columns' proposals are left unwritten, nprop / labels assume
                                 the full set.  Honoured by FLOWB200_KNN_TCGEN05 (KNN_EXACT_FP64 searches all). */
+  int32_t flow_refine;       /* flowb200_flow_pair's fields: 0 = integer vectors (flowb200_flow_from_labels), 1 =
+                                sub-pixel vectors (flowb200_flow_subpixel); the check runs on either.  Default 0. */
 } flowb200_params;
 
 int flowb200_version(void);
@@ -205,6 +207,17 @@ int flowb200_slot_copy(const int64_t* table, int n_entries, int32_t* vec, float*
 int flowb200_flow_from_labels(const int32_t* pvec, const int32_t* labels, int H, int W, int K,
                               double* flow_yx, float* uvv, flowb200_stream_t stream);
 
+/* ---- sub-pixel flow (no reference counterpart; DESIGN section 4.8) ----
+ * flowb200_flow_from_labels with every vector refined per axis by the vertex of the parabola through the untruncated
+ * data costs c(e) = sum68_numpy_order(|desc_src(p) - desc_tgt(p + v + e)|) at e = 0 and e = -1, +1 along that axis:
+ * offset = (c- - c+) / (2 (c- - 2 c0 + c+)) in float32 round-to-nearest, applied when the three targets lie in the
+ * frame and c0 < c-, c0 < c+, clamped to [-0.5, 0.5], else 0.  uvv: float32 [H][W][3] = (dx + ox, dy + oy, 1).
+ * A label in [0, K) outside [0, nprop) or a (-1,-1) fill vector gives (dx, dy, 1) unrefined; a label outside [0, K)
+ * gives (0, 0, 0).  desc_src / desc_tgt: float32 [H][W][68], 16-byte aligned.  No workspace.  EINVAL for a null or
+ * misaligned pointer, H < 1, W < 1 or K outside 1..512. */
+int flowb200_flow_subpixel(const float* desc_src, const float* desc_tgt, const int32_t* pvec, const int32_t* nprop,
+                           const int32_t* labels, int H, int W, int K, float* uvv, flowb200_stream_t stream);
+
 /* ---- A13/A14  consistencyCheck / fowardBackwardConsistency (postprocessing.py:79-117) ----
  * flow1 (in place) and flow2: float32 [A][B][3] = (dx, dy, valid).  Quirk Q5 (dx added to the row index)
  * is reproduced.  Only pixels a0<=a<a1, b0<=b<b1 are checked (whole image: 0,A,0,B).  A valid pixel whose target
@@ -236,7 +249,8 @@ int flowb200_epe(const float* test_uvv, const float* gt_uvv, int H, int W, float
                  flowb200_stream_t stream);
 
 /* ---- whole path, device resident: two DAISYs, per direction kNN + random proposals + `sweeps` BCD
- *      sweeps, then the forward/backward check.  bgr0/bgr1: uint8 [H][W][3].
+ *      sweeps + label -> flow (sub-pixel with p->flow_refine = 1), then the forward/backward check.
+ *      bgr0/bgr1: uint8 [H][W][3].  p->flow_refine outside {0, 1}: FLOWB200_EINVAL.
  * out_fwd: float32 [H][W][3] checked forward field (sparse_field.npy layout); out_fwd_raw / out_bwd_raw
  * (optional): unchecked (dx,dy,1) fields of both directions. directions: 1 = forward only (no check),
  * 2 = forward + backward + check. */

@@ -23,7 +23,7 @@ class CParams(C.Structure):
         ("cell_radius", C.c_int32), ("k_cell", C.c_int32), ("n_gauss", C.c_int32), ("sigma", C.c_float),
         ("maxnprop", C.c_int32), ("tphi", C.c_float), ("tpsi", C.c_int32), ("lamda", C.c_double),
         ("cost_shift", C.c_int32), ("bcd_mode", C.c_int32), ("knn_mode", C.c_int32), ("con_tresh", C.c_float),
-        ("cell_x0", C.c_int32), ("cell_x1", C.c_int32),
+        ("cell_x0", C.c_int32), ("cell_x1", C.c_int32), ("flow_refine", C.c_int32),
     ]
 
 
@@ -60,6 +60,7 @@ SYMBOLS = {
     "flowb200_best_labels": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P]),
     "flowb200_slot_copy": (C.c_int, [_P, C.c_int, _P, _P, C.c_int, C.c_int, _P, C.c_int, _P]),
     "flowb200_flow_from_labels": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P, _P]),
+    "flowb200_flow_subpixel": (C.c_int, [_P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int, _P, _P]),
     "flowb200_consistency": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_float, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
     "flowb200_segments_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
     "flowb200_remove_small_segments": (C.c_int, [_P, C.c_int, C.c_int, C.c_float, C.c_int, _P, C.c_size_t, _P]),

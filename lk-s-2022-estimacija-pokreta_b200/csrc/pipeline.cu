@@ -119,7 +119,7 @@ extern "C" size_t flowb200_pair_workspace_bytes(const flowb200_params* p) {
   return pair_layout(p).total;
 }
 
-// one direction = proposals (search + random), then BCD + flow field
+// one direction = proposals (search + random), then BCD + flow field (integer, or sub-pixel with p->flow_refine)
 static int run_proposals(const flowb200_params* p, const PairLayout& L, char* ws, int d, uint64_t seed,
                          cudaStream_t stream) {
   const float* src = reinterpret_cast<const float*>(ws + L.desc[d]);
@@ -149,8 +149,12 @@ static int run_bcd(const flowb200_params* p, const PairLayout& L, char* ws, int 
                         p->cost_shift, sweeps, nullptr, ws + L.bcd_ws[d],
                         flowb200_bcd_workspace_bytes(p->H, p->W, p->maxnprop), stream);
   if (rc) return rc;
-  return flowb200_flow_from_labels(pvec, labels, p->H, p->W, p->maxnprop, nullptr,
-                                   reinterpret_cast<float*>(ws + L.uvv[d]), stream);
+  float* uvv = reinterpret_cast<float*>(ws + L.uvv[d]);
+  if (p->flow_refine)   // both directions' descriptors stay in the workspace until the call returns
+    return flowb200_flow_subpixel(reinterpret_cast<const float*>(ws + L.desc[d]),
+                                  reinterpret_cast<const float*>(ws + L.desc[1 - d]), pvec, nprop, labels, p->H, p->W,
+                                  p->maxnprop, uvv, stream);
+  return flowb200_flow_from_labels(pvec, labels, p->H, p->W, p->maxnprop, nullptr, uvv, stream);
 }
 
 static int run_direction(const flowb200_params* p, const PairLayout& L, char* ws, int d, int sweeps, uint64_t seed,
@@ -165,6 +169,7 @@ extern "C" int flowb200_flow_pair(const uint8_t* bgr0, const uint8_t* bgr1, cons
   if (!bgr0 || !bgr1 || !p || !out_fwd || !workspace) return FLOWB200_EINVAL;
   if (directions != 1 && directions != 2) return FLOWB200_EINVAL;
   if (sweeps < 0) return FLOWB200_EINVAL;
+  if (p->flow_refine != 0 && p->flow_refine != 1) return FLOWB200_EINVAL;
   const PairLayout L = pair_layout(p);
   if (workspace_bytes < L.total) return FLOWB200_EWORKSPACE;
   char* ws = static_cast<char*>(workspace);

@@ -1,8 +1,13 @@
 // Label -> flow gather and the forward/backward consistency check.
 //   flow_from_labels : vratiKonacniFlow (daisy i flann.py:192-197 / python bcd.py:90-95) fused with
 //                      FlowImage.ucitajFlow's (dx, dy, valid=1) float32 layout (postprocessing.py:7-17)
+//   flow_subpixel    : flow_from_labels with each vector refined to sub-pixel precision (DESIGN section 4.8;
+//                      no reference counterpart)
 //   consistency      : consistencyCheck / fowardBackwardConsistency (postprocessing.py:79-117)
-// Both are HBM-bound streaming kernels: 28 B/pixel algorithmic (SURVEY.md section 8d).
+// flow_from_labels and consistency are HBM-bound streaming kernels: 28 B/pixel algorithmic (SURVEY.md section 8d);
+// flow_subpixel reads six descriptor rows per pixel: 1652 B/pixel, mostly from L2 (DESIGN section 4.8).
+#include <climits>
+
 #include "common.cuh"
 
 namespace flowb200 {
@@ -22,6 +27,75 @@ __global__ void flow_from_labels_kernel(const int32_t* __restrict__ pvec, const 
     uvv[3 * (size_t)i + 1] = (float)dy;
     uvv[3 * (size_t)i + 2] = 1.0f;
   }
+}
+
+// Sub-pixel refinement (DESIGN section 4.8): per axis, the vertex of the parabola through the data costs of the chosen
+// target and its two neighbours along that axis.  One thread per pixel; the source row stays in registers and each
+// target row is read as 17 float4 loads (rows are 272 B: 16-byte aligned when the base is).  Every float32 operation
+// is an explicit round-to-nearest intrinsic, so that tests/subpixel_oracle.py restates it bit for bit.
+__device__ __forceinline__ float subpixel_cost(const float (&s)[kDescDim], const float* __restrict__ row) {
+  float t[kDescDim];
+  const float4* r4 = reinterpret_cast<const float4*>(row);
+#pragma unroll
+  for (int k = 0; k < kDescDim / 4; ++k) {
+    const float4 v = __ldg(r4 + k);
+    t[4 * k] = v.x;
+    t[4 * k + 1] = v.y;
+    t[4 * k + 2] = v.z;
+    t[4 * k + 3] = v.w;
+  }
+  return sum68_numpy_order([&](int d) { return fabsf(__fsub_rn(s[d], t[d])); });
+}
+
+// (c- - c+) / (2 (c- - 2 c0 + c+)) where c0 is a strict minimum, clamped to [-0.5, 0.5]; 0 otherwise
+__device__ __forceinline__ float subpixel_offset(float cm, float c0, float cp) {
+  if (!(c0 < cm && c0 < cp)) return 0.f;
+  const float num = __fsub_rn(cm, cp);
+  const float den = __fmul_rn(2.f, __fadd_rn(__fsub_rn(cm, __fmul_rn(2.f, c0)), cp));
+  return fminf(fmaxf(__fdiv_rn(num, den), -0.5f), 0.5f);
+}
+
+__global__ void __launch_bounds__(128) subpixel_kernel(const float* __restrict__ desc_src,
+                                                       const float* __restrict__ desc_tgt,
+                                                       const int32_t* __restrict__ pvec,
+                                                       const int32_t* __restrict__ nprop,
+                                                       const int32_t* __restrict__ labels, int H, int W, int K,
+                                                       float* __restrict__ uvv) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= H * W) return;
+  float* o = uvv + 3 * (size_t)i;
+  const int l = labels[i];
+  if (l < 0 || l >= K) {   // names no slot: no vector
+    o[0] = 0.f;
+    o[1] = 0.f;
+    o[2] = 0.f;
+    return;
+  }
+  const int32_t v = pvec[(size_t)i * K + l];
+  const int dy = vec_dy(v), dx = vec_dx(v);
+  const int y = i / W, x = i - y * W, ty = y + dy, tx = x + dx;
+  float ox = 0.f, oy = 0.f;
+  if (l < nprop[i] && v != -1 && ty >= 0 && ty < H && tx >= 0 && tx < W) {
+    float s[kDescDim];
+    const float4* s4 = reinterpret_cast<const float4*>(desc_src + (size_t)i * kDescDim);
+#pragma unroll
+    for (int k = 0; k < kDescDim / 4; ++k) {
+      const float4 a = __ldg(s4 + k);
+      s[4 * k] = a.x;
+      s[4 * k + 1] = a.y;
+      s[4 * k + 2] = a.z;
+      s[4 * k + 3] = a.w;
+    }
+    const float* t = desc_tgt + ((size_t)ty * W + tx) * kDescDim;
+    const float c0 = subpixel_cost(s, t);
+    if (tx >= 1 && tx + 1 < W)
+      ox = subpixel_offset(subpixel_cost(s, t - kDescDim), c0, subpixel_cost(s, t + kDescDim));
+    if (ty >= 1 && ty + 1 < H)
+      oy = subpixel_offset(subpixel_cost(s, t - (size_t)W * kDescDim), c0, subpixel_cost(s, t + (size_t)W * kDescDim));
+  }
+  o[0] = __fadd_rn((float)dx, ox);
+  o[1] = __fadd_rn((float)dy, oy);
+  o[2] = 1.0f;
 }
 
 // One thread per checked pixel (a, b) = (row, col) of flow1.  float32 arithmetic with explicit
@@ -177,6 +251,19 @@ extern "C" int flowb200_flow_from_labels(const int32_t* pvec, const int32_t* lab
   if (!pvec || !labels || H <= 0 || W <= 0 || K <= 0) return FLOWB200_EINVAL;
   int n = H * W;
   flow_from_labels_kernel<<<(n + 255) / 256, 256, 0, stream>>>(pvec, labels, n, K, flow_yx, uvv);
+  FB_LAUNCH_CHECK();
+  return FLOWB200_OK;
+}
+
+extern "C" int flowb200_flow_subpixel(const float* desc_src, const float* desc_tgt, const int32_t* pvec,
+                                      const int32_t* nprop, const int32_t* labels, int H, int W, int K, float* uvv,
+                                      flowb200_stream_t stream) {
+  if (!desc_src || !desc_tgt || !pvec || !nprop || !labels || !uvv) return FLOWB200_EINVAL;
+  if (H < 1 || W < 1 || K < 1 || K > 512 || (long long)H * W > INT_MAX) return FLOWB200_EINVAL;
+  // descriptor rows are read as float4
+  if ((reinterpret_cast<uintptr_t>(desc_src) | reinterpret_cast<uintptr_t>(desc_tgt)) & 15) return FLOWB200_EINVAL;
+  const int n = H * W;
+  subpixel_kernel<<<(n + 127) / 128, 128, 0, stream>>>(desc_src, desc_tgt, pvec, nprop, labels, H, W, K, uvv);
   FB_LAUNCH_CHECK();
   return FLOWB200_OK;
 }

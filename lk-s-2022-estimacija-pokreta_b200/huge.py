@@ -320,7 +320,10 @@ def flow_pair_sharded(bgr0, bgr1, p: FlowParams, sweeps, directions, seed, bcd_m
         else:   # the float64 programme is not split: replicated
             ops.bcd(pvec, lcost, nprop, labels, sweeps, mode=_lib.BCD_FP64_F32COST | mrf, lamda=p.lamda, tpsi=p.tpsi,
                     cost_shift=p.cost_shift)
-        uvv.append(ops.flow_from_labels(pvec, labels, want_yx=False)[1])
+        if p.flow_refine:
+            uvv.append(ops.flow_subpixel(src, tgt, pvec, nprop, labels))
+        else:
+            uvv.append(ops.flow_from_labels(pvec, labels, want_yx=False)[1])
         del pvec, lcost
     out = uvv[0].clone()
     if directions == 2:

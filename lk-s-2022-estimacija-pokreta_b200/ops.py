@@ -41,7 +41,7 @@ def cparams(p: FlowParams, bcd_mode=_lib.BCD_FP64_F32COST, knn_mode=None):
     return _lib.CParams(H=p.H, W=p.W, cellw=p.cellw, cellh=p.cellh, cell_radius=p.cell_radius, k_cell=p.k_cell,
                         n_gauss=p.n_gauss, sigma=p.sigma, maxnprop=p.maxnprop, tphi=p.tphi, tpsi=p.tpsi,
                         lamda=p.lamda, cost_shift=p.cost_shift, bcd_mode=bcd_mode, knn_mode=knn_mode,
-                        con_tresh=p.con_tresh, cell_x0=p.cell_x0, cell_x1=p.cell_x1)
+                        con_tresh=p.con_tresh, cell_x0=p.cell_x0, cell_x1=p.cell_x1, flow_refine=p.flow_refine)
 
 
 def _workspace(nbytes, device):
@@ -236,6 +236,21 @@ def flow_from_labels(pvec, labels, want_yx=True, want_uvv=True):
     _lib.check(lib.flowb200_flow_from_labels(_ptr(pvec, torch.int32), _ptr(labels, torch.int32), H, W, K, _ptr(yx),
                                              _ptr(uvv), _stream()), "flowb200_flow_from_labels")
     return yx, uvv
+
+
+def flow_subpixel(desc_src, desc_tgt, pvec, nprop, labels):
+    """flow_from_labels with every vector refined per axis to the vertex of the parabola through the data costs of the
+    target and its two neighbours (DESIGN section 4.8).  Returns uvv float32 (H,W,3) = (dx + ox, dy + oy, 1)."""
+    lib = _lib.load()
+    H, W, K = pvec.shape
+    assert tuple(desc_src.shape) == (H, W, 68) and tuple(desc_tgt.shape) == (H, W, 68)
+    assert tuple(nprop.shape) == (H, W) and tuple(labels.shape) == (H, W)
+    uvv = torch.empty((H, W, 3), dtype=torch.float32, device=pvec.device)
+    _lib.check(lib.flowb200_flow_subpixel(_ptr(desc_src, torch.float32, "desc_src"),
+                                          _ptr(desc_tgt, torch.float32, "desc_tgt"), _ptr(pvec, torch.int32, "pvec"),
+                                          _ptr(nprop, torch.int32, "nprop"), _ptr(labels, torch.int32, "labels"), H, W,
+                                          K, _ptr(uvv), _stream()), "flowb200_flow_subpixel")
+    return uvv
 
 
 def consistency(flow1, flow2, tresh, region=None):

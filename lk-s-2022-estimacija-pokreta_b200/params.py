@@ -31,6 +31,7 @@ class FlowParams:
     knn_mode: int = 0            # FLOWB200_KNN_* (0 = float64 CUDA cores, 1 = tcgen05 prefilter + exact re-rank)
     cell_x0: int = 0             # target cell columns searched: [cell_x0, cell_x1); 0, 0 = all (huge.py: a rank's band)
     cell_x1: int = 0
+    flow_refine: int = 0         # flow_pair's fields: 0 = integer vectors, 1 = sub-pixel (flowb200_flow_subpixel)
 
     @property
     def ncellx(self):
@@ -67,6 +68,8 @@ class FlowParams:
             raise ValueError("maxnprop > 512 not supported")
         if (self.cell_x0, self.cell_x1) != (0, 0) and not 0 <= self.cell_x0 < self.cell_x1 <= self.ncellx:
             raise ValueError("cell_x0 / cell_x1 must select a non-empty range of cell columns")
+        if self.flow_refine not in (0, 1):
+            raise ValueError("flow_refine must be 0 (integer vectors) or 1 (sub-pixel)")
         return self
 
 
