@@ -237,7 +237,9 @@ int flowb200_remove_small_segments(float* flow, int A, int B, float tresh, int m
 /* ---- edge.canny_ivice (edge.py:19-35; SURVEY 8f row 4): EpicFlow's edge input ----
  * bgr: uint8 [H][W][3].  inverted_edges: float32 [H][W], 0.0f on an edge, 1.0f elsewhere (edge.py:29).
  * cvtColor(BGR2GRAY) -> GaussianBlur(3x3, sigma 0) -> Canny(low, high) (the reference passes 100, 200), L1 gradient,
- * aperture 3: OpenCV's 8-bit integer arithmetic, bit-identical (csrc/edges_core.cuh). */
+ * aperture 3: OpenCV's 8-bit integer arithmetic, bit-identical (csrc/edges_core.cuh).  low and high are cvFloor of
+ * cv2.Canny's threshold1 and threshold2 and may come in either order: as in cv::Canny, they are swapped when
+ * low > high. */
 size_t flowb200_edges_workspace_bytes(int H, int W);
 int flowb200_canny_edges(const uint8_t* bgr, int H, int W, int low, int high, float* inverted_edges, void* workspace,
                          size_t workspace_bytes, flowb200_stream_t stream);

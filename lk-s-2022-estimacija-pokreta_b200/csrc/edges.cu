@@ -99,6 +99,11 @@ extern "C" int flowb200_canny_edges(const uint8_t* bgr, int H, int W, int low, i
     return FLOWB200_EINVAL;
   const EdgeLayout L = edge_layout(H, W);
   if (workspace_bytes < L.total) return FLOWB200_EWORKSPACE;
+  if (low > high) {   // cv::Canny swaps its thresholds when threshold1 > threshold2
+    const int t = low;
+    low = high;
+    high = t;
+  }
   char* ws = static_cast<char*>(workspace);
   uint8_t* blur = reinterpret_cast<uint8_t*>(ws + L.blur);
   uint8_t* pmap = reinterpret_cast<uint8_t*>(ws + L.pmap);

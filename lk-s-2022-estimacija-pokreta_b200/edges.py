@@ -15,14 +15,15 @@ from . import _lib
 
 
 def canny_edges(img_bgr, threshold1=100, threshold2=200):
-    """uint8 (H,W,3) BGR array -> float32 (H,W) `(255 - cv2.Canny(...)) / 255` (edge.py:21-29)."""
+    """uint8 (H,W,3) BGR array -> float32 (H,W) `(255 - cv2.Canny(...)) / 255` (edge.py:21-29).  The thresholds
+    may come in either order, as for cv2.Canny: the smaller one is the low threshold."""
     img = np.ascontiguousarray(img_bgr, dtype=np.uint8)
     if img.ndim != 3 or img.shape[2] != 3:
         raise TypeError("expected an (H,W,3) uint8 BGR image")
     H, W = img.shape[:2]
     out = np.empty((H, W), dtype=np.float32)
     L = _lib.load()
-    # cv::Canny compares the integer L1 magnitude with cvFloor of both thresholds
+    # cv::Canny compares the integer L1 magnitude with cvFloor of both thresholds (the library swaps them if needed)
     _lib.check(L.flowb200_canny_edges_host(img.ctypes.data, H, W, math.floor(threshold1), math.floor(threshold2),
                                            out.ctypes.data), "flowb200_canny_edges_host")
     return out

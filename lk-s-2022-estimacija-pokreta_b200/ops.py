@@ -11,6 +11,7 @@ through the C ABI (include/flowb200.h).  torch only owns the memory.  Device lay
   uvv     float32 (H, W, 3)         (dx, dy, valid)                           (postprocessing.py:7-17)
 """
 import ctypes as C
+import math
 
 import torch
 
@@ -280,15 +281,17 @@ def remove_small_segments(flow, tresh, min_segment_size, workspace=None):
 
 def canny_edges(bgr, low=100, high=200, workspace=None):
     """edge.canny_ivice (edge.py:19-35) without the file I/O: uint8 (H,W,3) device tensor -> float32 (H,W),
-    0.0 on an edge, 1.0 elsewhere."""
+    0.0 on an edge, 1.0 elsewhere.  `low` and `high` are floored like cv2.Canny's thresholds and may come in either
+    order (the smaller one is the low threshold)."""
     lib = _lib.load()
     H, W, ch = bgr.shape
     assert ch == 3
     out = torch.empty((H, W), dtype=torch.float32, device=bgr.device)
     if workspace is None:
         workspace = torch.empty(int(lib.flowb200_edges_workspace_bytes(H, W)), dtype=torch.uint8, device=bgr.device)
-    _lib.check(lib.flowb200_canny_edges(_ptr(bgr, torch.uint8, "bgr"), H, W, int(low), int(high), _ptr(out),
-                                        _ptr(workspace), workspace.numel(), _stream()), "flowb200_canny_edges")
+    _lib.check(lib.flowb200_canny_edges(_ptr(bgr, torch.uint8, "bgr"), H, W, math.floor(low), math.floor(high),
+                                        _ptr(out), _ptr(workspace), workspace.numel(), _stream()),
+               "flowb200_canny_edges")
     return out
 
 

@@ -56,11 +56,19 @@ def _inplace_field(flow, name):
 
 
 def removeSmallSegments(flow, tresh, min_segment_size):
-    """In place on flow, returns None like the reference (:29-76)."""
+    """In place on flow, returns None like the reference (:29-76).
+
+    A segment of `count` pixels is removed when `count > 1 and count < min_segment_size` (:73).  With an integer count
+    a fractional bound acts like its ceiling, clamped to [0, 2**31 - 1]; NaN and -inf remove nothing (bound 0) and
+    +inf removes every segment of two or more pixels (bound 2**31 - 1), as that comparison implies."""
     f = _inplace_field(flow, "flow")
     L = _lib.load()
-    # `1 < count < min_segment_size` (:73) with an integer count: a fractional bound acts like its ceiling
-    bound = max(0, min(int(math.ceil(min_segment_size)), 2**31 - 1))
+    try:
+        bound = max(0, min(int(math.ceil(min_segment_size)), 2**31 - 1))
+    except ValueError:      # NaN: the comparison is always false
+        bound = 0
+    except OverflowError:   # +inf: every count of two or more is below it; -inf: none is
+        bound = 2**31 - 1 if min_segment_size > 0 else 0
     _lib.check(L.flowb200_remove_small_segments_host(f.ctypes.data, f.shape[0], f.shape[1], float(tresh), bound),
                "flowb200_remove_small_segments_host")
 

@@ -14,6 +14,7 @@ OpenCV's integer arithmetic as restated here (8-bit input, aperture 3, L2gradien
            vertical (|dy| << 15 > |dx| * 13573 + (|dx| << 16)): m > up and m >= down; diagonal: m > both
            neighbours on the diagonal the signs of dx, dy select
   hysteresis  survivors with mag > high are edges; survivors 8-connected to an edge are edges
+  thresholds  floored; swapped when low > high (cv::Canny takes them in either order)
 """
 import numpy as np
 
@@ -89,9 +90,13 @@ def hysteresis(pmap):
 
 
 def canny(img_u8, low=100, high=200):
-    """cv2.Canny(img, low, high) -> uint8 {0, 255}."""
+    """cv2.Canny(img, low, high) -> uint8 {0, 255}.  Like cv::Canny, the thresholds are floored and taken in either
+    order: when low > high the two are swapped (floor is monotonic, so swapping before or after it is the same)."""
     dx, dy = sobel3(img_u8)
-    return hysteresis(nms_map(dx, dy, int(np.floor(low)), int(np.floor(high)))).astype(np.uint8) * 255
+    lo, hi = int(np.floor(low)), int(np.floor(high))
+    if lo > hi:
+        lo, hi = hi, lo
+    return hysteresis(nms_map(dx, dy, lo, hi)).astype(np.uint8) * 255
 
 
 def canny_ivice(bgr, low=100, high=200):

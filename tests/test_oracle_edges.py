@@ -82,3 +82,31 @@ def test_device_arithmetic_on_host_vs_oracle_random(emul):
         assert np.array_equal(emul(img, lo, hi), want), (it, img.shape, lo, hi)
         edges += int((want == 0).sum())
     assert edges > 20000
+
+
+@pytest.mark.parametrize("shape", [(60, 70), (8, 8), (150, 199)])
+def test_oracle_descending_thresholds_equal_cv2(shape):
+    """cv2.Canny takes its thresholds in either order; so does the oracle.  On blurred noise most survivors are weak,
+    so the order matters: the unswapped pair gives another edge map at (200, 100) or (90, 30)."""
+    from helpers import canny_blurred_noise, canny_pmap
+    rng = np.random.default_rng(shape[0] * 31 + shape[1])
+    differs = 0
+    for it in range(4):
+        bl = cv2.GaussianBlur(cv2.cvtColor(canny_blurred_noise(rng, *shape), cv2.COLOR_BGR2GRAY), (3, 3), 0)
+        for lo, hi in ((200, 100), (90, 30), (60, 20), (40.5, -3.5), (-0.5, -2.5)):
+            want = cv2.Canny(image=bl, threshold1=lo, threshold2=hi)
+            assert np.array_equal(oe.canny(bl, lo, hi), want), (it, lo, hi)
+            differs += not np.array_equal(oe.hysteresis(canny_pmap(bl, lo, hi)), want > 0)
+    assert differs >= 4
+
+
+def test_device_arithmetic_on_host_descending_thresholds(emul):
+    """The host build of the per-pixel functions with the library's swap, at descending pairs, against cv2."""
+    from helpers import canny_blurred_noise
+    rng = np.random.default_rng(5)
+    for H, W in ((60, 70), (33, 17)):
+        img = canny_blurred_noise(rng, H, W)
+        for lo, hi in ((200, 100), (90, 30)):
+            bl = cv2.GaussianBlur(cv2.cvtColor(img, cv2.COLOR_BGR2GRAY), (3, 3), 0)
+            want = np.array((255 - cv2.Canny(image=bl, threshold1=lo, threshold2=hi)) / 255, dtype="float32")
+            assert np.array_equal(emul(img, min(lo, hi), max(lo, hi)), want)
